@@ -57,7 +57,6 @@ SIGNATURES = {
     "ep_tc_linear_dx_bf16": (c_int, [c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p]),
     "ep_tc_chain_fwd_bf16": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_f, c_p, c_p,
                                      c_int, c_p]),
-    "ep_tc_chain_dx_bf16": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ep_tc_dw_workspace_bytes": (c_sz, []),
     "ep_tc_linear_dw_bf16": (c_int, [c_int, c_int, c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_sz, c_int, c_p]),
     "ep_grad_sqnorm_f32": (c_int, [c_sz, c_p, c_p, c_p]),
@@ -96,7 +95,7 @@ KERNELS_PER_CALL = {
     "ep_grad_sqnorm_f32": 2, "ep_adam_clip_step_f32": 1, "ep_fps_f64": 1, "ep_bounds_f64": 2,
     "ep_voxel_select_f64": 6, "ep_gather_rows_f32": 1, "ep_knn_grid_f64": 1, "ep_fem_elements_f64": 1, "ep_fem_segment_sum_f64": 1, "ep_scatter_add_rows_f32": 1,
     "ep_tc_pack_rows_bf16": 1, "ep_tc_pack_weight_bf16": 1, "ep_tc_linear_fwd_bf16": 1, "ep_tc_linear_final_bf16": 1,
-    "ep_tc_linear_dx_bf16": 1, "ep_tc_linear_dw_bf16": 2, "ep_tc_chain_fwd_bf16": 1, "ep_tc_chain_dx_bf16": 1,
+    "ep_tc_linear_dx_bf16": 1, "ep_tc_linear_dw_bf16": 2, "ep_tc_chain_fwd_bf16": 1,
     "ep_halo_exchange_f32": 1,
 }
 launch_counter = 0

@@ -547,110 +547,6 @@ eigen_bwd_fused_sym_kernel(int row0, int n, int k, int lpr_shift, const int32_t*
   }
 }
 
-// k = 32 specialisation of the fused symmetric backward.  Gather phase as above (8 lanes x float4 per row, 4 rows
-// per warp); for the 32 x 32 product every lane keeps ITS column of S in 32 registers and the four MU rows of the
-// warp are broadcast from shared memory (8 LDS.128 per row instead of 32 per lane-row), then the result returns to
-// the float4 layout through shared memory for the coalesced store.
-__global__ void __launch_bounds__(256)
-eigen_bwd_fused_sym_k32_kernel(int row0, int n, const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                               const float* __restrict__ valK, const float* __restrict__ valM,
-                               const float* __restrict__ KU, const float* __restrict__ MU, int ld,
-                               const float* __restrict__ coef, float out_scale_v,
-                               const float* __restrict__ out_scale_dev, float* __restrict__ dU, int ldo) {
-  constexpr int k = 32;
-  __shared__ __align__(16) float sm_mu[8][4][32];
-  __shared__ __align__(16) float sm_out[8][4][32];
-  const float out_scale = out_scale_dev ? __ldg(out_scale_dev) : out_scale_v;
-  const float c_res = coef[0];
-  const float* c_lam = coef + 1;
-  const float* c_num = c_lam + k;
-  const float* c_den = c_num + k;
-  const float* c_G = c_den + k;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  float S_col[32];
-#pragma unroll
-  for (int m = 0; m < 32; ++m) {
-    float v = __ldg(c_G + m * k + lane) + __ldg(c_G + lane * k + m);
-    if (m == lane) v += 2.f * __ldg(c_den + m);
-    S_col[m] = v;
-  }
-  const int lane_r = lane & 7, rsub = lane >> 3;
-  const int cofs = 4 * lane_r;
-  // coef + 1 is not 16-byte aligned: scalar loads
-  const float4 lam4 = make_float4(__ldg(c_lam + cofs), __ldg(c_lam + cofs + 1), __ldg(c_lam + cofs + 2), __ldg(c_lam + cofs + 3));
-  const float4 a24 = make_float4(2.f * __ldg(c_num + cofs), 2.f * __ldg(c_num + cofs + 1), 2.f * __ldg(c_num + cofs + 2),
-                                 2.f * __ldg(c_num + cofs + 3));
-  const float* c_mean = c_G + k * k;
-  const float4 gm4 = make_float4(__ldg(c_mean + cofs), __ldg(c_mean + cofs + 1), __ldg(c_mean + cofs + 2), __ldg(c_mean + cofs + 3));
-  const long long rows_per_grid = (long long)gridDim.x * 32;                  // 8 warps x 4 rows per CTA
-  const long long n_iter = ((long long)n + rows_per_grid - 1) / rows_per_grid;
-  for (long long it = 0; it < n_iter; ++it) {
-    const long long ri = it * rows_per_grid + (long long)blockIdx.x * 32 + warp * 4 + rsub;
-    const bool valid = ri < n;
-    const long long row = row0 + ri;
-    const int start = valid ? __ldg(rowptr + row) : 0;
-    const int end = valid ? __ldg(rowptr + row + 1) : 0;
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    float m_rowsum = 0.f;
-    for (int j = start; j < end; j += 4) {
-      int c[4]; float kk[4], mm[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const bool ok = (j + u) < end;
-        c[u] = ok ? __ldg(col + j + u) : -1;
-        kk[u] = ok ? __ldg(valK + j + u) : 0.f;
-        mm[u] = ok ? __ldg(valM + j + u) : 0.f;
-        m_rowsum += mm[u];
-      }
-      float4 ku[4], mu[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        if (c[u] >= 0) {
-          ku[u] = __ldg(reinterpret_cast<const float4*>(KU + (size_t)c[u] * ld + cofs));
-          mu[u] = __ldg(reinterpret_cast<const float4*>(MU + (size_t)c[u] * ld + cofs));
-        } else { ku[u] = make_float4(0.f, 0.f, 0.f, 0.f); mu[u] = ku[u]; }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        acc.x = fmaf(kk[u] - lam4.x * mm[u], ku[u].x - lam4.x * mu[u].x, acc.x);
-        acc.y = fmaf(kk[u] - lam4.y * mm[u], ku[u].y - lam4.y * mu[u].y, acc.y);
-        acc.z = fmaf(kk[u] - lam4.z * mm[u], ku[u].z - lam4.z * mu[u].z, acc.z);
-        acc.w = fmaf(kk[u] - lam4.w * mm[u], ku[u].w - lam4.w * mu[u].w, acc.w);
-      }
-    }
-    acc.x = fmaf(acc.x, c_res, m_rowsum * gm4.x); acc.y = fmaf(acc.y, c_res, m_rowsum * gm4.y);
-    acc.z = fmaf(acc.z, c_res, m_rowsum * gm4.z); acc.w = fmaf(acc.w, c_res, m_rowsum * gm4.w);
-    float4 mu_i = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (valid) {
-      const float4 ku_i = __ldg(reinterpret_cast<const float4*>(KU + (size_t)row * ld + cofs));
-      mu_i = __ldg(reinterpret_cast<const float4*>(MU + (size_t)row * ld + cofs));
-      acc.x = fmaf(a24.x, ku_i.x, acc.x); acc.y = fmaf(a24.y, ku_i.y, acc.y);
-      acc.z = fmaf(a24.z, ku_i.z, acc.z); acc.w = fmaf(a24.w, ku_i.w, acc.w);
-    }
-    *reinterpret_cast<float4*>(&sm_mu[warp][rsub][cofs]) = mu_i;
-    __syncwarp();
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      float o = 0.f;
-#pragma unroll
-      for (int m4 = 0; m4 < 8; ++m4) {
-        const float4 mv = *reinterpret_cast<const float4*>(&sm_mu[warp][r][4 * m4]);       // broadcast
-        o = fmaf(mv.x, S_col[4 * m4], o); o = fmaf(mv.y, S_col[4 * m4 + 1], o);
-        o = fmaf(mv.z, S_col[4 * m4 + 2], o); o = fmaf(mv.w, S_col[4 * m4 + 3], o);
-      }
-      sm_out[warp][r][lane] = o;
-    }
-    __syncwarp();
-    const float4 o4 = *reinterpret_cast<const float4*>(&sm_out[warp][rsub][cofs]);
-    if (valid) {
-      acc.x = (acc.x + o4.x) * out_scale; acc.y = (acc.y + o4.y) * out_scale;
-      acc.z = (acc.z + o4.z) * out_scale; acc.w = (acc.w + o4.w) * out_scale;
-      *reinterpret_cast<float4*>(dU + (size_t)row * ldo + cofs) = acc;
-    }
-    __syncwarp();
-  }
-}
-
 template <int KP>
 int launch_bwd_prepare(int n, int k, const float* U, int ldu, const float* KU, const float* MU, int ld,
                        const float* coef, float* KU_bar, float* MU_bar, float* D, cudaStream_t st) {
@@ -823,15 +719,6 @@ int ep_eigen_bwd_gather_sym_rows_f32(int row0, int n, int k, const int32_t* rowp
   const long long cap = (long long)ep::sm_count() * 8;
   if (grid > cap) grid = cap;
   cudaStream_t st = ep::as_stream(stream);
-  if (k == 32 && ep::tune_flag(2) && !gram_in_out) {
-    long long g32 = ((long long)n + 31) / 32;
-    const long long cap32 = (long long)ep::sm_count() * 8;
-    if (g32 > cap32) g32 = cap32;
-    eigen_bwd_fused_sym_k32_kernel<<<(unsigned)g32, 256, 0, st>>>(row0, n, rowptr, col, valK, valM, KU, MU, ld, coef,
-                                                                  out_scale, out_scale_dev, dU, ldo);
-    EP_LAUNCH_CHECK("eigen_bwd_fused_sym_k32_kernel");
-    return EP_OK;
-  }
 #define EP_FUSED_LAUNCH(KVT, G) eigen_bwd_fused_sym_kernel<KVT, G><<<(unsigned)grid, 256, smem, st>>>( \
       row0, n, k, lpr_shift, rowptr, col, valK, valM, KU, MU, ld, coef, out_scale, out_scale_dev, dU, ldo)
   if (gram_in_out) {

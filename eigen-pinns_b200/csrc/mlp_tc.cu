@@ -216,316 +216,16 @@ __global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs
 }
 
 // ------------------------------------------------------------------------------------------- layer chain
-// tc_chain_kernel: ALL layers of the corrector MLP for a pair of 128-vertex tiles in one persistent CTA.
-//   MODE_CHAIN_FWD  x0 -> relu(. W0^T + b0) -> ... -> . W_{L-1}^T + b_{L-1}   (corrector_model.py:31)
-//   MODE_CHAIN_DX   dZ_{L-1} -> (. W_{L-1}) * mask_{L-2} -> ... -> dZ_0        (autograd of :258)
+// tc_chain2_kernel: ALL layers of the corrector MLP forward in one launch (corrector_model.py:31),
+//   x0 -> relu(. W0^T + b0) -> ... -> . W_{L-1}^T + b_{L-1},
+// run by CLUSTERS OF TWO CTAs with tcgen05.mma.cta_group::2.
 // The activation tile never leaves the SM between layers: the epilogue of layer l writes bf16 straight into the
 // shared-memory slot that is the A operand of layer l+1 (same packed K-major layout, in place) and, because the
 // backward pass needs it, streams the same 16-byte chunks to HBM (write-only traffic; nothing is read back).
-// Weights do not fit one SM (0.72 MB for 82->256x6->32), so they stream from L2 through a ring of 16 KB K-slabs;
-// two tiles advance in lock step so that every slab feeds two MMAs (M = 256 per weight pass halves the L2 traffic).
-// TMEM: tile 0 accumulates in columns [0, 256), tile 1 in [256, 512).
-// Warp roles: warp 0 = weight-slab TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..17 = epilogue
-// (TMEM lane quadrant = warp % 4, tile = ((warp - 2) / 4) % 2, column half = (warp - 2) / 8: four warps per
-// scheduler, because draining an accumulator is latency bound - TMEM load, convert, store - not issue bound);
-// the first epilogue thread also issues the input-tile TMA of the next pair as soon as the last layer's MMAs have
-// retired.  Measured per 256-wide layer and tile pair (clock64 trace, B200): 32 MMAs issue in 4300 clk.
-// Algorithmic HBM bytes per vertex (forward, 82->256x6->32): read 2*96, write 6*(2*256 + 32) + 2*4*32 -> 3.7 KB,
-// against 6.9 KB for the layer-by-layer kernels (every hidden activation was read back once).
-constexpr int CH_MAX_LAYERS = 8;
-constexpr int CH_CBW = 8;                // 32-column blocks per epilogue warp: 8 -> 8 epilogue warps, 4 -> 16
-constexpr int CH_THREADS = 64 + (8 / CH_CBW) * 256;
-constexpr int CH_STAGES = 5;
-constexpr int CH_SLAB_BYTES = 16384;          // K = 32 rows of a 256-wide weight matrix
-constexpr int CH_ACT_BYTES = 65536;           // one 128 x 256 bf16 tile
-
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-struct ChainLayer {
-  const uint8_t* B;        // packed weights [KC][N][8] bf16 (W for the forward chain, W^T for the dX chain)
-  const float* bias;       // forward: bias[0..n_bias) or NULL
-  uint8_t* out_packed;     // [tile][N/8][128][8] or NULL (not stored)
-  uint32_t* mask;          // forward: ReLU bit mask written (may be NULL); dX: ReLU bit mask read
-  int KC, N, n_bias, pad_;
-};
-struct ChainArgs {
-  const uint8_t* A0;       // packed input tiles, L[0].KC chunks each
-  int n_tiles, n_layers;
-  ChainLayer L[CH_MAX_LAYERS];
-  float* corr; int ldc;    // forward, last layer: fp32 rows (corr may be NULL)
-  const float* U_base; float* U_pred; int ldu; float scale; const float* scale_dev;
-  int n_rows, n_out, relu;
-  unsigned long long* trace;   // optional timing trace of CTA 0 (clock64 stamps), experiments only
-};
-enum ChainMode { MODE_CHAIN_FWD = 0, MODE_CHAIN_DX = 1 };
-
-template <int MODE>
-__global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_constant__ ChainArgs a) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  uint8_t* act0 = smem;
-  uint8_t* act1 = smem + CH_ACT_BYTES;
-  uint8_t* ring = smem + 2 * CH_ACT_BYTES;
-  float* bias_s = reinterpret_cast<float*>(ring + CH_STAGES * CH_SLAB_BYTES);          // [CH_MAX_LAYERS][256]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + CH_MAX_LAYERS * 256);
-  uint64_t* wfull = bars;                     // [CH_STAGES]
-  uint64_t* wempty = bars + CH_STAGES;        // [CH_STAGES]
-  uint64_t* in_full = wempty + CH_STAGES;     // input tiles of a pair have landed
-  uint64_t* acc_full = in_full + 1;           // all MMAs of one layer (both tiles) have retired
-  uint64_t* act_ready = acc_full + 1;         // all epilogue threads: next operand written, accumulators drained
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(act_ready + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int L = a.n_layers;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < CH_STAGES; ++s) { mbar_init(&wfull[s], 1); mbar_init(&wempty[s], 1); }
-    mbar_init(in_full, 1);
-    mbar_init(acc_full, 1);
-    mbar_init(act_ready, CH_THREADS - 64);
-    fence_barrier_init();
-  }
-  if (MODE == MODE_CHAIN_FWD) {
-    for (int i = threadIdx.x; i < L * 256; i += blockDim.x) {
-      const int l = i >> 8, c = i & 255;
-      bias_s[i] = (a.L[l].bias && c < a.L[l].n_bias) ? a.L[l].bias[c] : 0.f;
-    }
-  }
-  if (warp == 1) tmem_alloc(tmem_slot, TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int n_pairs = (a.n_tiles + 1) >> 1;
-  const uint32_t in_bytes = (uint32_t)a.L[0].KC * CHUNK_BYTES;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      int stage = 0; uint32_t phase = 0;
-      for (int pair = blockIdx.x; pair < n_pairs; pair += gridDim.x) {
-        for (int l = 0; l < L; ++l) {
-          const uint32_t slab_bytes = (uint32_t)a.L[l].N * 64u;
-          const int n_slabs = a.L[l].KC >> 2;
-          const uint8_t* src = a.L[l].B;
-          for (int s = 0; s < n_slabs; ++s) {
-            mbar_wait(&wempty[stage], phase ^ 1);
-            mbar_expect_tx(&wfull[stage], slab_bytes);
-            bulk_g2s(ring + stage * CH_SLAB_BYTES, src + (size_t)s * slab_bytes, slab_bytes, &wfull[stage]);
-            if (++stage == CH_STAGES) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      int stage = 0; uint32_t phase = 0;
-      uint32_t g = 0, pi = 0;
-      const uint32_t a0 = smem_u32(act0), a1 = smem_u32(act1);
-      for (int pair = blockIdx.x; pair < n_pairs; pair += gridDim.x, ++pi) {
-        const bool two = (2 * pair + 1) < a.n_tiles;
-        for (int l = 0; l < L; ++l, ++g) {
-          if (l == 0) mbar_wait(in_full, pi & 1);
-          if (g > 0) mbar_wait(act_ready, (g - 1) & 1);
-          tc_fence_after();
-          if (a.trace && blockIdx.x == 0 && g < 64) a.trace[g * 8 + 0] = clock64();      // operands ready
-          const int N = a.L[l].N;
-          const uint32_t idesc = make_idesc(TILE_M, N, false, false);
-          const uint32_t b_lbo = (uint32_t)N * 16;
-          const int n_slabs = a.L[l].KC >> 2;
-          for (int s = 0; s < n_slabs; ++s) {
-            mbar_wait(&wfull[stage], phase);
-            tc_fence_after();
-            const uint32_t b_base = smem_u32(ring + stage * CH_SLAB_BYTES);
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-              const uint64_t bdesc = make_desc(b_base + (uint32_t)(j * 2) * b_lbo, b_lbo, 128);
-              const uint32_t a_off = (uint32_t)(s * 4 + j * 2) * CHUNK_BYTES;
-              const uint32_t accum = (s | j) != 0 ? 1u : 0u;
-              umma_bf16(tmem_base, make_desc(a0 + a_off, CHUNK_BYTES, 128), bdesc, idesc, accum);
-              if (two) umma_bf16(tmem_base + 256u, make_desc(a1 + a_off, CHUNK_BYTES, 128), bdesc, idesc, accum);
-            }
-            umma_commit(&wempty[stage]);
-            if (++stage == CH_STAGES) { stage = 0; phase ^= 1; }
-          }
-          umma_commit(acc_full);
-          if (a.trace && blockIdx.x == 0 && g < 64) a.trace[g * 8 + 1] = clock64();      // all MMAs issued
-        }
-      }
-    }
-  } else {
-    // 16 epilogue warps: TMEM lane quadrant q = warp % 4, tile t, column half hf (column blocks 4 hf .. 4 hf + 3)
-    const int e = warp - 2;
-    const int q = warp & 3;
-    const int t = (e >> 2) & 1;
-    const int hf = (CH_CBW == 4) ? (e >> 3) : 0;
-    const int r = q * 32 + lane;
-    uint8_t* act = t ? act1 : act0;
-    const bool elected = (warp == 2 && lane == 0);
-    auto issue_input = [&](int pair) {
-      const int t0 = 2 * pair;
-      const bool two = (t0 + 1) < a.n_tiles;
-      mbar_expect_tx(in_full, two ? 2 * in_bytes : in_bytes);
-      bulk_g2s(act0, a.A0 + (size_t)t0 * in_bytes, in_bytes, in_full);
-      if (two) bulk_g2s(act1, a.A0 + (size_t)(t0 + 1) * in_bytes, in_bytes, in_full);
-    };
-    if (elected && (int)blockIdx.x < n_pairs) issue_input(blockIdx.x);
-    const float scale = (MODE == MODE_CHAIN_FWD && a.scale_dev) ? *a.scale_dev : a.scale;
-    const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)t * 256u + (uint32_t)hf * (CH_CBW * 32u);
-    const bool vec_out = ((a.ldc | a.ldu | a.n_out) & 3) == 0 &&
-                         ((reinterpret_cast<uintptr_t>(a.corr) | reinterpret_cast<uintptr_t>(a.U_base) |
-                           reinterpret_cast<uintptr_t>(a.U_pred)) & 15u) == 0;
-    uint32_t g = 0;
-    for (int pair = blockIdx.x; pair < n_pairs; pair += gridDim.x) {
-      const int tile = 2 * pair + t;
-      const bool valid = tile < a.n_tiles;            // warp-uniform
-      const long long row = (long long)tile * TILE_M + r;
-      for (int l = 0; l < L; ++l, ++g) {
-        // layer parameters into registers once (the parameter struct is indexed dynamically)
-        const int N = a.L[l].N, ncb = N >> 5;
-        const int my_cb = min(CH_CBW, ncb - CH_CBW * hf);   // column blocks of this warp (<= 0: none)
-        uint8_t* const out_packed = a.L[l].out_packed;
-        uint32_t* const mask_ptr = a.L[l].mask;
-        const float* bl = bias_s + l * 256 + hf * (CH_CBW * 32);
-        const bool last = (l == L - 1);
-        const bool work = valid && my_cb > 0;            // warp-uniform
-        uint32_t mw[CH_CBW];
-        float4 ub[8];
-        const bool final_rows = MODE == MODE_CHAIN_FWD && last && work && row < a.n_rows;
-        if (MODE == MODE_CHAIN_DX && work) {             // ReLU mask words of this row, fetched before the MMAs finish
-          const uint32_t* mrow = mask_ptr + (size_t)row * ncb + CH_CBW * hf;
-          if ((my_cb & 3) == 0) {
-#pragma unroll
-            for (int w4 = 0; w4 < CH_CBW / 4; ++w4) {
-              const uint4 m0 = 4 * w4 < my_cb ? __ldg(reinterpret_cast<const uint4*>(mrow) + w4) : make_uint4(0u, 0u, 0u, 0u);
-              mw[4 * w4] = m0.x; mw[4 * w4 + 1] = m0.y; mw[4 * w4 + 2] = m0.z; mw[4 * w4 + 3] = m0.w;
-            }
-          } else {
-#pragma unroll
-            for (int w = 0; w < CH_CBW; ++w) mw[w] = w < my_cb ? __ldg(mrow + w) : 0u;
-          }
-        }
-        if (final_rows && vec_out && a.U_pred) {         // first 32 columns of the U_base row: in flight during the MMAs
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            const int col = hf * (CH_CBW * 32) + 4 * j;
-            ub[j] = col < a.n_out ? __ldg(reinterpret_cast<const float4*>(a.U_base + (size_t)row * a.ldu + col))
-                                  : make_float4(0.f, 0.f, 0.f, 0.f);
-          }
-        }
-        mbar_wait(acc_full, g & 1);
-        tc_fence_after();
-        if (a.trace && blockIdx.x == 0 && g < 64 && threadIdx.x == 64) a.trace[g * 8 + 2] = clock64();   // accumulators ready
-        if (last && elected) {                         // operand buffers are free: fetch the next pair's input now
-          const int next = pair + (int)gridDim.x;
-          if (next < n_pairs) issue_input(next);
-        }
-        if (work) {
-          if (MODE == MODE_CHAIN_FWD && last) {
-            // fp32 rows: every thread owns one vertex row and writes whole 128-byte lines of it
-            const bool in_rows = row < a.n_rows;
-            for (int cb = 0; cb < my_cb; ++cb) {
-              const int col0 = hf * (CH_CBW * 32) + cb * 32;
-              if (cb > 0 && vec_out && in_rows && a.U_pred) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                  const int col = col0 + 4 * j;
-                  ub[j] = col < a.n_out ? __ldg(reinterpret_cast<const float4*>(a.U_base + (size_t)row * a.ldu + col))
-                                        : make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-              }
-              uint32_t v[32];
-              tmem_ld32(t_addr + cb * 32, v);
-              if (in_rows) {
-                if (vec_out) {
-#pragma unroll
-                  for (int j = 0; j < 8; ++j) {
-                    const int col = col0 + 4 * j;
-                    if (col < a.n_out) {
-                      const float4 bj = *reinterpret_cast<const float4*>(bl + cb * 32 + 4 * j);
-                      float4 c;
-                      c.x = __uint_as_float(v[4 * j]) + bj.x;     c.y = __uint_as_float(v[4 * j + 1]) + bj.y;
-                      c.z = __uint_as_float(v[4 * j + 2]) + bj.z; c.w = __uint_as_float(v[4 * j + 3]) + bj.w;
-                      if (a.corr) *reinterpret_cast<float4*>(a.corr + (size_t)row * a.ldc + col) = c;
-                      if (a.U_pred) {
-                        float4 u;
-                        u.x = __fadd_rn(ub[j].x, __fmul_rn(scale, c.x)); u.y = __fadd_rn(ub[j].y, __fmul_rn(scale, c.y));
-                        u.z = __fadd_rn(ub[j].z, __fmul_rn(scale, c.z)); u.w = __fadd_rn(ub[j].w, __fmul_rn(scale, c.w));
-                        *reinterpret_cast<float4*>(a.U_pred + (size_t)row * a.ldu + col) = u;
-                      }
-                    }
-                  }
-                } else {
-#pragma unroll
-                  for (int j = 0; j < 32; ++j) {
-                    const int col = col0 + j;
-                    if (col < a.n_out) {
-                      const float c = __uint_as_float(v[j]) + bl[cb * 32 + j];
-                      if (a.corr) a.corr[(size_t)row * a.ldc + col] = c;
-                      if (a.U_pred)
-                        a.U_pred[(size_t)row * a.ldu + col] =
-                            __fadd_rn(__ldg(a.U_base + (size_t)row * a.ldu + col), __fmul_rn(scale, c));
-                    }
-                  }
-                }
-              }
-            }
-          } else {
-            const size_t tile_off = (size_t)tile * (N >> 3) * CHUNK_BYTES + (size_t)r * 16;
-            const bool to_smem = !last;
-            uint32_t bits[CH_CBW];
-#pragma unroll
-            for (int cb = 0; cb < CH_CBW; ++cb) {
-              if (cb < my_cb) {
-                float4 b4[8];
-                if (MODE == MODE_CHAIN_FWD) {              // bias of these 32 columns: in flight with the TMEM load
-#pragma unroll
-                  for (int j = 0; j < 8; ++j) b4[j] = *reinterpret_cast<const float4*>(bl + cb * 32 + 4 * j);
-                }
-                uint32_t v[32];
-                tmem_ld32(t_addr + cb * 32, v);
-                uint32_t w[16];
-                if (MODE == MODE_CHAIN_FWD) bits[cb] = epi_block_fwd(v, b4, w);
-                else epi_block_dx(v, mw[cb], w);
-#pragma unroll
-                for (int g4 = 0; g4 < 4; ++g4) {
-                  const uint4 o = make_uint4(w[4 * g4], w[4 * g4 + 1], w[4 * g4 + 2], w[4 * g4 + 3]);
-                  const size_t c_off = (size_t)((hf * CH_CBW + cb) * 4 + g4) * CHUNK_BYTES;
-                  if (to_smem) *reinterpret_cast<uint4*>(act + c_off + (size_t)r * 16) = o;
-                  if (out_packed) *reinterpret_cast<uint4*>(out_packed + tile_off + c_off) = o;
-                }
-              } else if (MODE == MODE_CHAIN_FWD) {
-                bits[cb] = 0u;
-              }
-            }
-            if (MODE == MODE_CHAIN_FWD && mask_ptr) {      // this warp's four mask words of the row in one 16-byte store
-              uint32_t* mrow = mask_ptr + (size_t)row * ncb + CH_CBW * hf;
-              if ((my_cb & 3) == 0) {
-#pragma unroll
-                for (int w4 = 0; w4 < CH_CBW / 4; ++w4)
-                  if (4 * w4 < my_cb)
-                    reinterpret_cast<uint4*>(mrow)[w4] = make_uint4(bits[4 * w4], bits[4 * w4 + 1], bits[4 * w4 + 2], bits[4 * w4 + 3]);
-              } else {
-#pragma unroll
-                for (int cb = 0; cb < CH_CBW; ++cb) if (cb < my_cb) mrow[cb] = bits[cb];
-              }
-            }
-          }
-        }
-        if (a.trace && blockIdx.x == 0 && g < 64 && threadIdx.x == 64) a.trace[g * 8 + 3] = clock64();   // drained
-        if (!last) fence_proxy_async_smem();           // generic-proxy writes -> visible to the MMA (async proxy)
-        tc_fence_before();
-        mbar_arrive(act_ready);
-        if (a.trace && blockIdx.x == 0 && g < 64 && threadIdx.x == 64) a.trace[g * 8 + 4] = clock64();   // arrived
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, TMEM_COLS); }
-}
-
-// ------------------------------------------------------------------------------------------- layer chain, CTA pairs
-// tc_chain2_kernel: the same layer chain, run by CLUSTERS OF TWO CTAs with tcgen05.mma.cta_group::2.
-// What the single-CTA kernel cannot do is overlap the MMAs of one tile with the drain of another: both TMEM accumulators
-// and all shared memory that the weights leave belong to the tile pair in flight.  A CTA pair changes the budget:
+// Weights do not fit one SM (0.72 MB for 82->256x6->32), so they stream from L2 through a ring of K = 32 slabs.
+// Why CTA pairs: a single CTA that holds two tiles cannot overlap the MMAs of one tile with the drain of another, since
+// both TMEM accumulators and all shared memory that the weights leave belong to the tile pair in flight.  A CTA pair
+// changes the budget:
 //   * one MMA covers M = 256 rows, 128 from each CTA's operand tile, and the hardware takes HALF of the B operand from
 //     each CTA's shared memory: a CTA stores only its N/2 output columns of every weight slab (8 KB instead of 16 KB per
 //     K = 32), so a ring of 80 KB holds a whole layer (64 KB) and each CTA streams every layer ONCE per two tiles;
@@ -543,9 +243,9 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
 //   act_ready[u]  [512/-]    every epilogue thread of BOTH CTAs has drained its part of the accumulator and written +
 //                            fenced its part of the next operand (the peer's threads arrive remotely)
 // The peer forwards `landed` and `in_full` with one thread (warp 1, otherwise idle there).  Learned the hard
-// way (tools/chain2_check.py traces): (1) a remote arrive with .release.cluster semantics from the 256 epilogue threads
-// costs ~2000 clk per step - it waits for the thread's outstanding HBM stores; the default semantics do not, and the
-// operand tile is fenced into the async proxy before the arrive anyway; (2) every mbarrier try_wait in the
+// way (clock64 traces, tools/prof_chain.py): (1) a remote arrive with .release.cluster semantics from the 256 epilogue
+// threads costs ~2000 clk per step - it waits for the thread's outstanding HBM stores; the default semantics do not, and
+// the operand tile is fenced into the async proxy before the arrive anyway; (2) every mbarrier try_wait in the
 // MMA-issuing thread costs ~250 clk while the tensor pipe saturates shared memory, so a wait per weight slab (16 per
 // layer) starves the tensor pipe (360 instead of 130 clk per MMA) - hence one barrier per LAYER and merged counts: the
 // MMA thread waits for at most three barriers per (layer, slot) step and then issues 16 MMAs back to back.
@@ -553,12 +253,36 @@ __global__ void __launch_bounds__(CH_THREADS, 1) tc_chain_kernel(const __grid_co
 // a CTA's half of a slab is one contiguous bulk copy; three warps take turns issuing them (a thread sustains one
 // cp.async.bulk round per ~635 clk whatever its size, tools/micro/bulk_bw.cu).
 // Work: cluster c takes units c, c + n_clusters, ...; unit = tiles (2 unit, 2 unit + 1), one per CTA.
-// Measured (B200, 998,562 rows, 82->256x6->32): forward 0.99 ms against 1.08 ms for the single-CTA kernel, dZ chain
-// 0.76 against 0.80 ms, bit-identical outputs.  Per 256-wide layer and CTA (two tiles): ~7800 clk against 10100; the
-// tensor pipe is busy 34 % of the time (ncu, profiles/r02_ncu_chain2_summary.csv).  What bounds it now is the drain:
-// 2600-3500 clk per 128 x 256 tile whether 8 or 16 warps do it, with or without the TMEM load of the next block in
-// flight - the L1 / shared-memory data pipe carries 1400 wavefronts per tile for the epilogue (64 KB st.shared + 64 KB
-// st.global + bias reads) plus 1024 for the MMA operands of the other slot (69 % busy over the kernel).
+// Algorithmic HBM bytes per vertex (82->256x6->32): read 2*96, write 6*(2*256 + 32) + 2*4*32 -> 3.7 KB, against
+// 6.9 KB for the layer-by-layer kernels (every hidden activation is read back once).
+// Measured (B200, 998,562 rows, 82->256x6->32): 0.99 ms against 1.08 ms for a single-CTA chain over the same tile pairs,
+// bit-identical outputs.  Per 256-wide layer and CTA (two tiles): ~7800 clk against 10100; the tensor pipe is busy 34 %
+// of the time (ncu, profiles/r02_ncu_chain2_summary.csv).  What bounds it now is the drain: 2600-3500 clk per
+// 128 x 256 tile whether 8 or 16 warps do it, with or without the TMEM load of the next block in flight - the L1 /
+// shared-memory data pipe carries 1400 wavefronts per tile for the epilogue (64 KB st.shared + 64 KB st.global + bias
+// reads) plus 1024 for the MMA operands of the other slot (69 % busy over the kernel).
+constexpr int CH_MAX_LAYERS = 8;
+constexpr int CH_ACT_BYTES = 65536;           // one 128 x 256 bf16 tile
+
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+struct ChainLayer {
+  const uint8_t* B;        // packed weights [KC][N][8] bf16, followed by their "pair" copy
+  const float* bias;       // bias[0..n_bias) or NULL
+  uint8_t* out_packed;     // [tile][N/8][128][8] or NULL (not stored)
+  uint32_t* mask;          // ReLU bit mask written, or NULL (not stored)
+  int KC, N, n_bias, pad_;
+};
+struct ChainArgs {
+  const uint8_t* A0;       // packed input tiles, L[0].KC chunks each
+  int n_tiles, n_layers;
+  ChainLayer L[CH_MAX_LAYERS];
+  float* corr; int ldc;    // last layer: fp32 rows (corr may be NULL)
+  const float* U_base; float* U_pred; int ldu; float scale; const float* scale_dev;
+  int n_rows, n_out, relu;
+  unsigned long long* trace;   // optional timing trace of CTA 0 (clock64 stamps), experiments only
+};
+
 constexpr int C2_PRODUCERS = 3;               // weight-issuing warps: 0, 10, 11
 constexpr int C2_THREADS = 384;               // + warp 1: MMA issuer (leader) / forwarder (peer), warps 2..9: epilogue.
                                               // Twelve warps = three per scheduler = up to 168 registers; a 13th caps at 128.
@@ -599,7 +323,6 @@ __device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols));
 }
 
-template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C2_THREADS, 1)
 tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
   extern __shared__ __align__(128) uint8_t smem[];
@@ -629,11 +352,9 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
     }
     fence_barrier_init();
   }
-  if (MODE == MODE_CHAIN_FWD) {
-    for (int i = threadIdx.x; i < L * 256; i += blockDim.x) {
-      const int l = i >> 8, c = i & 255;
-      bias_s[i] = (a.L[l].bias && c < a.L[l].n_bias) ? a.L[l].bias[c] : 0.f;
-    }
+  for (int i = threadIdx.x; i < L * 256; i += blockDim.x) {
+    const int l = i >> 8, c = i & 255;
+    bias_s[i] = (a.L[l].bias && c < a.L[l].n_bias) ? a.L[l].bias[c] : 0.f;
   }
   if (warp == 1) tmem_alloc2(tmem_slot, TMEM_COLS);
   tc_fence_before();
@@ -758,7 +479,7 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
       }
     };
     if (elected) { if (my_units > 0) issue_input(0); if (my_units > 1) issue_input(1); }
-    const float scale = (MODE == MODE_CHAIN_FWD && a.scale_dev) ? *a.scale_dev : a.scale;
+    const float scale = a.scale_dev ? *a.scale_dev : a.scale;
     const bool vec_out = ((a.ldc | a.ldu | a.n_out) & 3) == 0 &&
                          ((reinterpret_cast<uintptr_t>(a.corr) | reinterpret_cast<uintptr_t>(a.U_base) |
                            reinterpret_cast<uintptr_t>(a.U_pred)) & 15u) == 0;
@@ -779,19 +500,8 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
           const long long row = (long long)tile * TILE_M + r;
           uint8_t* act = u ? act1 : act0;
           const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)u * 256u + (uint32_t)hf * 128u;
-          uint32_t mw[4];
           float4 ub[8];
-          if (MODE == MODE_CHAIN_DX && work) {
-            const uint32_t* mrow = mask_ptr + (size_t)row * ncb + 4 * hf;
-            if (my_cb == 4) {
-              const uint4 m0 = __ldg(reinterpret_cast<const uint4*>(mrow));
-              mw[0] = m0.x; mw[1] = m0.y; mw[2] = m0.z; mw[3] = m0.w;
-            } else {
-#pragma unroll
-              for (int w = 0; w < 4; ++w) mw[w] = w < my_cb ? __ldg(mrow + w) : 0u;
-            }
-          }
-          const bool final_rows = MODE == MODE_CHAIN_FWD && last && work && row < a.n_rows;
+          const bool final_rows = last && work && row < a.n_rows;
           if (final_rows && vec_out && a.U_pred) {
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
@@ -806,7 +516,7 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
           if (a.trace && blockIdx.x == 0 && tg < 64 && threadIdx.x == 64) a.trace[tg * 8 + 2] = clock64();   // accumulator ready
           if (last && elected && (j + u + 2) < my_units) issue_input(j + u + 2);     // slot u's operand tile is free
           if (work) {
-            if (MODE == MODE_CHAIN_FWD && last) {
+            if (last) {
               const bool in_rows = row < a.n_rows;
               for (int cb = 0; cb < my_cb; ++cb) {
                 const int col0 = hf * 128 + cb * 32;
@@ -867,8 +577,7 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
                   tmem_ld32_wait(v);
                   if (cb + 1 < my_cb) tmem_ld32_issue(t_addr + (cb + 1) * 32, (cb & 1) ? va : vb);
                   uint32_t w[16];
-                  if (MODE == MODE_CHAIN_FWD) bits[cb] = epi_block_fwd_sb(v, bl + cb * 32, w);
-                  else epi_block_dx(v, mw[cb], w);
+                  bits[cb] = epi_block_fwd_sb(v, bl + cb * 32, w);
 #pragma unroll
                   for (int g4 = 0; g4 < 4; ++g4) {
                     const uint4 o = make_uint4(w[4 * g4], w[4 * g4 + 1], w[4 * g4 + 2], w[4 * g4 + 3]);
@@ -876,11 +585,11 @@ tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
                     if (to_smem) *reinterpret_cast<uint4*>(act + c_off + (size_t)r * 16) = o;
                     if (out_packed) *reinterpret_cast<uint4*>(out_packed + tile_off + c_off) = o;
                   }
-                } else if (MODE == MODE_CHAIN_FWD) {
+                } else {
                   bits[cb] = 0u;
                 }
               }
-              if (MODE == MODE_CHAIN_FWD && mask_ptr) {
+              if (mask_ptr) {
                 uint32_t* mrow = mask_ptr + (size_t)row * ncb + 4 * hf;
                 if (my_cb == 4) {
                   *reinterpret_cast<uint4*>(mrow) = make_uint4(bits[0], bits[1], bits[2], bits[3]);
@@ -1211,38 +920,22 @@ int launch_linear(const LinearArgs& a, cudaStream_t st, int max_ctas = 0) {
 
 bool dims_ok(int kp, int np) { return kp % 32 == 0 && np % 32 == 0 && kp >= 32 && np >= 32 && kp <= 256 && np <= 256; }
 
-template <int MODE>
 int launch_chain(const ChainArgs& a, cudaStream_t st) {
-  const size_t smem = 2 * (size_t)CH_ACT_BYTES + (size_t)CH_STAGES * CH_SLAB_BYTES + sizeof(float) * CH_MAX_LAYERS * 256 +
-                      8 * (2 * CH_STAGES + 3) + 16 + 128;
+  // one cluster of two CTAs per unit of two tiles, at most one CTA per SM
+  const size_t smem = 2 * (size_t)CH_ACT_BYTES + (size_t)C2_STAGES * C2_SLOT_BYTES + sizeof(float) * CH_MAX_LAYERS * 256 +
+                      8 * C2_N_BARRIERS + 16 + 128;
   static bool configured = false;
   if (!configured) {
-    EP_CUDA_CHECK(cudaFuncSetAttribute(tc_chain_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    EP_CUDA_CHECK(cudaFuncSetAttribute(tc_chain2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
   const int n_pairs = (a.n_tiles + 1) / 2;
+  int clusters = ep::sm_count() / 2;
+  if (clusters > n_pairs) clusters = n_pairs;
   ChainArgs b = a;
-  if (ep::tune_flag(6) == 0) {
-    // default: CTA pairs (tcgen05 cta_group::2), one cluster of two per unit of two tiles
-    const size_t smem2 = 2 * (size_t)CH_ACT_BYTES + (size_t)C2_STAGES * C2_SLOT_BYTES + sizeof(float) * CH_MAX_LAYERS * 256 +
-                         8 * C2_N_BARRIERS + 16 + 128;
-    static bool configured2 = false;
-    if (!configured2) {
-      EP_CUDA_CHECK(cudaFuncSetAttribute(tc_chain2_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-      configured2 = true;
-    }
-    int clusters = ep::sm_count() / 2;
-    if (clusters > n_pairs) clusters = n_pairs;
-    b.trace = reinterpret_cast<unsigned long long*>(((uintptr_t)(uint32_t)ep::tune_flag(4) << 32) | (uint32_t)ep::tune_flag(3));
-    tc_chain2_kernel<MODE><<<2 * clusters, C2_THREADS, smem2, st>>>(b);
-    EP_LAUNCH_CHECK("tc_chain2_kernel");
-    return EP_OK;
-  }
   b.trace = reinterpret_cast<unsigned long long*>(((uintptr_t)(uint32_t)ep::tune_flag(4) << 32) | (uint32_t)ep::tune_flag(3));
-  int grid = ep::sm_count();
-  if (grid > n_pairs) grid = n_pairs;
-  tc_chain_kernel<MODE><<<grid, CH_THREADS, smem, st>>>(b);
-  EP_LAUNCH_CHECK("tc_chain_kernel");
+  tc_chain2_kernel<<<2 * clusters, C2_THREADS, smem, st>>>(b);
+  EP_LAUNCH_CHECK("tc_chain2_kernel");
   return EP_OK;
 }
 
@@ -1366,25 +1059,7 @@ int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, const int*
   }
   a.corr = corr; a.ldc = ldc; a.U_base = U_base; a.U_pred = U_pred; a.ldu = ldu; a.scale = scale; a.scale_dev = scale_dev;
   a.n_rows = n; a.n_out = k; a.relu = 1;
-  return launch_chain<MODE_CHAIN_FWD>(a, ep::as_stream(stream));
-}
-
-int ep_tc_chain_dx_bf16(int n, int n_layers, const int* dims_padded, const void* dZ_packed, const void* const* WTp,
-                        const void* const* relu_mask, void* const* dZ_out, ep_stream_t stream) {
-  EP_REQUIRE(n > 0 && dZ_packed && WTp && relu_mask && dZ_out, "bad argument");
-  if (int rc = chain_dims_ok("ep_tc_chain_dx_bf16", n_layers, dims_padded)) return rc;
-  ChainArgs a{};
-  a.A0 = static_cast<const uint8_t*>(dZ_packed);
-  a.n_tiles = n_tiles_for(n); a.n_layers = n_layers;
-  for (int l = 0; l < n_layers; ++l) {
-    EP_REQUIRE(WTp[l] && relu_mask[l] && dZ_out[l], "null pointer in a layer table");
-    a.L[l].B = static_cast<const uint8_t*>(WTp[l]);
-    a.L[l].KC = dims_padded[l] / 8; a.L[l].N = dims_padded[l + 1];
-    a.L[l].out_packed = static_cast<uint8_t*>(dZ_out[l]);
-    a.L[l].mask = const_cast<uint32_t*>(static_cast<const uint32_t*>(relu_mask[l]));
-  }
-  a.n_rows = n;
-  return launch_chain<MODE_CHAIN_DX>(a, ep::as_stream(stream));
+  return launch_chain(a, ep::as_stream(stream));
 }
 
 size_t ep_tc_dw_workspace_bytes(void) { return sizeof(float) * (size_t)ep::sm_count() * (256 * 256 + 256); }

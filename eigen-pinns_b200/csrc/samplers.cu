@@ -464,7 +464,7 @@ int ep_voxel_select_f64(int64_t n_points, const double* pts, const double* lo, d
   EP_REQUIRE(nb < 0x7fffffffLL, "voxel grid too large");
   voxel_init_kernel<<<stream_grid(n_vox, 256), 256, 0, st>>>(n_vox, tab_d, tab_i);
   EP_LAUNCH_CHECK("voxel_init_kernel");
-  if (n_vox <= kVoxelSmemMax && ep::tune_flag(9) == 0) {
+  if (n_vox <= kVoxelSmemMax) {
     int grid = 2 * ep::sm_count();
     const long long need = ep::ceil_div64(n_points, 256);
     if (need < grid) grid = (int)need;

@@ -197,7 +197,7 @@ extern "C" {
 
 int ep_tune_set(int key, int value) {
   if (key == 1 && value >= 1 && value <= 64) { g_spmm_waves = value; return EP_OK; }
-  if (key >= 2 && key < 16) { ep::set_tune_flag(key, value); return EP_OK; }
+  if (key == 3 || key == 4) { ep::set_tune_flag(key, value); return EP_OK; }
   ep::set_error("ep_tune_set: unknown key or bad value");
   return EP_ERR_INVALID;
 }

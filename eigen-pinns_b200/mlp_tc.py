@@ -1,7 +1,6 @@
 """bf16 tensor-core back end of the corrector MLP ("perf mode"): host-side buffer management around
 the tcgen05 kernels of csrc/mlp_tc.cu.  Same interface as engine.Fp32Mlp."""
 import ctypes
-import os
 
 import torch
 
@@ -34,7 +33,7 @@ def unpack_rows(packed, n, d_padded):
 
 
 def _table(values, ctype=ctypes.c_void_p):
-    """Host array for the layer tables of ep_tc_chain_* (device pointers or ints inside)."""
+    """Host array for the layer tables of ep_tc_chain_fwd_bf16 (device pointers or ints inside)."""
     arr = (ctype * len(values))()
     for i, v in enumerate(values):
         arr[i] = v if ctype is ctypes.c_int else (v.data_ptr() if v is not None else None)
@@ -42,19 +41,14 @@ def _table(values, ctype=ctypes.c_void_p):
 
 
 class TcMlp:
-    """Forward: ONE launch for all layers (ep_tc_chain_fwd_bf16) unless chain_fwd=False.  Backward: per layer the dW
-    kernel and the dX kernel run concurrently on half of the SMs each (default, measured fastest on B200: 1.93 ms vs
-    2.03 ms at 1 M vertices), or with chain_bwd=True one launch for the whole dZ chain (ep_tc_chain_dx_bf16, one gradient
-    buffer per layer) followed by one dW launch per layer.  All variants produce bit-identical results.
-    `chain=` sets both switches; the environment variables EP_TC_CHAIN_FWD / EP_TC_CHAIN_BWD (0 / 1) override."""
+    """Forward: ONE launch for all layers (ep_tc_chain_fwd_bf16, CTA pairs).  chain_fwd=False runs the layer-by-layer
+    kernels instead, the bit-exact reference the tests compare the chain against.  Backward, layer by layer from the
+    top: the dW kernel of layer l (side stream) and the dX kernel that produces dZ of layer l - 1 (main stream) run
+    concurrently on two disjoint shares of the SMs; layer 0 needs no dX, so its dW kernel takes the whole GPU."""
 
-    def __init__(self, n, params, device, h=None, chain=None, chain_fwd=None, chain_bwd=None):
+    def __init__(self, n, params, device, h=None, chain_fwd=True):
         self.p, self.n, self.dev = params, n, device
-        env = os.environ.get
-        self.chain_fwd = bool(chain if chain is not None else (chain_fwd if chain_fwd is not None
-                                                               else env("EP_TC_CHAIN_FWD", "1") == "1"))
-        self.chain_bwd = bool(chain if chain is not None else (chain_bwd if chain_bwd is not None
-                                                               else env("EP_TC_CHAIN_BWD", "0") == "1"))
+        self.chain_fwd = bool(chain_fwd)
         dims = params.dims                                    # [in, h1, ..., out]
         L = len(dims) - 1
         if L < 2:
@@ -71,11 +65,7 @@ class TcMlp:
         self.acts = [rows(self.pd[l + 1]) for l in range(L - 1)]             # outputs of hidden layers
         self.masks = [torch.zeros(query("ep_tc_relu_mask_bytes", n, self.pd[l + 1]), **u8) for l in range(L - 1)]
         wmax = max(self.pd[1:-1])
-        if self.chain_bwd:
-            self.dzs = [rows(self.pd[l + 1]) for l in range(L - 1)]          # gradient w.r.t. every hidden pre-activation
-            self.dz = None
-        else:
-            self.dz = [rows(wmax) for _ in range(2)]
+        self.dz = [rows(wmax) for _ in range(2)]
         self.dz_out = rows(self.pd[-1])
         self.Wp = [torch.zeros(query("ep_tc_packed_weight_bytes", self.pd[l + 1], self.pd[l]), **u8) for l in range(L)]
         self.WTp = [torch.zeros_like(w) for w in self.Wp]
@@ -84,8 +74,7 @@ class TcMlp:
         self.corr = torch.empty((n, dims[-1]), dtype=torch.float32, device=device)
         self.side_stream = torch.cuda.Stream(device=device)
         self.sm_count = torch.cuda.get_device_properties(device).multi_processor_count
-        self.overlap = True
-        self.dx_share = float(os.environ.get("EP_DX_SHARE", "0.56"))   # measured: tools/dx_share_sweep.py, backward 2.11 -> 1.93 ms vs an even split
+        self.dx_share = 0.56           # measured: tools/dx_share_sweep.py, backward 2.11 -> 1.93 ms vs an even split
         self._packed_version = None
         self.want_corr = True          # engine sets False: only U_pred is needed inside the training step
         if self.chain_fwd:
@@ -93,11 +82,6 @@ class TcMlp:
             self._t_out = _table(dims[1:], ctypes.c_int)
             self._t_Wp, self._t_b = _table(self.Wp), _table(list(self.p.b))
             self._t_acts, self._t_masks = _table(self.acts), _table(self.masks)
-        if self.chain_bwd:
-            self._t_bpd = _table(self.pd[::-1][:L], ctypes.c_int)           # pd[L], pd[L-1], ..., pd[1]
-            self._t_WT = _table([self.WTp[l] for l in range(L - 1, 0, -1)])
-            self._t_bmasks = _table([self.masks[l] for l in range(L - 2, -1, -1)])
-            self._t_dzs = _table([self.dzs[l] for l in range(L - 2, -1, -1)])
         if h is not None:
             self.input_changed(h)
 
@@ -141,18 +125,6 @@ class TcMlp:
         main = torch.cuda.current_stream()
         side = self.side_stream
         pack_rows(d_out, self.pd[-1], out=self.dz_out)
-        if self.chain_bwd:
-            if L > 1:
-                call("ep_tc_chain_dx_bf16", self.n, L - 1, self._t_bpd, _p(self.dz_out), self._t_WT, self._t_bmasks,
-                     self._t_dzs, _stream())
-            for l in range(L - 1, -1, -1):
-                dz, dz_w = (self.dz_out, self.pd[-1]) if l == L - 1 else (self.dzs[l], self.pd[l + 1])
-                act = self.acts[l - 1] if l > 0 else self.x0
-                call("ep_tc_linear_dw_bf16", self.n, self.dims[l + 1], self.dims[l], dz_w, self.pd[l], _p(dz), _p(act),
-                     _p(self.p.dW[l]), _p(self.p.db[l]), _p(self.ws), self.ws_bytes, 0, _stream())
-                if on_layer_grads is not None:
-                    on_layer_grads(l)
-            return
         dz, dz_w = self.dz_out, self.pd[-1]
         # SMs for the dX kernel / for the dW kernel of a concurrent pair (dX moves slightly more bytes and has the
         # heavier epilogue: an even split lets dW finish early and leaves dX alone on half of the machine)
@@ -160,21 +132,18 @@ class TcMlp:
         n_dw = self.sm_count - n_dx
         for l in range(L - 1, -1, -1):
             act = self.acts[l - 1] if l > 0 else self.x0
-            concurrent = self.overlap and l > 0
-            if concurrent:
+            if l > 0:
                 side.wait_stream(main)
                 with torch.cuda.stream(side):
                     call("ep_tc_linear_dw_bf16", self.n, self.dims[l + 1], self.dims[l], dz_w, self.pd[l], _p(dz), _p(act),
                          _p(self.p.dW[l]), _p(self.p.db[l]), _p(self.ws), self.ws_bytes, n_dw, _stream())
+                nxt = self.dz[l & 1]
+                call("ep_tc_linear_dx_bf16", self.n, dz_w, self.pd[l], _p(dz), _p(self.WTp[l]), _p(self.masks[l - 1]),
+                     _p(nxt), n_dx, _stream())
+                main.wait_stream(side)
+                dz, dz_w = nxt, self.pd[l]
             else:
                 call("ep_tc_linear_dw_bf16", self.n, self.dims[l + 1], self.dims[l], dz_w, self.pd[l], _p(dz), _p(act),
                      _p(self.p.dW[l]), _p(self.p.db[l]), _p(self.ws), self.ws_bytes, 0, _stream())
-            if l > 0:
-                nxt = self.dz[l & 1]
-                call("ep_tc_linear_dx_bf16", self.n, dz_w, self.pd[l], _p(dz), _p(self.WTp[l]), _p(self.masks[l - 1]),
-                     _p(nxt), n_dx if concurrent else 0, _stream())
-                if concurrent:
-                    main.wait_stream(side)
-                dz, dz_w = nxt, self.pd[l]
             if on_layer_grads is not None:
                 on_layer_grads(l)

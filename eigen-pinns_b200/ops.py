@@ -5,7 +5,6 @@ torch is only the allocator / stream / autograd plumbing.  CPU tensors are rejec
 no fallback path.
 """
 import ctypes
-import os
 
 import torch
 
@@ -185,12 +184,12 @@ def eigen_bwd_prepare(U, KU, MU, coef, KU_bar=None, MU_bar=None, D=None):
     return KU_bar, MU_bar, D
 
 
-# k x k term of the backward on the tensor cores (tcgen05 kind::tf32, 3 passes) instead of SIMT shuffles; EP_TC_GRAM=0
-# selects the one-kernel SIMT form
-TENSOR_CORE_GRAM = os.environ.get("EP_TC_GRAM", "1") == "1"
+# k x k term of the backward on the tensor cores (tcgen05 kind::tf32, 3 passes) instead of SIMT shuffles, for
+# k >= TENSOR_CORE_GRAM_MIN_K; below it the one-kernel SIMT form runs
+TENSOR_CORE_GRAM = True
 # measured on B200: at k = 32 the SIMT product hides behind the gather (0.45 vs 0.54 ms at 1 M vertices), at k = 64 the
 # tensor-core form wins (15.8 vs 16.4 ms at 16.7 M vertices; 21.6 ms before KU / MU were interleaved)
-TENSOR_CORE_GRAM_MIN_K = int(os.environ.get("EP_TC_GRAM_MIN_K", "64"))
+TENSOR_CORE_GRAM_MIN_K = 64
 
 
 def eigen_bwd_fused_ok(pair, k, *tensors):

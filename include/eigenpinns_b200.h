@@ -10,7 +10,7 @@
  * Conventions
  *   - plain pointers and sizes only; no torch / C++ types cross the boundary
  *   - all array pointers are DEVICE pointers unless the function name ends in _host; the tiny
- *     parameter arrays `dims`, `lo` (voxel grid) and the layer tables of ep_tc_chain_* are HOST arrays
+ *     parameter arrays `dims`, `lo` (voxel grid) and the layer tables of ep_tc_chain_fwd_bf16 are HOST arrays
  *   - one device and one stream per process are assumed by the cached launch configuration
  *     (SM count, opted-in shared-memory sizes, the gradient-norm scratch)
  *   - dense matrices are row-major with an explicit leading dimension (elements)
@@ -52,9 +52,10 @@ EP_API const char* ep_last_error_string(void);
 /* sm_count, compute capability of the current device; fails (EP_ERR_CUDA) without a GPU. */
 EP_API int ep_device_info(int* sm_count, int* cc_major, int* cc_minor);
 
-/* Tuning knobs for experiments (key 1: SpMM persistent grid = value full-machine waves, default 4;
- * key 2: 1 = k-32 register-resident variant of the fused backward, 0 = generic variant (default; measured
- * faster: both are instruction-issue bound, 0.29 ms vs 0.35 ms at 1 M vertices)). */
+/* Knobs for experiments.  Key 1: SpMM persistent grid = value full-machine waves (1..64, default 4).
+ * Keys 3 / 4: low / high 32 bits of the address of a device buffer of 64 x 8 uint64 (0 = off) that
+ * ep_tc_chain_fwd_bf16 fills with clock64 stamps of its first CTA, 8 per (layer, slot) step.  Any other key returns
+ * EP_ERR_INVALID. */
 EP_API int ep_tune_set(int key, int value);
 
 /* ---- sparse operators: torch.sparse.mm(K_t, U), torch.sparse.mm(M_t, U) ----------------
@@ -224,7 +225,7 @@ EP_API int ep_tc_pack_rows_bf16(int n, int d, int d_padded, const float* X, int 
                          ep_stream_t stream);
 /* W fp32 [out x in] (nn.Linear layout) -> Wp [in_p/8][out_p][8] and, if WTp != NULL, WTp [out_p/8][in_p][8].
  * Each buffer holds TWO copies (ep_tc_packed_weight_bytes accounts for both): the layout above, then the same matrix
- * as [K/32][half of N][4][N/2][8] - the order in which a CTA pair of the chain kernels (tcgen05 cta_group::2) streams
+ * as [K/32][half of N][4][N/2][8] - the order in which a CTA pair of the chain kernel (tcgen05 cta_group::2) streams
  * its half of every K = 32 slab with one contiguous bulk copy. */
 EP_API int ep_tc_pack_weight_bf16(int out, int in, int out_padded, int in_padded, const float* W, void* Wp,
                            void* WTp, ep_stream_t stream);
@@ -246,10 +247,13 @@ EP_API int ep_tc_linear_final_bf16(int n, int in_padded, int out, int out_padded
  * SMs each and the same tile order, so the dZ tiles one of them pulls from HBM are L2 hits for the other). */
 EP_API int ep_tc_linear_dx_bf16(int n, int out_padded, int in_padded, const void* dZ_packed, const void* WTp,
                          const void* relu_mask, void* dZprev_packed, int max_ctas, ep_stream_t stream);
-/* All layers in ONE launch ("fused MLP over vertex tiles", corrector_model.py:12-21,31): a persistent CTA takes two
- * 128-vertex tiles through every layer; the activation tile stays in shared memory between layers (the epilogue of
- * layer l writes the A operand of layer l+1 in place), weights stream from L2 in 16 KB K-slabs shared by both tiles.
- * Hidden activations and ReLU masks are still written to HBM (the backward needs them) but never read back.
+/* All layers in ONE launch ("fused MLP over vertex tiles", corrector_model.py:12-21,31), run by persistent clusters of
+ * two CTAs (tcgen05 cta_group::2): one MMA covers 256 vertices, 128 from each CTA, and each CTA keeps its own two tiles
+ * in ping-pong, so the tensor cores work on one tile while the epilogue drains the other.  An activation tile stays in
+ * shared memory between layers (the epilogue of layer l writes the A operand of layer l+1 in place); weights stream
+ * from L2 in K = 32 slabs, each CTA holding its half of the output columns (the second copy of ep_tc_pack_weight_bf16),
+ * so a cluster reads every layer once per four tiles.  Hidden activations and ReLU masks are still written to HBM (the
+ * backward needs them) but never read back.
  * Layer tables are HOST arrays of n_layers entries (device pointers inside): dims_padded[n_layers + 1] padded widths
  * (input first), dims_out[n_layers] true output widths (bias lengths; dims_out[n_layers-1] = k), Wp / bias per layer,
  * act_out / relu_mask_out per hidden layer (tables or entries may be NULL: not stored).  The last layer writes fp32
@@ -259,11 +263,6 @@ EP_API int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, con
                          const void* const* Wp, const float* const* bias, void* const* act_out,
                          void* const* relu_mask_out, float* corr, int ldc, const float* U_base, float scale,
                          const float* scale_dev, float* U_pred, int ldu, ep_stream_t stream);
-/* Gradient chain dZ_{L-1} -> dZ_{L-2} -> ... in one launch: layer j computes dZ_out[j] = (dZ_in W) * [act > 0] with
- * WTp[j] the packed transpose ([K/8][N][8], K = dims_padded[j], N = dims_padded[j+1]) and relu_mask[j] the bit mask the
- * forward wrote for the activation of width dims_padded[j+1].  Every dZ_out[j] is stored (the dW kernels read them). */
-EP_API int ep_tc_chain_dx_bf16(int n, int n_layers, const int* dims_padded, const void* dZ_packed, const void* const* WTp,
-                        const void* const* relu_mask, void* const* dZ_out, ep_stream_t stream);
 /* dW = dZ^T act (fp32 [out x in]) and db = column sums of dZ; deterministic two-stage reduction. */
 EP_API size_t ep_tc_dw_workspace_bytes(void);
 EP_API int ep_tc_linear_dw_bf16(int n, int out, int in, int out_padded, int in_padded, const void* dZ_packed,

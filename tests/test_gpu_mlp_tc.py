@@ -166,21 +166,15 @@ def test_bf16_training_tracks_reference():
                                     (128 * 149 * 2 + 5, [82, 256, 128, 256, 10]),
                                     (40000, [82, 256, 256, 256, 256, 256, 256, 32]),
                                     (128 * (74 * 6 + 37) + 77, [82, 256, 256, 256, 32])])
-@pytest.mark.parametrize("pair_kernel", [True, False])
-def test_chain_kernels_equal_layerwise(n, dims, pair_kernel):
-    """The fused all-layer kernels (ep_tc_chain_fwd_bf16 / ep_tc_chain_dx_bf16) must reproduce the layer-by-layer
-    kernels BIT FOR BIT: same bf16 roundings, same K order of the fp32 accumulation in TMEM.  Both implementations:
-    tc_chain2_kernel (CTA pairs, tcgen05 cta_group::2: the default) and tc_chain_kernel (one CTA per tile pair,
-    ep_tune_set(6, 1)).  Sizes cover one row, ragged tiles, an odd tile count (a pair whose second CTA has no tile), odd
-    unit counts per cluster (a ping-pong step with one slot), several steps per cluster, layers of one weight slab."""
-    pkg("_cabi").call("ep_tune_set", 6, 0 if pair_kernel else 1)
-    try:
-        _chain_equals_layerwise(n, dims)
-    finally:
-        pkg("_cabi").call("ep_tune_set", 6, 0)
-
-
-def _chain_equals_layerwise(n, dims):
+@pytest.mark.parametrize("corr_out", [True, False], ids=["corr", "U_pred_only"])
+def test_chain_kernels_equal_layerwise(n, dims, corr_out):
+    """The fused all-layer forward (ep_tc_chain_fwd_bf16: tc_chain2_kernel, CTA pairs with tcgen05 cta_group::2) must
+    reproduce the layer-by-layer kernels BIT FOR BIT: same bf16 roundings, same K order of the fp32 accumulation in
+    TMEM.  Compared: corr, U_pred, every hidden activation and ReLU mask, and the gradients of the backward that reads
+    them.  Sizes cover one row, ragged tiles, an odd tile count (a pair whose second CTA has no tile), odd unit counts
+    per cluster (a ping-pong step with one slot), several steps per cluster, layers of one weight slab.
+    corr_out=False is the configuration of the training step (want_corr = False): the chain writes U_pred only and
+    must leave corr untouched; the layer-by-layer reference always writes corr."""
     engine, tcm = pkg("engine"), pkg("mlp_tc")
     g = torch.Generator().manual_seed(n)
     Ws = [torch.randn(dims[i + 1], dims[i], generator=g) / np.sqrt(dims[i]) for i in range(len(dims) - 1)]
@@ -192,15 +186,20 @@ def _chain_equals_layerwise(n, dims):
     res = []
     for chain in (False, True):
         p = engine.FlatParams(Ws, bs, dev())
-        m = tcm.TcMlp(n, p, dev(), h, chain=chain)
-        m.overlap = False                       # same dW grid (all SMs) in both variants
+        m = tcm.TcMlp(n, p, dev(), h, chain_fwd=chain)
+        m.want_corr = corr_out
+        m.corr.fill_(float("nan"))
         up = torch.full_like(U, float("nan"))
         corr = m.forward(h, U, 0.25, up).clone()
         m.backward(h, d_out)
         torch.cuda.synchronize()
         res.append((corr, up, [a.clone() for a in m.acts], [a.clone() for a in m.masks], p.grad.clone()))
     (c0, u0, a0, m0, g0), (c1, u1, a1, m1, g1) = res
-    assert torch.equal(c0, c1) and torch.equal(u0, u1)
+    assert torch.equal(u0, u1) and torch.isfinite(u1).all()
+    if corr_out:
+        assert torch.equal(c0, c1)
+    else:
+        assert torch.isfinite(c0).all() and torch.isnan(c1).all()
     for x, y in zip(a0, a1):
         assert torch.equal(x, y)
     for x, y in zip(m0, m1):

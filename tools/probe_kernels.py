@@ -42,10 +42,8 @@ def main():
     print("partials (+reduce): %.4f ms, %.0f GB/s" % (ms, 12 * n * k / ms / 1e6))
     acc = torch.zeros(6, dtype=torch.float64, device=dev)
     lam, coef = ops.eigen_finalize(k, n, P, 1000.0, 10.0, acc)
-    for variant in (0, 1):
-        cabi.call("ep_tune_set", 2, variant)
-        ms = timeit(lambda: ops.eigen_bwd_fused(pair, KU, MU, coef, 1.0, dU))
-        print("fused bwd variant %d: %.4f ms, %.0f GB/s" % (variant, ms, nbytes / ms / 1e6))
+    ms = timeit(lambda: ops.eigen_bwd_fused(pair, KU, MU, coef, 1.0, dU))
+    print("fused bwd: %.4f ms, %.0f GB/s" % (ms, nbytes / ms / 1e6))
 
 
 if __name__ == "__main__":

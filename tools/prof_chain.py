@@ -1,4 +1,5 @@
-"""Times (CUDA events) the pieces of the tensor-core MLP at the benchmark size; used under ncu for the chain kernels.
+"""Times (CUDA events) the tensor-core MLP at the benchmark size: forward chain against layer-by-layer forward (same
+backward), the forward chain without its activation / mask copies, and the in-kernel clock64 trace of the chain.
     python tools/prof_chain.py [n] [k] [reps]"""
 import ctypes
 import importlib
@@ -31,7 +32,7 @@ def main():
     out = {}
     for chain in (True, False):
         p = engine.FlatParams(Ws, bs, dev)
-        m = tcm.TcMlp(n, p, dev, h, chain=chain)
+        m = tcm.TcMlp(n, p, dev, h, chain_fwd=chain)
         m.want_corr = False
         ev = lambda: torch.cuda.Event(enable_timing=True)
         for _ in range(2):
@@ -51,17 +52,10 @@ def main():
             tb += e1.elapsed_time(e2)
         out["chain" if chain else "layerwise"] = (tf / reps, tb / reps)
         if chain:
-            # the dZ chain alone and the seven dW launches alone
-            L = m.L
             P = lambda t: ctypes.c_void_p(t.data_ptr())
             st = lambda: ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-            e0.record()
-            for _ in range(reps):
-                cabi.call("ep_tc_chain_dx_bf16", m.n, L - 1, m._t_bpd, P(m.dz_out), m._t_WT, m._t_bmasks, m._t_dzs, st())
-            e1.record()
-            torch.cuda.synchronize()
-            out["dx_chain"] = e0.elapsed_time(e1) / reps
-            # in-kernel timeline of CTA 0 (clock64 stamps per layer): ep_tune_set keys 3 / 4 carry a device pointer
+            # in-kernel timeline of CTA 0 (clock64 stamps per (layer, slot) step): ep_tune_set keys 3 / 4 carry a device
+            # pointer
             trace = torch.zeros(64 * 8, dtype=torch.int64, device=dev)
             ptr = trace.data_ptr()
             cabi.call("ep_tune_set", 3, ctypes.c_int(ptr & 0xFFFFFFFF if (ptr & 0xFFFFFFFF) < 2**31 else (ptr & 0xFFFFFFFF) - 2**32))
@@ -72,12 +66,12 @@ def main():
             cabi.call("ep_tune_set", 4, 0)
             tr = trace.view(64, 8).cpu().numpy()
             t0 = tr[0, 0]
-            print("layer g: ready  issued  acc_full  drained  arrived   (clk since first; MMA issue, MMA tail, epilogue, handoff)")
-            for gi in range(21):
+            print("step (layer, slot): ready issued acc_full drained arrived  (clk since first)")
+            for gi in range(30):
                 r = tr[gi] - t0
-                nxt = tr[gi + 1, 0] - t0
-                print("%2d: %7d %7d %7d %7d %7d   issue %5d tail %5d epi %5d fence %4d handoff %5d" % (
-                    gi, r[0], r[1], r[2], r[3], r[4], r[1] - r[0], r[2] - r[1], r[3] - r[2], r[4] - r[3], nxt - r[4]))
+                print("%2d (l%d u%d): %7d %7d %7d %7d %7d   issue %5d tail %5d epi %5d arrive %4d" % (
+                    gi, (gi // 2) % m.L, gi % 2, r[0], r[1], r[2], r[3], r[4], r[1] - r[0], r[2] - r[1], r[3] - r[2],
+                    r[4] - r[3]))
             # experiment: the forward chain without the HBM copies of activations / masks (not a product path)
             for label, acts_t, masks_t in (("fwd_no_act_no_mask", None, None), ("fwd_no_mask", m._t_acts, None),
                                            ("fwd_no_act", None, m._t_masks)):
