@@ -23,11 +23,16 @@ SIGNATURES = {
     "ep_spmm2_csr_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_p, c_int, c_p]),
     "ep_spmm2_sum_csr_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_int, c_f, c_p,
                                      c_p, c_int, c_p]),
+    "ep_spmm_csr_f64": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p, c_int, c_p]),
+    "ep_spmm2_csr_f64": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_p, c_int, c_p]),
+    "ep_spmm2_sum_csr_f64": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_int, c_d, c_p,
+                                     c_p, c_int, c_p]),
     "ep_neighbor_mean_concat_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_int, c_p, c_int, c_p]),
     "ep_spmm_concat_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p, c_int, c_p]),
     "ep_eigen_partials_len": (c_sz, [c_int]),
     "ep_eigen_partials_workspace_bytes": (c_sz, [c_int]),
     "ep_eigen_partials_f32": (c_int, [c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_p, c_sz, c_p]),
+    "ep_eigen_partials_f64": (c_int, [c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_p, c_sz, c_p]),
     "ep_eigen_coef_len": (c_sz, [c_int]),
     "ep_eigen_finalize_f32": (c_int, [c_int, c_d, c_p, c_f, c_f, c_int, c_p, c_f, c_f, c_f, c_f, c_f, c_p, c_p, c_p, c_p,
                                       c_p]),
@@ -44,6 +49,10 @@ SIGNATURES = {
     "ep_linear_fwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_int, c_p]),
     "ep_linear_bwd_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
     "ep_linear_bwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_int, c_int,
+                                  c_p, c_p, c_p, c_sz, c_p]),
+    "ep_linear_fwd_f64": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_int, c_p]),
+    "ep_linear_bwd_workspace_bytes_f64": (c_sz, [c_int, c_int, c_int]),
+    "ep_linear_bwd_f64": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_int, c_int,
                                   c_p, c_p, c_p, c_sz, c_p]),
     "ep_tc_pad_features": (c_int, [c_int, c_int]),
     "ep_tc_packed_rows_bytes": (c_sz, [c_int, c_int]),
@@ -97,6 +106,8 @@ KERNELS_PER_CALL = {
     "ep_tc_pack_rows_bf16": 1, "ep_tc_pack_weight_bf16": 1, "ep_tc_linear_fwd_bf16": 1, "ep_tc_linear_final_bf16": 1,
     "ep_tc_linear_dx_bf16": 1, "ep_tc_linear_dw_bf16": 2, "ep_tc_chain_fwd_bf16": 1,
     "ep_halo_exchange_f32": 1,
+    "ep_spmm_csr_f64": 1, "ep_spmm2_csr_f64": 1, "ep_spmm2_sum_csr_f64": 1, "ep_eigen_partials_f64": 2,
+    "ep_linear_fwd_f64": 1, "ep_linear_bwd_f64": 5,
 }
 launch_counter = 0
 launch_by_entry = {}          # entry point -> kernels launched through it (bench.py reports the per-step table)

@@ -31,7 +31,7 @@ void set_tune_flag(int key, int value) { if (key >= 0 && key < 16) g_tune[key] =
 
 extern "C" {
 
-int ep_version(void) { return 10000 * 0 + 100 * 2 + 0; }
+int ep_version(void) { return 10000 * 0 + 100 * 3 + 0; }
 
 const char* ep_last_error_string(void) { return ep::g_err; }
 

@@ -1,7 +1,8 @@
 // Eigen-loss kernels: Rayleigh quotient, residual, Gram / orthonormality (forward partials,
 // finalisation, analytic backward).  Reference arithmetic: src/multigrid_model.py:291-348.
 //
-// Data layout: U, KU, MU are row-major n x k fp32 in HBM.  The four column sums behind the Rayleigh
+// Data layout: U, KU, MU are row-major n x k fp32 in HBM (the partials kernel also takes fp64 for the notebook
+// variants).  The four column sums behind the Rayleigh
 // quotient and the one-pass residual expansion sum(KU^2) - 2 lam sum(KU MU) + lam^2 sum(MU^2) are
 // accumulated in fp64 from the first product on (exact products, ~1e-16 relative sums), so the
 // expansion stays accurate near convergence where the residual is a tiny difference of large terms.
@@ -16,6 +17,30 @@ __device__ __forceinline__ bool ep_aligned16(const void* p) { return (reinterpre
 
 __host__ __device__ inline int partials_len(int k) { return k * k + 5 * k; }   // G | num | sKK | sKM | sMM | colsum(MU)
 
+// rows per tile of the partials kernel: the three R x KP tiles take at most 24 KB of static shared memory
+// (fp32: R = 32, 16 at KP = 128; fp64: R = 32, 32, 16, 8 for KP = 16 ... 128)
+template <typename T>
+__host__ __device__ constexpr int partial_rows(int kp) {
+  return 8192 / (kp * (int)sizeof(T)) < 32 ? 8192 / (kp * (int)sizeof(T)) : 32;
+}
+
+// 16-byte vector of the partials kernel's input type (global loads and shared-memory reads)
+template <typename T> struct Vec16;
+template <> struct Vec16<float> {
+  using type = float4;
+  static constexpr int N = 4;
+  __device__ static float4 zero() { return make_float4(0.f, 0.f, 0.f, 0.f); }
+  __device__ static float4 make(const float (&t)[4]) { return make_float4(t[0], t[1], t[2], t[3]); }
+  __device__ static void split(float4 v, float* t) { t[0] = v.x; t[1] = v.y; t[2] = v.z; t[3] = v.w; }
+};
+template <> struct Vec16<double> {
+  using type = double2;
+  static constexpr int N = 2;
+  __device__ static double2 zero() { return make_double2(0.0, 0.0); }
+  __device__ static double2 make(const double (&t)[2]) { return make_double2(t[0], t[1]); }
+  __device__ static void split(double2 v, double* t) { t[0] = v.x; t[1] = v.y; }
+};
+
 inline int partial_blocks(int n, int rows_per_tile) {
   int tiles = ep::ceil_div(n, rows_per_tile);
   int cap = ep::sm_count() * 4;
@@ -26,20 +51,24 @@ inline int partial_blocks(int n, int rows_per_tile) {
 // Gram / column-sum partials.  KP = padded column count; each thread owns a TG x TG block of the Gram
 // matrix, (KP/TG)^2 threads form a sub-group and the 256 / (KP/TG)^2 sub-groups take alternate rows of the
 // tile, so every FMA group costs two 16-byte shared-memory reads (TG = 4: 16 FMA per 2 LDS.128).
-template <int KP, int TG>
+// T = double (the notebook variants) accumulates the Gram matrix straight in fp64: there is no fp32 stage to fold.
+template <typename T, int KP, int TG>
 __global__ void __launch_bounds__(kPartialThreads)
-eigen_partials_kernel(int n, int k, const float* __restrict__ U, int ldu, const float* __restrict__ KU,
-                      const float* __restrict__ MU, int ld, double* __restrict__ block_out) {
+eigen_partials_kernel(int n, int k, const T* __restrict__ U, int ldu, const T* __restrict__ KU,
+                      const T* __restrict__ MU, int ld, double* __restrict__ block_out) {
   constexpr int TPD = KP / TG;
   constexpr int NT = TPD * TPD;
   constexpr int NSG = kPartialThreads / NT;
-  constexpr int R = (KP == 128) ? 16 : 32;
+  constexpr int R = partial_rows<T>(KP);
   constexpr int CPL = (KP + 31) / 32;
+  constexpr bool kFold = sizeof(T) == 4;          // fp32 input: fp32 Gram tiles folded into fp64
   constexpr int FLUSH = 4;                       // fold fp32 -> fp64 every FLUSH tiles
   static_assert(NT * NSG == kPartialThreads && NSG >= 1, "bad tiling");
-  __shared__ __align__(16) float Us[R][KP];
-  __shared__ __align__(16) float KUs[R][KP];
-  __shared__ __align__(16) float MUs[R][KP];
+  __shared__ __align__(16) T Us[R][KP];
+  __shared__ __align__(16) T KUs[R][KP];
+  __shared__ __align__(16) T MUs[R][KP];
+  using V = typename Vec16<T>::type;
+  constexpr int VW = Vec16<T>::N;
   __shared__ double red[(NSG > 1) ? KP * KP : 8 * KP];
 
   const int tid = threadIdx.x;
@@ -62,34 +91,34 @@ eigen_partials_kernel(int n, int k, const float* __restrict__ U, int ldu, const 
   const int n_tiles = (n + R - 1) / R;
   int since_flush = 0;
   // Register-staged double buffering: the next tile's global loads are in flight while this tile is reduced.
-  constexpr int VPT = (R * KP / 4 + kPartialThreads - 1) / kPartialThreads;     // float4 per thread per array
-  const bool vec_ok = (k % 4 == 0) && (ldu % 4 == 0) && (ld % 4 == 0) && ep_aligned16(U) && ep_aligned16(KU) && ep_aligned16(MU);
-  float4 pu[VPT], pk[VPT], pm[VPT];
+  constexpr int VPT = (R * KP / VW + kPartialThreads - 1) / kPartialThreads;     // 16-byte vectors per thread per array
+  const bool vec_ok = (k % VW == 0) && (ldu % VW == 0) && (ld % VW == 0) && ep_aligned16(U) && ep_aligned16(KU) && ep_aligned16(MU);
+  V pu[VPT], pk[VPT], pm[VPT];
   auto prefetch = [&](int tile) {
     const int row0 = tile * R;
 #pragma unroll
     for (int v = 0; v < VPT; ++v) {
-      const int e4 = tid + v * kPartialThreads;          // float4 index inside the R x KP tile
-      const int r = e4 / (KP / 4), c = (e4 - r * (KP / 4)) * 4;
+      const int e4 = tid + v * kPartialThreads;          // vector index inside the R x KP tile
+      const int r = e4 / (KP / VW), c = (e4 - r * (KP / VW)) * VW;
       const int row = row0 + r;
-      float4 zu = make_float4(0.f, 0.f, 0.f, 0.f), zk = zu, zm = zu;
+      V zu = Vec16<T>::zero(), zk = zu, zm = zu;
       if (r < R && row < n && c < k) {
         if (vec_ok) {
-          zu = __ldg(reinterpret_cast<const float4*>(U + (size_t)row * ldu + c));
-          zk = __ldg(reinterpret_cast<const float4*>(KU + (size_t)row * ld + c));
-          zm = __ldg(reinterpret_cast<const float4*>(MU + (size_t)row * ld + c));
+          zu = __ldg(reinterpret_cast<const V*>(U + (size_t)row * ldu + c));
+          zk = __ldg(reinterpret_cast<const V*>(KU + (size_t)row * ld + c));
+          zm = __ldg(reinterpret_cast<const V*>(MU + (size_t)row * ld + c));
         } else {
-          float tu[4], tk[4], tm[4];
+          T tu[VW], tk[VW], tm[VW];
 #pragma unroll
-          for (int j = 0; j < 4; ++j) {
+          for (int j = 0; j < VW; ++j) {
             const bool ok = (c + j) < k;
-            tu[j] = ok ? __ldg(U + (size_t)row * ldu + c + j) : 0.f;
-            tk[j] = ok ? __ldg(KU + (size_t)row * ld + c + j) : 0.f;
-            tm[j] = ok ? __ldg(MU + (size_t)row * ld + c + j) : 0.f;
+            tu[j] = ok ? __ldg(U + (size_t)row * ldu + c + j) : T(0);
+            tk[j] = ok ? __ldg(KU + (size_t)row * ld + c + j) : T(0);
+            tm[j] = ok ? __ldg(MU + (size_t)row * ld + c + j) : T(0);
           }
-          zu = make_float4(tu[0], tu[1], tu[2], tu[3]);
-          zk = make_float4(tk[0], tk[1], tk[2], tk[3]);
-          zm = make_float4(tm[0], tm[1], tm[2], tm[3]);
+          zu = Vec16<T>::make(tu);
+          zk = Vec16<T>::make(tk);
+          zm = Vec16<T>::make(tm);
         }
       }
       pu[v] = zu; pk[v] = zk; pm[v] = zm;
@@ -101,31 +130,32 @@ eigen_partials_kernel(int n, int k, const float* __restrict__ U, int ldu, const 
 #pragma unroll
     for (int v = 0; v < VPT; ++v) {
       const int e4 = tid + v * kPartialThreads;
-      const int r = e4 / (KP / 4), c = (e4 - r * (KP / 4)) * 4;
+      const int r = e4 / (KP / VW), c = (e4 - r * (KP / VW)) * VW;
       if (r < R) {
-        *reinterpret_cast<float4*>(&Us[r][c]) = pu[v];
-        *reinterpret_cast<float4*>(&KUs[r][c]) = pk[v];
-        *reinterpret_cast<float4*>(&MUs[r][c]) = pm[v];
+        *reinterpret_cast<V*>(&Us[r][c]) = pu[v];
+        *reinterpret_cast<V*>(&KUs[r][c]) = pk[v];
+        *reinterpret_cast<V*>(&MUs[r][c]) = pm[v];
       }
     }
     __syncthreads();
     if (tile + (int)gridDim.x < n_tiles) prefetch(tile + gridDim.x);
 #pragma unroll 2
     for (int r = sg; r < R; r += NSG) {
-      float a[TG], b[TG];
+      T a[TG], b[TG];
 #pragma unroll
-      for (int i = 0; i < TG; i += 4) {
-        const float4 t = *reinterpret_cast<const float4*>(&Us[r][ty * TG + i]);
-        a[i] = t.x; a[i + 1] = t.y; a[i + 2] = t.z; a[i + 3] = t.w;
-        const float4 u = *reinterpret_cast<const float4*>(&MUs[r][tx * TG + i]);
-        b[i] = u.x; b[i + 1] = u.y; b[i + 2] = u.z; b[i + 3] = u.w;
+      for (int i = 0; i < TG; i += VW) {
+        Vec16<T>::split(*reinterpret_cast<const V*>(&Us[r][ty * TG + i]), a + i);
+        Vec16<T>::split(*reinterpret_cast<const V*>(&MUs[r][tx * TG + i]), b + i);
       }
 #pragma unroll
       for (int i = 0; i < TG; ++i)
 #pragma unroll
-        for (int j = 0; j < TG; ++j) g32[i][j] = fmaf(a[i], b[j], g32[i][j]);
+        for (int j = 0; j < TG; ++j) {
+          if constexpr (kFold) g32[i][j] = fmaf(a[i], b[j], g32[i][j]);
+          else                 g64[i][j] = fma(a[i], b[j], g64[i][j]);
+        }
     }
-    if (++since_flush == FLUSH) {
+    if (kFold && ++since_flush == FLUSH) {
       since_flush = 0;
 #pragma unroll
       for (int i = 0; i < TG; ++i)
@@ -157,7 +187,8 @@ eigen_partials_kernel(int n, int k, const float* __restrict__ U, int ldu, const 
 #pragma unroll
   for (int i = 0; i < TG; ++i)
 #pragma unroll
-    for (int j = 0; j < TG; ++j) g64[i][j] += (double)g32[i][j];
+    for (int j = 0; j < TG; ++j)
+      if (kFold) g64[i][j] += (double)g32[i][j];
 
   double* out = block_out + (size_t)blockIdx.x * partials_len(k);
   if (NSG > 1) {                                  // combine the row sub-groups in a fixed order
@@ -632,11 +663,36 @@ int ep_eigen_partials_f32(int n, int k, const float* U, int ldu, const float* KU
     return EP_ERR_WORKSPACE;
   }
   double* blocks = static_cast<double*>(workspace);
-  if (k <= 16)      eigen_partials_kernel<16, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
-  else if (k <= 32) eigen_partials_kernel<32, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
-  else if (k <= 64) eigen_partials_kernel<64, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
-  else              eigen_partials_kernel<128, 8><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  if (k <= 16)      eigen_partials_kernel<float, 16, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else if (k <= 32) eigen_partials_kernel<float, 32, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else if (k <= 64) eigen_partials_kernel<float, 64, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else              eigen_partials_kernel<float, 128, 8><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
   EP_LAUNCH_CHECK("eigen_partials_kernel");
+  reduce_partials_kernel<<<ep::ceil_div(len, 8), 256, 0, st>>>(grid, len, blocks, out);
+  EP_LAUNCH_CHECK("reduce_partials_kernel");
+  return EP_OK;
+}
+
+int ep_eigen_partials_f64(int n, int k, const double* U, int ldu, const double* KU, const double* MU, int ld,
+                          double* out, void* workspace, size_t workspace_bytes, ep_stream_t stream) {
+  EP_REQUIRE(n >= 0 && k > 0, "bad size");
+  EP_REQUIRE(k <= 128, "k > 128 not instantiated");
+  EP_REQUIRE(out && workspace && (n == 0 || (U && KU && MU)), "null pointer");
+  EP_REQUIRE(ldu >= k && ld >= k, "leading dimension < k");
+  cudaStream_t st = ep::as_stream(stream);
+  const int len = partials_len(k);
+  const int rows = partial_rows<double>(k <= 16 ? 16 : k <= 32 ? 32 : k <= 64 ? 64 : 128);
+  const int grid = partial_blocks(n, rows);           // <= 4 blocks per SM, as in fp32: same workspace size
+  if (workspace_bytes < sizeof(double) * (size_t)len * grid) {
+    ep::set_error("ep_eigen_partials_f64: workspace too small");
+    return EP_ERR_WORKSPACE;
+  }
+  double* blocks = static_cast<double*>(workspace);
+  if (k <= 16)      eigen_partials_kernel<double, 16, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else if (k <= 32) eigen_partials_kernel<double, 32, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else if (k <= 64) eigen_partials_kernel<double, 64, 4><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  else              eigen_partials_kernel<double, 128, 8><<<grid, kPartialThreads, 0, st>>>(n, k, U, ldu, KU, MU, ld, blocks);
+  EP_LAUNCH_CHECK("eigen_partials_kernel<double>");
   reduce_partials_kernel<<<ep::ceil_div(len, 8), 256, 0, st>>>(grid, len, blocks, out);
   EP_LAUNCH_CHECK("reduce_partials_kernel");
   return EP_OK;

@@ -1,30 +1,35 @@
 // CSR SpMM family for the stiffness / mass operators (HBM-bound gather kernels).
 //
-// Layout: A is CSR (int32 rowptr/col, fp32 val), X / Y are row-major n x k fp32.  A "row
-// group" of LPR lanes owns one output row; every lane owns V consecutive columns (V = 4 when
-// k, the leading dimensions and the base pointers allow 16-byte accesses), so one gathered
-// row of X is read with LPR coalesced 16-byte loads (k = 32 -> 8 lanes x 16 B = one 128-byte
-// line).  With ~7 non-zeros per FEM row the non-zero loop is unrolled by 4 so that four
+// Layout: A is CSR (int32 rowptr/col, fp32 or fp64 val), X / Y are row-major n x k of the same
+// scalar type.  A "row group" of LPR lanes owns one output row; every lane owns V consecutive
+// columns (V = 4 floats or 2 doubles when k, the leading dimensions and the base pointers allow
+// 16-byte accesses), so one gathered row of X is read with LPR coalesced 16-byte loads (k = 32
+// fp32 -> 8 lanes x 16 B = one 128-byte line; fp64 -> 16 lanes x 16 B = two lines).  With ~7 non-zeros per FEM row the non-zero loop is unrolled by 4 so that four
 // gathers are in flight per lane before the first FMA.
 //
 // Algorithmic traffic (SURVEY 8d): single  8 nnz + 4 (n+1) + 8 n k   bytes
 //                                  dual   12 nnz + 4 (n+1) + 12 n k  (both products)
 //                                  sum    12 nnz + 4 (n+1) + 16 n k  (+4 n k when D given)
+// fp64 (the notebook variants): 8-byte values and rows, e.g. dual 20 nnz + 4 (n+1) + 24 n k.
 #include "ep_common.cuh"
 
 namespace {
 
 int g_spmm_waves = 4;      // persistent grid = this many full-machine waves (measured best on B200; tunable: ep_tune_set)
 
-template <int V> struct VecT;
-template <> struct VecT<1> { using type = float; };
-template <> struct VecT<2> { using type = float2; };
-template <> struct VecT<4> { using type = float4; };
+template <typename S, int V> struct VecT;
+template <> struct VecT<float, 1> { using type = float; };
+template <> struct VecT<float, 2> { using type = float2; };
+template <> struct VecT<float, 4> { using type = float4; };
+template <> struct VecT<double, 1> { using type = double; };
+template <> struct VecT<double, 2> { using type = double2; };
 
-template <int V> __device__ __forceinline__ typename VecT<V>::type vzero();
-template <> __device__ __forceinline__ float vzero<1>() { return 0.f; }
-template <> __device__ __forceinline__ float2 vzero<2>() { return make_float2(0.f, 0.f); }
-template <> __device__ __forceinline__ float4 vzero<4>() { return make_float4(0.f, 0.f, 0.f, 0.f); }
+template <typename T> __device__ __forceinline__ T vzero();
+template <> __device__ __forceinline__ float vzero<float>() { return 0.f; }
+template <> __device__ __forceinline__ float2 vzero<float2>() { return make_float2(0.f, 0.f); }
+template <> __device__ __forceinline__ float4 vzero<float4>() { return make_float4(0.f, 0.f, 0.f, 0.f); }
+template <> __device__ __forceinline__ double vzero<double>() { return 0.0; }
+template <> __device__ __forceinline__ double2 vzero<double2>() { return make_double2(0.0, 0.0); }
 
 __device__ __forceinline__ void vfma(float a, float x, float& acc) { acc = fmaf(a, x, acc); }
 __device__ __forceinline__ void vfma(float a, float2 x, float2& acc) {
@@ -34,28 +39,36 @@ __device__ __forceinline__ void vfma(float a, float4 x, float4& acc) {
   acc.x = fmaf(a, x.x, acc.x); acc.y = fmaf(a, x.y, acc.y);
   acc.z = fmaf(a, x.z, acc.z); acc.w = fmaf(a, x.w, acc.w);
 }
+__device__ __forceinline__ void vfma(double a, double x, double& acc) { acc = fma(a, x, acc); }
+__device__ __forceinline__ void vfma(double a, double2 x, double2& acc) {
+  acc.x = fma(a, x.x, acc.x); acc.y = fma(a, x.y, acc.y);
+}
 __device__ __forceinline__ float vadd(float a, float b) { return a + b; }
 __device__ __forceinline__ float2 vadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
 __device__ __forceinline__ float4 vadd(float4 a, float4 b) {
   return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w);
 }
+__device__ __forceinline__ double vadd(double a, double b) { return a + b; }
+__device__ __forceinline__ double2 vadd(double2 a, double2 b) { return make_double2(a.x + b.x, a.y + b.y); }
 __device__ __forceinline__ float vscale(float a, float s) { return a * s; }
 __device__ __forceinline__ float2 vscale(float2 a, float s) { return make_float2(a.x * s, a.y * s); }
 __device__ __forceinline__ float4 vscale(float4 a, float s) {
   return make_float4(a.x * s, a.y * s, a.z * s, a.w * s);
 }
+__device__ __forceinline__ double vscale(double a, double s) { return a * s; }
+__device__ __forceinline__ double2 vscale(double2 a, double s) { return make_double2(a.x * s, a.y * s); }
 
 // MODE 0: YA = A XA            MODE 1: YA = A XA, YB = B XA
 // MODE 2: YA = s (A XA + B XB + D)
-template <int V, int MODE>
+template <typename S, int V, int MODE>
 __global__ void __launch_bounds__(256)
 spmm_kernel(int n_rows, int kv, int lpr_shift, const int32_t* __restrict__ rowptr,
-            const int32_t* __restrict__ col, const float* __restrict__ valA,
-            const float* __restrict__ valB, const float* __restrict__ XA,
-            const float* __restrict__ XB, int ldx, const float* __restrict__ D, int ldd,
-            float out_scale, const float* __restrict__ out_scale_dev, float* __restrict__ YA,
-            float* __restrict__ YB, int ldy) {
-  using T = typename VecT<V>::type;
+            const int32_t* __restrict__ col, const S* __restrict__ valA,
+            const S* __restrict__ valB, const S* __restrict__ XA,
+            const S* __restrict__ XB, int ldx, const S* __restrict__ D, int ldd,
+            S out_scale, const S* __restrict__ out_scale_dev, S* __restrict__ YA,
+            S* __restrict__ YB, int ldy) {
+  using T = typename VecT<S, V>::type;
   const int lpr = 1 << lpr_shift;
   const int lane = (int)(threadIdx.x & (lpr - 1));
   const long long groups_per_grid = ((long long)gridDim.x * blockDim.x) >> lpr_shift;
@@ -65,26 +78,26 @@ spmm_kernel(int n_rows, int kv, int lpr_shift, const int32_t* __restrict__ rowpt
     const int start = __ldg(rowptr + row);
     const int end = __ldg(rowptr + row + 1);
     for (int cv = lane; cv < kv; cv += lpr) {
-      T accA = vzero<V>();
-      T accB = vzero<V>();
-      const float* xa = XA + (size_t)cv * V;
-      const float* xb = (MODE == 2) ? XB + (size_t)cv * V : nullptr;
+      T accA = vzero<T>();
+      T accB = vzero<T>();
+      const S* xa = XA + (size_t)cv * V;
+      const S* xb = (MODE == 2) ? XB + (size_t)cv * V : nullptr;
       for (int j = start; j < end; j += 4) {
         int c[4];
-        float a[4], b[4];
+        S a[4], b[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
           const bool ok = (j + u) < end;
           c[u] = ok ? __ldg(col + j + u) : -1;
-          a[u] = ok ? __ldg(valA + j + u) : 0.f;
-          b[u] = (MODE != 0 && ok) ? __ldg(valB + j + u) : 0.f;
+          a[u] = ok ? __ldg(valA + j + u) : S(0);
+          b[u] = (MODE != 0 && ok) ? __ldg(valB + j + u) : S(0);
         }
         T x[4], y[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-          x[u] = (c[u] >= 0) ? __ldg(reinterpret_cast<const T*>(xa + (size_t)c[u] * ldx)) : vzero<V>();
+          x[u] = (c[u] >= 0) ? __ldg(reinterpret_cast<const T*>(xa + (size_t)c[u] * ldx)) : vzero<T>();
           if (MODE == 2)
-            y[u] = (c[u] >= 0) ? __ldg(reinterpret_cast<const T*>(xb + (size_t)c[u] * ldx)) : vzero<V>();
+            y[u] = (c[u] >= 0) ? __ldg(reinterpret_cast<const T*>(xb + (size_t)c[u] * ldx)) : vzero<T>();
         }
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -106,22 +119,22 @@ spmm_kernel(int n_rows, int kv, int lpr_shift, const int32_t* __restrict__ rowpt
   }
 }
 
-template <int MODE>
-int launch_spmm(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const float* valA,
-                const float* valB, const float* XA, const float* XB, int ldx, const float* D, int ldd,
-                float out_scale, const float* out_scale_dev, float* YA, float* YB, int ldy, cudaStream_t st) {
+template <typename S, int MODE>
+int launch_spmm(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const S* valA,
+                const S* valB, const S* XA, const S* XB, int ldx, const S* D, int ldd,
+                S out_scale, const S* out_scale_dev, S* YA, S* YB, int ldy, cudaStream_t st) {
   if (n_rows == 0 || k == 0) return EP_OK;
   int V = 1;
   auto ok_for = [&](int v) {
     if (k % v || ldx % v || ldy % v) return false;
     if (D && ldd % v) return false;
-    const size_t mask = (size_t)v * 4 - 1;
+    const size_t mask = (size_t)v * sizeof(S) - 1;
     const void* ptrs[] = {XA, XB, D, YA, YB};
     for (const void* p : ptrs)
       if (p && (reinterpret_cast<uintptr_t>(p) & mask)) return false;
     return true;
   };
-  if (ok_for(4)) V = 4; else if (ok_for(2)) V = 2;
+  if (sizeof(S) == 4 && ok_for(4)) V = 4; else if (ok_for(2)) V = 2;     // widest access: 16 bytes
   const int kv = k / V;
   int lpr_shift = 0;
   while ((1 << lpr_shift) < kv && lpr_shift < 5) ++lpr_shift;
@@ -131,9 +144,11 @@ int launch_spmm(int n_rows, int k, const int32_t* rowptr, const int32_t* col, co
   const long long cap = (long long)ep::sm_count() * 8 * g_spmm_waves;      // 8 CTAs of 256 threads fill one SM
   if (grid > cap) grid = cap;
 #define EP_SPMM_LAUNCH(VV)                                                                      \
-  spmm_kernel<VV, MODE><<<(unsigned)grid, block, 0, st>>>(n_rows, kv, lpr_shift, rowptr, col,   \
+  spmm_kernel<S, VV, MODE><<<(unsigned)grid, block, 0, st>>>(n_rows, kv, lpr_shift, rowptr, col,   \
       valA, valB, XA, XB, ldx, D, ldd, out_scale, out_scale_dev, YA, YB, ldy)
-  if (V == 4) EP_SPMM_LAUNCH(4); else if (V == 2) EP_SPMM_LAUNCH(2); else EP_SPMM_LAUNCH(1);
+  if (V == 1) EP_SPMM_LAUNCH(1);
+  else if (V == 2) EP_SPMM_LAUNCH(2);
+  else if constexpr (sizeof(S) == 4) EP_SPMM_LAUNCH(4);
 #undef EP_SPMM_LAUNCH
   EP_LAUNCH_CHECK("spmm_kernel");
   return EP_OK;
@@ -207,8 +222,17 @@ int ep_spmm_csr_f32(int n_rows, int k, const int32_t* rowptr, const int32_t* col
   EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
   EP_REQUIRE(rowptr && (n_rows == 0 || (col && val && X && Y)), "null pointer");
   EP_REQUIRE(ldx >= k && ldy >= k, "leading dimension < k");
-  return launch_spmm<0>(n_rows, k, rowptr, col, val, nullptr, X, nullptr, ldx, nullptr, 0, 1.f, nullptr, Y,
-                        nullptr, ldy, ep::as_stream(stream));
+  return launch_spmm<float, 0>(n_rows, k, rowptr, col, val, nullptr, X, nullptr, ldx, nullptr, 0, 1.f, nullptr, Y,
+                               nullptr, ldy, ep::as_stream(stream));
+}
+
+int ep_spmm_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const double* val,
+                    const double* X, int ldx, double* Y, int ldy, ep_stream_t stream) {
+  EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
+  EP_REQUIRE(rowptr && (n_rows == 0 || (col && val && X && Y)), "null pointer");
+  EP_REQUIRE(ldx >= k && ldy >= k, "leading dimension < k");
+  return launch_spmm<double, 0>(n_rows, k, rowptr, col, val, nullptr, X, nullptr, ldx, nullptr, 0, 1.0, nullptr, Y,
+                                nullptr, ldy, ep::as_stream(stream));
 }
 
 int ep_spmm2_csr_f32(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const float* valA,
@@ -217,8 +241,18 @@ int ep_spmm2_csr_f32(int n_rows, int k, const int32_t* rowptr, const int32_t* co
   EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
   EP_REQUIRE(rowptr && (n_rows == 0 || (col && valA && valB && X && YA && YB)), "null pointer");
   EP_REQUIRE(ldx >= k && ldy >= k, "leading dimension < k");
-  return launch_spmm<1>(n_rows, k, rowptr, col, valA, valB, X, nullptr, ldx, nullptr, 0, 1.f, nullptr, YA, YB,
-                        ldy, ep::as_stream(stream));
+  return launch_spmm<float, 1>(n_rows, k, rowptr, col, valA, valB, X, nullptr, ldx, nullptr, 0, 1.f, nullptr, YA, YB,
+                               ldy, ep::as_stream(stream));
+}
+
+int ep_spmm2_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const double* valA,
+                     const double* valB, const double* X, int ldx, double* YA, double* YB, int ldy,
+                     ep_stream_t stream) {
+  EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
+  EP_REQUIRE(rowptr && (n_rows == 0 || (col && valA && valB && X && YA && YB)), "null pointer");
+  EP_REQUIRE(ldx >= k && ldy >= k, "leading dimension < k");
+  return launch_spmm<double, 1>(n_rows, k, rowptr, col, valA, valB, X, nullptr, ldx, nullptr, 0, 1.0, nullptr, YA, YB,
+                                ldy, ep::as_stream(stream));
 }
 
 int ep_spmm2_sum_csr_f32(int n_rows, int k, const int32_t* rowptr, const int32_t* col,
@@ -228,8 +262,19 @@ int ep_spmm2_sum_csr_f32(int n_rows, int k, const int32_t* rowptr, const int32_t
   EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
   EP_REQUIRE(rowptr && (n_rows == 0 || (col && valA && valB && XA && XB && Y)), "null pointer");
   EP_REQUIRE(ldx >= k && ldy >= k && (!D || ldd >= k), "leading dimension < k");
-  return launch_spmm<2>(n_rows, k, rowptr, col, valA, valB, XA, XB, ldx, D, ldd, out_scale, out_scale_dev, Y, nullptr,
-                        ldy, ep::as_stream(stream));
+  return launch_spmm<float, 2>(n_rows, k, rowptr, col, valA, valB, XA, XB, ldx, D, ldd, out_scale, out_scale_dev, Y,
+                               nullptr, ldy, ep::as_stream(stream));
+}
+
+int ep_spmm2_sum_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col,
+                         const double* valA, const double* valB, const double* XA, const double* XB,
+                         int ldx, const double* D, int ldd, double out_scale, const double* out_scale_dev, double* Y,
+                         int ldy, ep_stream_t stream) {
+  EP_REQUIRE(n_rows >= 0 && k >= 0, "negative size");
+  EP_REQUIRE(rowptr && (n_rows == 0 || (col && valA && valB && XA && XB && Y)), "null pointer");
+  EP_REQUIRE(ldx >= k && ldy >= k && (!D || ldd >= k), "leading dimension < k");
+  return launch_spmm<double, 2>(n_rows, k, rowptr, col, valA, valB, XA, XB, ldx, D, ldd, out_scale, out_scale_dev, Y,
+                                nullptr, ldy, ep::as_stream(stream));
 }
 
 int ep_neighbor_mean_concat_f32(int n, int d, const int32_t* rowptr, const int32_t* col,
@@ -254,7 +299,7 @@ int ep_spmm_concat_f32(int n, int d, const int32_t* rowptr, const int32_t* col, 
   cudaStream_t st = ep::as_stream(stream);
   copy2d_kernel<<<grid_for((long long)n * d, 256), 256, 0, st>>>(n, d, x, ldx, H, ldh);
   EP_LAUNCH_CHECK("copy2d_kernel");
-  return launch_spmm<0>(n, d, rowptr, col, val, nullptr, x, nullptr, ldx, nullptr, 0, 1.f, nullptr, H + d,
+  return launch_spmm<float, 0>(n, d, rowptr, col, val, nullptr, x, nullptr, ldx, nullptr, 0, 1.f, nullptr, H + d,
                         nullptr, ldh, st);
 }
 

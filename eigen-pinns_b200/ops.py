@@ -3,6 +3,10 @@
 Every function here enqueues hand-written sm_100a kernels on torch's current CUDA stream;
 torch is only the allocator / stream / autograd plumbing.  CPU tensors are rejected: there is
 no fallback path.
+
+The SpMM, partials and dense-layer wrappers also take float64 tensors (the notebook variants train in double):
+the dtype of the inputs selects the _f64 entry point, and operators must have the same dtype as the dense
+operands (OperatorPair(..., dtype=torch.float64)).  Nothing is cast implicitly.
 """
 import ctypes
 
@@ -36,13 +40,30 @@ def _rowmajor(t):
     return t
 
 
+_SUFFIX = {torch.float32: "f32", torch.float64: "f64"}
+
+
+def _scalar(t):
+    """Entry-point suffix for a tensor of the fp32 / fp64 families."""
+    if t.dtype not in _SUFFIX:
+        raise TypeError("expected torch.float32 or torch.float64, got %s" % t.dtype)
+    return _SUFFIX[t.dtype]
+
+
+def _check_op(t, op):
+    """Dense operand t of a product with CSR operator(s) op (CsrMatrix or OperatorPair): same dtype, no cast."""
+    if t.dtype != op.dtype:
+        raise TypeError("operator values are %s but the dense operand is %s" % (op.dtype, t.dtype))
+    return _check(t, op.dtype)
+
+
 # ------------------------------------------------------------------------------- SpMM
 def spmm(A: CsrMatrix, X, out=None):
-    """Y = A X (fp32).  reference: torch.sparse.mm, src/multigrid_model.py:309-310."""
-    X = _check(_rowmajor(X))
+    """Y = A X (fp32, or fp64 for an fp64 A).  reference: torch.sparse.mm, src/multigrid_model.py:309-310."""
+    X = _check_op(_rowmajor(X), A)
     k = X.shape[1]
-    Y = out if out is not None else torch.empty((A.shape[0], k), device=X.device, dtype=torch.float32)
-    call("ep_spmm_csr_f32", A.shape[0], k, _ptr(A.rowptr), _ptr(A.col), _ptr(A.val), _ptr(X), X.stride(0),
+    Y = out if out is not None else torch.empty((A.shape[0], k), device=X.device, dtype=A.dtype)
+    call("ep_spmm_csr_" + _scalar(X), A.shape[0], k, _ptr(A.rowptr), _ptr(A.col), _ptr(A.val), _ptr(X), X.stride(0),
          _ptr(Y), Y.stride(0), _stream())
     return Y
 
@@ -56,28 +77,30 @@ def spmm2(pair: OperatorPair, X, out_K=None, out_M=None, rows=None):
     """(K X, M X) with one pass over the shared sparsity pattern.  rows=(a, b) restricts the product to that row
     range (outputs are still indexed by the full row number): the sharded engine computes interior rows while
     the halo exchange is in flight, then the boundary rows."""
-    X = _check(_rowmajor(X))
+    X = _check_op(_rowmajor(X), pair)
     k = X.shape[1]
     n = pair.n
-    KU = out_K if out_K is not None else torch.empty((n, k), device=X.device, dtype=torch.float32)
-    MU = out_M if out_M is not None else torch.empty((n, k), device=X.device, dtype=torch.float32)
+    KU = out_K if out_K is not None else torch.empty((n, k), device=X.device, dtype=pair.dtype)
+    MU = out_M if out_M is not None else torch.empty((n, k), device=X.device, dtype=pair.dtype)
     assert KU.stride(0) == MU.stride(0)
     a, b = (0, n) if rows is None else rows
     if b <= a:
         return KU, MU
     ld = KU.stride(0)
-    call("ep_spmm2_csr_f32", b - a, k, _off(pair.K.rowptr, a), _ptr(pair.K.col), _ptr(pair.K.val), _ptr(pair.M.val),
+    call("ep_spmm2_csr_" + _scalar(X), b - a, k, _off(pair.K.rowptr, a), _ptr(pair.K.col), _ptr(pair.K.val), _ptr(pair.M.val),
          _ptr(X), X.stride(0), _off(KU, a * ld), _off(MU, a * ld), ld, _stream())
     return KU, MU
 
 
 def spmm2_sum(KT: CsrMatrix, MT: CsrMatrix, XA, XB, D=None, scale=1.0, out=None, scale_dev=None):
     """out = scale * (KT XA + MT XB + D); KT and MT share a pattern."""
-    XA, XB = _check(XA), _check(XB)
+    XA, XB = _check_op(XA, KT), _check_op(XB, MT)
+    if D is not None and D.dtype != KT.dtype:
+        raise TypeError("operator values are %s but D is %s" % (KT.dtype, D.dtype))
     k = XA.shape[1]
     assert XA.stride(0) == XB.stride(0)
-    Y = out if out is not None else torch.empty((KT.shape[0], k), device=XA.device, dtype=torch.float32)
-    call("ep_spmm2_sum_csr_f32", KT.shape[0], k, _ptr(KT.rowptr), _ptr(KT.col), _ptr(KT.val), _ptr(MT.val),
+    Y = out if out is not None else torch.empty((KT.shape[0], k), device=XA.device, dtype=KT.dtype)
+    call("ep_spmm2_sum_csr_" + _scalar(XA), KT.shape[0], k, _ptr(KT.rowptr), _ptr(KT.col), _ptr(KT.val), _ptr(MT.val),
          _ptr(XA), _ptr(XB), XA.stride(0), _ptr(D), D.stride(0) if D is not None else 0,
          float(scale), _ptr(scale_dev), _ptr(Y), Y.stride(0), _stream())
     return Y
@@ -142,13 +165,15 @@ class EigenWorkspace:
 
 
 def eigen_partials(U, KU, MU, out=None):
-    """fp64 [G (k*k) | num | sKK | sKM | sMM] for one level (see include/eigenpinns_b200.h)."""
-    U, KU, MU = _check(U), _check(KU), _check(MU)
+    """fp64 [G (k*k) | num | sKK | sKM | sMM] for one level (see include/eigenpinns_b200.h).  U, KU, MU are all fp32
+    or all fp64."""
+    dtype = torch.float64 if U.dtype == torch.float64 else torch.float32
+    U, KU, MU = _check(U, dtype), _check(KU, dtype), _check(MU, dtype)
     n, k = U.shape
     ws = EigenWorkspace.get(k, U.device)
     P = out if out is not None else torch.empty(ws.plen, dtype=torch.float64, device=U.device)
     assert KU.stride(0) == MU.stride(0)
-    call("ep_eigen_partials_f32", n, k, _ptr(U), U.stride(0), _ptr(KU), _ptr(MU), KU.stride(0), _ptr(P),
+    call("ep_eigen_partials_" + _scalar(U), n, k, _ptr(U), U.stride(0), _ptr(KU), _ptr(MU), KU.stride(0), _ptr(P),
          _ptr(ws.buf), ws.bytes, _stream())
     return P
 
@@ -342,13 +367,21 @@ def eigen_loss(U_pred, pairs, offsets, w_res, w_orth):
 
 
 # ------------------------------------------------------------------------------- MLP, fp32 path
+def _layer_dtype(X):
+    """fp64 activations run the fp64 layer kernels; everything else is checked against fp32 as before."""
+    return torch.float64 if X.dtype == torch.float64 else torch.float32
+
+
 def linear_fwd(X, W, b, relu, out=None):
-    X, W = _check(_rowmajor(X)), _check(W)
+    dtype = _layer_dtype(X)
+    X, W = _check(_rowmajor(X), dtype), _check(W, dtype)
+    if b is not None and b.dtype != dtype:
+        raise TypeError("X is %s but the bias is %s" % (dtype, b.dtype))
     n, d_in = X.shape
     d_out = W.shape[0]
     assert W.is_contiguous() and W.shape[1] == d_in
-    Y = out if out is not None else torch.empty((n, d_out), device=X.device, dtype=torch.float32)
-    call("ep_linear_fwd_f32", n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(b), _ptr(Y), Y.stride(0),
+    Y = out if out is not None else torch.empty((n, d_out), device=X.device, dtype=dtype)
+    call("ep_linear_fwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(b), _ptr(Y), Y.stride(0),
          1 if relu else 0, _stream())
     return Y
 
@@ -356,8 +389,8 @@ def linear_fwd(X, W, b, relu, out=None):
 _bwd_ws = {}
 
 
-def _linear_bwd_workspace(n, d_in, d_out, device):
-    need = query("ep_linear_bwd_workspace_bytes", n, d_in, d_out)
+def _linear_bwd_workspace(n, d_in, d_out, device, dtype=torch.float32):
+    need = query("ep_linear_bwd_workspace_bytes" + ("_f64" if dtype == torch.float64 else ""), n, d_in, d_out)
     key = str(device)
     buf = _bwd_ws.get(key)
     if buf is None or buf.numel() < need:
@@ -368,15 +401,16 @@ def _linear_bwd_workspace(n, d_in, d_out, device):
 
 def linear_bwd(X, W, dY, need_dX, relu_mask, dW=None, db=None, dX=None):
     """dX = (dY W) * [X > 0] (if need_dX), dW = dY^T X, db = colsum(dY)."""
-    X, W, dY = _check(_rowmajor(X)), _check(W), _check(_rowmajor(dY))
+    dtype = _layer_dtype(X)
+    X, W, dY = _check(_rowmajor(X), dtype), _check(W, dtype), _check(_rowmajor(dY), dtype)
     n, d_in = X.shape
     d_out = W.shape[0]
     dW = dW if dW is not None else torch.empty_like(W)
-    db = db if db is not None else torch.empty(d_out, device=X.device, dtype=torch.float32)
+    db = db if db is not None else torch.empty(d_out, device=X.device, dtype=dtype)
     if need_dX and dX is None:
-        dX = torch.empty((n, d_in), device=X.device, dtype=torch.float32)
-    buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device)
-    call("ep_linear_bwd_f32", n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(dY), dY.stride(0),
+        dX = torch.empty((n, d_in), device=X.device, dtype=dtype)
+    buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device, dtype)
+    call("ep_linear_bwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(dY), dY.stride(0),
          _ptr(dX) if need_dX else None, dX.stride(0) if need_dX else 0, 1 if relu_mask else 0, _ptr(dW), _ptr(db),
          _ptr(buf), need, _stream())
     return dX, dW, db

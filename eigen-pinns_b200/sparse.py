@@ -1,4 +1,4 @@
-"""Device-resident CSR operators (fp32 values, int32 indices).
+"""Device-resident CSR operators (fp32 values, or fp64 for the notebook variants; int32 indices).
 
 The reference converts every scipy matrix to a torch COO tensor on EVERY epoch
 (reference src/utils.py:14-20, called from src/multigrid_model.py:306-307); here the
@@ -19,24 +19,48 @@ def _to_csr_f32(A):
     return B
 
 
-class CsrMatrix:
-    """CSR matrix on one CUDA device."""
+def _to_csr_f64(A):
+    """scipy -> canonical CSR with fp64 values: duplicates are merged in fp64, values stay scipy's bit for bit."""
+    A = A.tocoo()
+    B = sp.coo_matrix((A.data.astype(np.float64), (A.row, A.col)), shape=A.shape).tocsr()
+    B.sum_duplicates()
+    B.sort_indices()
+    return B
 
-    def __init__(self, host_csr, device):
+
+_NP_DTYPE = {torch.float32: np.float32, torch.float64: np.float64}
+
+
+def _np_dtype(dtype):
+    if dtype not in _NP_DTYPE:
+        raise TypeError("CSR values are torch.float32 or torch.float64, not %s" % dtype)
+    return _NP_DTYPE[dtype]
+
+
+class CsrMatrix:
+    """CSR matrix on one CUDA device; `dtype` is the type of its values (torch.float32 or torch.float64)."""
+
+    def __init__(self, host_csr, device, dtype=torch.float32):
         if host_csr.nnz >= 2 ** 31 or max(host_csr.shape) >= 2 ** 31:
             raise ValueError("CsrMatrix uses int32 indices")
         self.shape = tuple(host_csr.shape)
         self.nnz = int(host_csr.nnz)
         self.device = torch.device(device)
+        self.dtype = dtype
         self._host = host_csr
         self.rowptr = torch.from_numpy(host_csr.indptr.astype(np.int32)).to(self.device)
         self.col = torch.from_numpy(host_csr.indices.astype(np.int32)).to(self.device)
-        self.val = torch.from_numpy(host_csr.data.astype(np.float32)).to(self.device)
+        self.val = torch.from_numpy(host_csr.data.astype(_np_dtype(dtype))).to(self.device)
         self._T = None
         self._symmetric = None
 
     @classmethod
-    def from_scipy(cls, A, device):
+    def from_scipy(cls, A, device, dtype=torch.float32):
+        """fp32 rounds the values first and then merges duplicates, as the reference's torch.FloatTensor + coalesce
+        does; fp64 keeps scipy's values."""
+        if dtype == torch.float64:
+            return cls(_to_csr_f64(A), device, dtype)
+        _np_dtype(dtype)
         return cls(_to_csr_f32(A), device)
 
     @classmethod
@@ -44,6 +68,7 @@ class CsrMatrix:
         """Wrap CSR arrays that already live on the GPU (e.g. from fem_device.assemble)."""
         obj = cls.__new__(cls)
         obj.shape, obj.nnz, obj.device = tuple(shape), int(col.numel()), rowptr.device
+        obj.dtype = val.dtype if val is not None else torch.float32
         obj._host, obj.rowptr, obj.col, obj.val = None, rowptr, col, val
         obj._T, obj._symmetric = None, symmetric
         return obj
@@ -67,6 +92,7 @@ class CsrMatrix:
         obj.shape = (n, n)
         obj.nnz = int(row.size)
         obj.device = torch.device(device)
+        obj.dtype = torch.float32
         obj._host = None
         rowptr = np.zeros(n + 1, dtype=np.int64)
         np.cumsum(counts, out=rowptr[1:])
@@ -101,7 +127,7 @@ class CsrMatrix:
         if self._T is None:
             T = self._need_host("transpose()").T.tocsr()
             T.sort_indices()
-            self._T = CsrMatrix(T, self.device)
+            self._T = CsrMatrix(T, self.device, self.dtype)
         return self._T
 
 
@@ -110,12 +136,17 @@ class OperatorPair:
     (always true for the FEM operators of src/Mesh.py) the dual kernel reads each gathered
     row of U once for both products."""
 
-    def __init__(self, K, M, device, assume_symmetric=None):
+    def __init__(self, K, M, device, assume_symmetric=None, dtype=torch.float32):
         """assume_symmetric=True: the GLOBAL operators are symmetric although these (possibly rectangular,
-        rank-local [owned | halo] column space) blocks cannot be checked - skips the transposes."""
-        self.K = K if isinstance(K, CsrMatrix) else CsrMatrix.from_scipy(K, device)
-        self.M = M if isinstance(M, CsrMatrix) else CsrMatrix.from_scipy(M, device)
+        rank-local [owned | halo] column space) blocks cannot be checked - skips the transposes.
+        dtype: value type of operators given as scipy matrices (torch.float64 for the notebook variants); operators
+        given as CsrMatrix keep their own, which must agree."""
+        self.K = K if isinstance(K, CsrMatrix) else CsrMatrix.from_scipy(K, device, dtype)
+        self.M = M if isinstance(M, CsrMatrix) else CsrMatrix.from_scipy(M, device, dtype)
         assert self.K.shape == self.M.shape
+        if self.K.dtype != self.M.dtype:
+            raise TypeError("K is %s but M is %s" % (self.K.dtype, self.M.dtype))
+        self.dtype = self.K.dtype
         self.n = self.K.shape[0]
         self.shared = (self.K.rowptr is self.M.rowptr and self.K.col is self.M.col) or (
             self.K.nnz == self.M.nnz and torch.equal(self.K.rowptr, self.M.rowptr) and torch.equal(self.K.col, self.M.col))
@@ -126,18 +157,18 @@ class OperatorPair:
             self.KT, self.MT = self.K, self.M
         else:
             KT, MT = self.K._need_host("transpose()").T.tocsr(), self.M._need_host("transpose()").T.tocsr()
-            self.KT, self.MT = CsrMatrix(_sorted(KT), device), CsrMatrix(_sorted(MT), device)
+            self.KT, self.MT = CsrMatrix(_sorted(KT), device, self.dtype), CsrMatrix(_sorted(MT), device, self.dtype)
 
     def _unify(self):
         """Pad both operators to the union pattern (explicit zeros) so one rowptr/col serves both."""
         K, M = self.K._host.tocoo(), self.M._host.tocoo()
         rows = np.concatenate([K.row, M.row])
         cols = np.concatenate([K.col, M.col])
-        zK, zM = np.zeros(K.nnz, np.float32), np.zeros(M.nnz, np.float32)
+        zK, zM = np.zeros(K.nnz, K.data.dtype), np.zeros(M.nnz, M.data.dtype)
         Ku = sp.coo_matrix((np.concatenate([K.data, zM]), (rows, cols)), shape=K.shape).tocsr()
         Mu = sp.coo_matrix((np.concatenate([zK, M.data]), (rows, cols)), shape=K.shape).tocsr()
         dev = self.K.device
-        self.K, self.M = CsrMatrix(_sorted(Ku), dev), CsrMatrix(_sorted(Mu), dev)
+        self.K, self.M = CsrMatrix(_sorted(Ku), dev, self.dtype), CsrMatrix(_sorted(Mu), dev, self.dtype)
         assert np.array_equal(Ku.indices, Mu.indices) and np.array_equal(Ku.indptr, Mu.indptr)
         self.shared = True
 

@@ -18,8 +18,11 @@ the C ABI and writes each notebook's functional on top of them with torch for th
   CoordinateMLP            the coordinate networks of the first two (x in R^3 -> U in R^k, SiLU)
   EigenfunctionNN          the network of the third (sin activations, lambda = |w| appended to every layer's input)
 
-The kernels are fp32 (fp64 accumulation in the Gram partials); the notebooks run the first two in fp64, so parity
-with the restated formulas (oracle/variants_port.py, fp64) is checked to fp32 tolerances in tests/test_gpu_variants.py.
+Every piece runs in fp32 (fp64 accumulation in the Gram partials) or, as the notebooks train, in fp64: the dtype of
+the tensors selects the kernels.  For fp64 build the operators with OperatorPair(K, M, device, dtype=torch.float64)
+and call .double() on the networks; activations stay torch element-wise in either precision.  Parity with the
+restated formulas (oracle/variants_port.py, fp64) is checked to fp32 tolerances in tests/test_gpu_variants.py and
+on the unrounded operators to fp64 tolerances in tests/test_gpu_variants_f64.py.
 Operators must be symmetric (FEM K and M are): the backward uses K^T = K.
 """
 import torch
@@ -38,7 +41,7 @@ class _OperatorStatsFn(torch.autograd.Function):
     def forward(ctx, U, pair, want_gram):
         if not pair.symmetric:
             raise ValueError("variants need symmetric operators (K^T = K, M^T = M)")
-        U = ops._check(ops._rowmajor(U))
+        U = ops._check_op(ops._rowmajor(U), pair)
         k = U.shape[1]
         KU, MU = ops.spmm2(pair, U)
         ctx.pair = pair
@@ -58,9 +61,9 @@ class _OperatorStatsFn(torch.autograd.Function):
         KU, MU = ctx.saved_tensors
         direct = None
         if gA is not None:
-            direct = ops.linear_fwd(KU, (gA + gA.t()).to(torch.float32).contiguous(), None, False)   # KU S, S symmetric
+            direct = ops.linear_fwd(KU, (gA + gA.t()).to(KU.dtype).contiguous(), None, False)   # KU S, S symmetric
         if gB is not None:
-            d = ops.linear_fwd(MU, (gB + gB.t()).to(torch.float32).contiguous(), None, False)
+            d = ops.linear_fwd(MU, (gB + gB.t()).to(KU.dtype).contiguous(), None, False)
             direct = d if direct is None else direct + d
         if gKU is None and gMU is None:
             return direct, None, None
@@ -149,7 +152,7 @@ def single_mode_loss(u, eigenvalue, pair: OperatorPair, previous=(), ortho_weigh
     uf, Luf, Muf = u.squeeze(1), Lu.squeeze(1), Mu.squeeze(1)
     eig = ((Luf - eigenvalue.reshape(()) * Muf) ** 2).mean()
     norm = (torch.dot(uf, Muf) - 1.0) ** 2
-    ortho = torch.zeros((), device=u.device)
+    ortho = torch.zeros((), dtype=u.dtype, device=u.device)
     for u_prev in previous:
         Mp = ops.spmm(pair.M, u_prev.detach().reshape(-1, 1).contiguous()).squeeze(1)
         ortho = ortho + torch.dot(uf, Mp) ** 2
@@ -169,7 +172,8 @@ def smoothness_loss(corr, U_pred, pair: OperatorPair, denom=None):
 
 # ------------------------------------------------------------------------------------- networks
 class KernelLinear(nn.Module):
-    """nn.Linear whose products run on the fp32 GEMM kernels of the C ABI (ep_linear_fwd_f32 / ep_linear_bwd_f32)."""
+    """nn.Linear whose products run on the GEMM kernels of the C ABI (ep_linear_fwd_f32 / ep_linear_bwd_f32, or the
+    _f64 entries after .double())."""
 
     def __init__(self, in_features, out_features):
         super().__init__()

@@ -14,7 +14,8 @@
  *   - one device and one stream per process are assumed by the cached launch configuration
  *     (SM count, opted-in shared-memory sizes, the gradient-norm scratch)
  *   - dense matrices are row-major with an explicit leading dimension (elements)
- *   - CSR: int32 rowptr[n+1], int32 col[nnz], fp32 val[nnz]
+ *   - CSR: int32 rowptr[n+1], int32 col[nnz], fp32 val[nnz]; the *_f64 entries take fp64 val[nnz] and fp64
+ *     dense operands (the notebook variants, which train in double)
  *   - every call takes the CUDA stream it is enqueued on (cudaStream_t as void*); nothing
  *     synchronises unless stated; no hidden allocation: workspaces are sized by *_workspace_bytes
  *   - return value: 0 = EP_OK, negative = error (see ep_status); ep_last_error_string()
@@ -80,6 +81,21 @@ EP_API int ep_spmm2_sum_csr_f32(int n_rows, int k, const int32_t* rowptr, const 
                          int ldx, const float* D, int ldd, float out_scale, const float* out_scale_dev,
                          float* Y, int ldy, ep_stream_t stream);
 
+/* fp64 forms of the three products above (same argument order, double in place of float; out_scale_dev is a
+ * device double).  They serve the notebook variants in double precision: K U, M U of
+ * scripts/simplified_loss.ipynb cell 0 and scripts/loss_with_rigid_body.ipynb cell 0 (torch.sparse.mm in fp64),
+ * L u, M u of delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1, L corr of
+ * delta_pinns_validation/multigrid_gnn_refine_fixed.ipynb cell 4, and the transposed products of their backward. */
+EP_API int ep_spmm_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col, const double* val,
+                    const double* X, int ldx, double* Y, int ldy, ep_stream_t stream);
+EP_API int ep_spmm2_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col,
+                     const double* valA, const double* valB, const double* X, int ldx,
+                     double* YA, double* YB, int ldy, ep_stream_t stream);
+EP_API int ep_spmm2_sum_csr_f64(int n_rows, int k, const int32_t* rowptr, const int32_t* col,
+                         const double* valA, const double* valB, const double* XA, const double* XB,
+                         int ldx, const double* D, int ldd, double out_scale, const double* out_scale_dev,
+                         double* Y, int ldy, ep_stream_t stream);
+
 /* ---- corrector input: h = cat([x, agg], dim=1) -----------------------------------------
  * SimpleCorrector.forward, corrector_model.py:23-30: agg_i = (sum over edges (i<-j) of x_j) /
  * max(deg_i, 1), edges given as CSR over destination rows (rowptr/col), summed in edge order.
@@ -105,6 +121,12 @@ EP_API int ep_spmm_concat_f32(int n, int d, const int32_t* rowptr, const int32_t
 EP_API size_t ep_eigen_partials_len(int k);                        /* k*k + 5*k doubles */
 EP_API size_t ep_eigen_partials_workspace_bytes(int k);
 EP_API int ep_eigen_partials_f32(int n, int k, const float* U, int ldu, const float* KU, const float* MU,
+                          int ld, double* out, void* workspace, size_t workspace_bytes,
+                          ep_stream_t stream);
+/* fp64 inputs, same output layout, workspace size and k <= 128; every product and sum is fp64 (no fp32 stage).
+ * The Gram matrices U^T K U and U^T M U of scripts/simplified_loss.ipynb cell 0 (UKU, UMU) and
+ * scripts/loss_with_rigid_body.ipynb cell 0 (B and the Rayleigh matrix) in the notebooks' precision. */
+EP_API int ep_eigen_partials_f64(int n, int k, const double* U, int ldu, const double* KU, const double* MU,
                           int ld, double* out, void* workspace, size_t workspace_bytes,
                           ep_stream_t stream);
 
@@ -207,6 +229,16 @@ EP_API size_t ep_linear_bwd_workspace_bytes(int n, int in, int out);
 EP_API int ep_linear_bwd_f32(int n, int in, int out, const float* X, int ldx, const float* W,
                       const float* dY, int lddy, float* dX, int lddx, int relu_mask,
                       float* dW, float* db, void* workspace, size_t workspace_bytes,
+                      ep_stream_t stream);
+/* fp64 forms (plain DFMA, same tiling and fixed-order split-K): the dense layers of the notebook networks in double -
+ * `MLP` of scripts/simplified_loss.ipynb cell 0 and scripts/loss_with_rigid_body.ipynb cell 0, `EigenfunctionNN` of
+ * delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1. */
+EP_API int ep_linear_fwd_f64(int n, int in, int out, const double* X, int ldx, const double* W, const double* b,
+                      double* Y, int ldy, int act, ep_stream_t stream);
+EP_API size_t ep_linear_bwd_workspace_bytes_f64(int n, int in, int out);
+EP_API int ep_linear_bwd_f64(int n, int in, int out, const double* X, int ldx, const double* W,
+                      const double* dY, int lddy, double* dX, int lddx, int relu_mask,
+                      double* dW, double* db, void* workspace, size_t workspace_bytes,
                       ep_stream_t stream);
 
 /* ---- corrector MLP, bf16 tcgen05 path ("perf mode") --------------------------------------
