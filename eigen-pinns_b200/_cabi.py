@@ -46,6 +46,10 @@ SIGNATURES = {
                                                  c_int, c_int, c_p]),
     "ep_scale_columns_rsqrt_f32": (c_int, [c_int, c_int, c_p, c_int, c_p, c_int, c_d, c_p, c_int, c_p]),
     "ep_axpy_out_f32": (c_int, [c_sz, c_f, c_p, c_p, c_p, c_p, c_p]),
+    "ep_mode_scale_fwd_f32": (c_int, [c_int, c_int, c_p, c_int, c_p, c_int, c_p, c_f, c_p, c_p, c_int, c_p]),
+    "ep_mode_scale_bwd_workspace_bytes": (c_sz, [c_int]),
+    "ep_mode_scale_bwd_f32": (c_int, [c_int, c_int, c_d, c_p, c_int, c_p, c_int, c_p, c_f, c_p, c_int, c_p, c_int,
+                                      c_p, c_p, c_sz, c_p]),
     "ep_linear_fwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_int, c_p]),
     "ep_linear_bwd_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
     "ep_linear_bwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_int, c_int,
@@ -108,6 +112,7 @@ KERNELS_PER_CALL = {
     "ep_halo_exchange_f32": 1,
     "ep_spmm_csr_f64": 1, "ep_spmm2_csr_f64": 1, "ep_spmm2_sum_csr_f64": 1, "ep_eigen_partials_f64": 2,
     "ep_linear_fwd_f64": 1, "ep_linear_bwd_f64": 5,
+    "ep_mode_scale_fwd_f32": 1, "ep_mode_scale_bwd_f32": 2,
 }
 launch_counter = 0
 launch_by_entry = {}          # entry point -> kernels launched through it (bench.py reports the per-step table)

@@ -149,10 +149,18 @@ def resolve_send_lists(plan: LevelPlan, group=None):
     return plan
 
 
+def _refuse_mode_scales(has_scales, w_smooth_corr):
+    if has_scales or float(w_smooth_corr) != 0.0:
+        raise NotImplementedError("the vertex-sharded step does not train per-mode scales or the smoothness of the "
+                                  "correction (w_smooth_corr): they would need the halo rows of the raw corrector output "
+                                  "and an all-reduce of the scale gradient; use the single-GPU TrainStepEngine")
+
+
 class ShardedTrainStepEngine(TrainStepEngine):
     def __init__(self, h_local, U_base_local, plans, params: FlatParams, cfg: StepConfig, lam_target=None,
                  mlp_mode="fp32", group=None, symmetric=True, pairs=None):
         dev = h_local.device
+        _refuse_mode_scales(params.mode_scales is not None, cfg.w_smooth_corr)
         if not symmetric:
             raise NotImplementedError("the vertex-sharded step needs symmetric K, M (FEM / tufted Laplacians): the "
                                       "transposed products of a non-symmetric operator would need a halo scatter-add")
@@ -263,6 +271,7 @@ def make_sharded_engine(gnn, x_feats, edge_index, U_base, K, M, lam_target, opti
     """Single-level helper used by bench.py: every rank holds the global arrays once at set-up, keeps its
     vertex range, and builds the rank-local engine."""
     import torch.nn as nn
+    _refuse_mode_scales(hasattr(gnn.model, "mode_scales"), getattr(gnn, "w_smooth_corr", 0.0))
     dev = gnn.device
     h_global = gnn.model.corrector_input(x_feats.to(dev), edge_index.to(dev))
     plan = resolve_send_lists(LevelPlan(K, M, rank, world), group)

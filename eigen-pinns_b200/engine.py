@@ -23,9 +23,10 @@ class FlatParams:
     Adam moments of the same shape).  nn.Module parameters are re-pointed at views of it so the
     module's state_dict keeps working while the optimiser kernel updates everything in one launch."""
 
-    def __init__(self, weights, biases, device):
+    def __init__(self, weights, biases, device, mode_scales=None):
         self.shapes = [(tuple(w.shape), tuple(b.shape)) for w, b in zip(weights, biases)]
-        total = sum(w.numel() + b.numel() for w, b in zip(weights, biases))
+        n_scales = 0 if mode_scales is None else mode_scales.numel()
+        total = sum(w.numel() + b.numel() for w, b in zip(weights, biases)) + n_scales
         self.flat = torch.empty(total, dtype=torch.float32, device=device)
         self.grad = torch.zeros_like(self.flat)
         self.m = torch.zeros_like(self.flat)
@@ -42,17 +43,26 @@ class FlatParams:
                 store.append(view)
                 gstore.append(self.grad[off:off + n].view(src.shape))
                 off += n
+        # learnable per-mode scales of the AdaptiveCorrector: k values after the last bias (None without them)
+        self.mode_scales = self.d_mode_scales = None
+        if mode_scales is not None:
+            self.mode_scales = self.flat[off:off + n_scales]
+            self.mode_scales.copy_(mode_scales.detach().reshape(-1).to(device=device, dtype=torch.float32))
+            self.d_mode_scales = self.grad[off:off + n_scales]
         self.step_count = 0
         self.sq_norm = torch.zeros(1, dtype=torch.float64, device=device)
 
     @classmethod
-    def adopt(cls, linears):
-        """Build from nn.Linear modules and make their parameters views of the flat buffer."""
+    def adopt(cls, linears, mode_scales=None):
+        """Build from nn.Linear modules (and the per-mode scale parameter, if any) and make their parameters views of
+        the flat buffer."""
         dev = linears[0].weight.device
-        fp = cls([l.weight for l in linears], [l.bias for l in linears], dev)
+        fp = cls([l.weight for l in linears], [l.bias for l in linears], dev, mode_scales=mode_scales)
         for lin, W, b in zip(linears, fp.W, fp.b):
             lin.weight.data = W
             lin.bias.data = b
+        if mode_scales is not None:
+            mode_scales.data = fp.mode_scales
         return fp
 
     @property
@@ -98,9 +108,10 @@ class Fp32Mlp:
 class StepConfig:
     def __init__(self, lr=1e-3, weight_decay=1e-5, corr_scale=10.0, w_res=1000.0, w_orth=10.0, w_trace=0.0,
                  w_order=0.0, w_eigen=0.0, grad_clip=10.0, beta1=0.9, beta2=0.999, eps=1e-8, ramp_epochs=5000.0,
-                 w_mean=0.0, w_smooth=0.0):
-        # w_mean / w_smooth: per-level zero-mean and smoothness terms of the notebook variants (SURVEY 8a-bis)
-        self.w_mean, self.w_smooth = w_mean, w_smooth
+                 w_mean=0.0, w_smooth=0.0, w_smooth_corr=0.0):
+        # w_mean / w_smooth: per-level zero-mean and smoothness terms of the notebook variants (SURVEY 8a-bis);
+        # w_smooth_corr: the smoothness of the correction, w sum corr o (K corr) / (n k) per level
+        self.w_mean, self.w_smooth, self.w_smooth_corr = w_mean, w_smooth, w_smooth_corr
         self.lr, self.weight_decay, self.corr_scale = lr, weight_decay, corr_scale
         self.w_res, self.w_orth, self.w_trace, self.w_order, self.w_eigen = w_res, w_orth, w_trace, w_order, w_eigen
         self.grad_clip, self.beta1, self.beta2, self.eps = grad_clip, beta1, beta2, eps
@@ -143,6 +154,20 @@ class TrainStepEngine:
             self.mlp.want_corr = False
         else:
             raise ValueError("mlp_mode must be 'fp32' or 'bf16'")
+        # Per-mode scales and / or the smoothness of the correction: the MLP writes the raw output c, then
+        # ep_mode_scale_fwd_f32 forms U_pred and ep_mode_scale_bwd_f32 runs after the eigen-loss backward.  Decided once
+        # here; without either the step keeps the plain path (the chain writes U_pred itself).
+        self.adaptive = params.mode_scales is not None or float(cfg.w_smooth_corr) != 0.0
+        self.Kc = None
+        if self.adaptive:
+            if mlp_mode == "bf16":
+                self.mlp.want_corr = True
+            if float(cfg.w_smooth_corr) != 0.0:
+                for li, pair in enumerate(pairs):
+                    if not pair.symmetric:
+                        raise ValueError("w_smooth_corr needs a symmetric K (level %d is not): the gradient uses "
+                                         "K^T = K" % li)
+                self.Kc = torch.empty((self.n_mlp, k), **f32)
         self.launches_per_step = None
         self.use_graph, self._graph, self.hyper = False, None, None
         self.fused_bwd = True          # symmetric operators: one-pass analytic backward
@@ -162,8 +187,36 @@ class TrainStepEngine:
 
     def forward(self, scale, scale_dev=None):
         m = self.n_mlp
-        return self.mlp.forward(self.h[:m], U_base=self.U_base[:m], scale=scale, U_pred=self.U_pred[:m],
-                                scale_dev=scale_dev)
+        if not self.adaptive:
+            return self.mlp.forward(self.h[:m], U_base=self.U_base[:m], scale=scale, U_pred=self.U_pred[:m],
+                                    scale_dev=scale_dev)
+        self.mlp.forward(self.h[:m])
+        self.mode_scale_forward(scale, scale_dev)
+        return self.corr_raw
+
+    @property
+    def corr_raw(self):
+        """Raw MLP output c (n_mlp x k, fp32): the last activation (fp32 mode) or the chain's corr output (bf16)."""
+        return self.mlp.acts[-1] if self.mlp_mode == "fp32" else self.mlp.corr
+
+    def mode_scale_forward(self, scale, scale_dev=None):
+        """U_pred = U_base + scale * (c o mode_scales) and, with w_smooth_corr, K c per level."""
+        m, c = self.n_mlp, self.corr_raw
+        ops.mode_scale_fwd(c, self.U_base[:m], self.params.mode_scales, scale, out=self.U_pred[:m], sigma_dev=scale_dev)
+        if self.Kc is not None:
+            for li, pair in enumerate(self.pairs):
+                s = self._level_slices(li)
+                ops.spmm(pair.K, c[s], out=self.Kc[s])
+
+    def mode_scale_backward(self):
+        """Per level: dCorr -> dL/dc in place, dL/dmode_scales into the flat gradient, smoothness of the correction
+        into loss_acc[8] / [5]."""
+        c, p = self.corr_raw, self.params
+        for li in range(len(self.pairs)):
+            s = self._level_slices(li)
+            ops.mode_scale_bwd(c[s], self.Kc[s] if self.Kc is not None else None, p.mode_scales, self.cfg.w_smooth_corr,
+                               self.dCorr[s], n_global=self._n_global(li), grad_s=p.d_mode_scales, accumulate=li > 0,
+                               loss_acc=self.loss_acc)
 
     def mlp_backward(self):
         m = self.n_mlp
@@ -203,6 +256,8 @@ class TrainStepEngine:
             ops.spmm2_sum(pair.KT, pair.MT, KU_bar[s], MU_bar[s], D[s], scale, out=self.dCorr[s], scale_dev=scale_dev)
             if li in self.projections:
                 self.projections[li].backward(self.dCorr[s], scale, scale_dev)
+        if self.adaptive:
+            self.mode_scale_backward()
 
     def optimizer_step(self, lr, hyper_dev=None):
         p, c = self.params, self.cfg

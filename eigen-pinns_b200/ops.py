@@ -312,6 +312,46 @@ def axpy_out(a, b, alpha, out=None, alpha_dev=None):
     return out
 
 
+def mode_scale_fwd(c, U_base, s, sigma, out=None, sigma_dev=None):
+    """out = U_base + sigma * (c o s): the AdaptiveCorrector's per-mode scales (s None = unit scales)."""
+    c, U_base = _check(c), _check(U_base)
+    n, k = c.shape
+    assert U_base.shape == (n, k) and (s is None or (s.numel() == k and s.is_contiguous()))
+    out = out if out is not None else torch.empty((n, k), device=c.device, dtype=torch.float32)
+    call("ep_mode_scale_fwd_f32", n, k, _ptr(c), c.stride(0), _ptr(U_base), U_base.stride(0),
+         _ptr(_check(s) if s is not None else None), float(sigma), _ptr(sigma_dev), _ptr(_check(out)), out.stride(0),
+         _stream())
+    return out
+
+
+_mode_scale_ws = {}
+
+
+def mode_scale_workspace(k, device):
+    """Device scratch of ep_mode_scale_bwd_f32 for this k (one per device and k; calls on one stream share it)."""
+    key = (k, str(device))
+    ws = _mode_scale_ws.get(key)
+    if ws is None:
+        ws = torch.empty(query("ep_mode_scale_bwd_workspace_bytes", k), dtype=torch.uint8, device=device)
+        _mode_scale_ws[key] = ws
+    return ws
+
+
+def mode_scale_bwd(c, Kc, s, w_smooth_corr, dcorr, n_global=None, grad_s=None, accumulate=False, loss_acc=None):
+    """In place: dcorr (= dL/dcorr) -> dL/dc; grad_s (k) = or += dL/ds; loss_acc[8], [5] += the smoothness of the
+    correction, w / (n k) sum corr o (K corr).  Kc = K c (None when w_smooth_corr = 0), s None = unit scales."""
+    c, dcorr = _check(c), _check(dcorr)
+    n, k = c.shape
+    assert dcorr.shape == (n, k) and (Kc is None or Kc.shape == (n, k))
+    ws = mode_scale_workspace(k, c.device)
+    call("ep_mode_scale_bwd_f32", n, k, float(n if n_global is None else n_global), _ptr(c), c.stride(0),
+         _ptr(_check(Kc) if Kc is not None else None), Kc.stride(0) if Kc is not None else k,
+         _ptr(_check(s) if s is not None else None), float(w_smooth_corr), _ptr(dcorr), dcorr.stride(0),
+         _ptr(_check(grad_s) if grad_s is not None else None), 1 if accumulate else 0, _ptr(loss_acc), _ptr(ws),
+         ws.numel(), _stream())
+    return dcorr
+
+
 class _EigenLossFn(torch.autograd.Function):
     """(w_res * sum_levels L_res, w_orth * sum_levels L_orth, lam_0, lam_1, ...) with the analytic
     backward of SURVEY Appendix A.  Reference: src/multigrid_model.py:291-324."""

@@ -27,6 +27,10 @@ OPTIONAL_FIELDS = {
     "aggregation": "mean",     # 'mean' (reference) | 'sum' (notebook variant without the degree division)
     "operator_type": "auto",   # level operators of the point samplers: "point_cloud" (robust_laplacian, as the
                                # reference), "fem" (Galerkin P^T K P of the mesh's FEM operators), "auto" (first if installed)
+    # notebook variant multigrid_gnn_refine_fixed.ipynb cell 4 (model_type 'adaptive' = learnable per-mode scales)
+    "mode_scale_init": 0.01,   # initial value of the AdaptiveCorrector's per-mode scales
+    "weight_smooth": 0.0,      # w * sum U_pred o (K U_pred) / (n k) per level
+    "weight_smooth_corr": 0.0, # w * sum corr o (K corr) / (n k) per level (the notebook uses one weight for both)
 }
 
 

@@ -116,8 +116,10 @@ class AdaptiveCorrector(SimpleCorrector):
     """Notebook variant with learnable per-mode scales (SURVEY 8a-bis, `AdaptiveCorrector` of
     delta_pinns_validation/multigrid_gnn_refine_fixed.ipynb cell 4): correction = net([x, mean_nbr x]) * mode_scales.
     Runs on the same kernels through autograd (aggregation, fused Linear+ReLU GEMMs); the scales are a torch parameter.
-    The fused TrainStepEngine does not carry the extra parameter and refuses this model - train it with the
-    autograd-capable methods (`_forward_pass`, `_compute_residual_ortho_loss`, variants.smoothness_loss)."""
+    MultigridGNN (model_type 'adaptive') trains it in the fused TrainStepEngine: the scales are the last k entries of
+    the flat parameter buffer (clip + Adam like every weight), U_pred = U_base + scale * (net o mode_scales) and the
+    scale gradient come from ep_mode_scale_fwd_f32 / ep_mode_scale_bwd_f32, in fp32 and bf16 MLP mode, eager or
+    graph-replayed.  The vertex-sharded engine refuses it."""
 
     def __init__(self, in_dim, out_dim, hidden_layers=(128, 64, 32), dropout=0.0, init_scale=0.01):
         super().__init__(in_dim, out_dim, list(hidden_layers), dropout)

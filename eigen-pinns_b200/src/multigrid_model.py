@@ -18,7 +18,7 @@ from scipy.linalg import eigh
 
 import _backend
 import utils
-from corrector_model import SimpleCorrector, SpectralCorrector
+from corrector_model import AdaptiveCorrector, SimpleCorrector, SpectralCorrector
 
 _ops = _backend.module("ops")
 _engine = _backend.module("engine")
@@ -34,8 +34,8 @@ class MultigridGNN:
         self.device = torch.device("cuda", torch.cuda.current_device())
         self.model = None
         self.model_type = config.model_type.lower()
-        if self.model_type not in ['simple', 'spectral']:
-            raise ValueError(f"model_type must be 'simple' or 'spectral', got '{self.model_type}'")
+        if self.model_type not in ['simple', 'spectral', 'adaptive']:
+            raise ValueError(f"model_type must be 'simple', 'spectral' or 'adaptive', got '{self.model_type}'")
         for src, dst in (("epochs", "epochs"), ("learning_rate", "lr"), ("corrector_scale", "corr_scale"),
                          ("weight_residual", "w_res"), ("weight_orthogonal", "w_orth"),
                          ("weight_projection", "w_proj"), ("weight_trace", "w_trace"), ("w_order", "w_order"),
@@ -51,6 +51,11 @@ class MultigridGNN:
         self.loss_read_delay = int(getattr(config, "loss_read_delay", 1))
         self.graph_after_epochs = 3 if getattr(config, "cuda_graph", True) else -1
         self.seed = getattr(config, "seed", None)
+        # notebook variant (multigrid_gnn_refine_fixed.ipynb cell 4): 'adaptive' = SimpleCorrector times learnable
+        # per-mode scales; smoothness of U_pred and of the correction, w sum u o (K u) / (n k) per level
+        self.mode_scale_init = float(getattr(config, "mode_scale_init", 0.01))
+        self.w_smooth = float(getattr(config, "weight_smooth", 0.0))
+        self.w_smooth_corr = float(getattr(config, "weight_smooth_corr", 0.0))
         self.loss_history = []
 
     # ------------------------------------------------------------------ top level
@@ -151,6 +156,8 @@ class MultigridGNN:
             torch.manual_seed(self.seed)
         if self.model_type == 'simple':
             self.model = SimpleCorrector(input_dim, n_modes, hidden_layers, dropout, aggregation=self.aggregation)
+        elif self.model_type == 'adaptive':
+            self.model = AdaptiveCorrector(input_dim, n_modes, hidden_layers, dropout, init_scale=self.mode_scale_init)
         else:
             self.model = SpectralCorrector(input_dim, n_modes, hidden_layers, dropout)
         self.model = self.model.to(self.device)
@@ -172,21 +179,19 @@ class MultigridGNN:
                      optimizer):
         if self.dropout and self.dropout > 0.0:
             raise NotImplementedError("the fused training step supports dropout = 0.0 (the reference default)")
-        if hasattr(self.model, "mode_scales"):
-            raise NotImplementedError("the fused training step has no per-mode scale parameter (AdaptiveCorrector): "
-                                      "train it through the autograd-capable methods instead")
         x_feats = self._dev_f32(x_feats)
-        if self.model_type == 'simple':
+        if self.model_type in ('simple', 'adaptive'):
             h = self.model.corrector_input(x_feats, edge_index.to(self.device))
         else:
             h = self.model.corrector_input(x_feats, A_norm)
         linears = [m for m in self.model.net if isinstance(m, nn.Linear)]
-        params = _engine.FlatParams.adopt(linears)
+        params = _engine.FlatParams.adopt(linears, mode_scales=getattr(self.model, "mode_scales", None))
         group = optimizer.param_groups[0]
         cfg = _engine.StepConfig(lr=group['lr'], weight_decay=group['weight_decay'], corr_scale=self.corr_scale,
                                  w_res=self.w_res, w_orth=self.w_orth, w_trace=self.w_trace, w_order=self.w_order,
                                  w_eigen=self.w_eigen, grad_clip=self.grad_clip, beta1=group['betas'][0],
-                                 beta2=group['betas'][1], eps=group['eps'])
+                                 beta2=group['betas'][1], eps=group['eps'], w_smooth=self.w_smooth,
+                                 w_smooth_corr=self.w_smooth_corr)
         pairs = [self._pair(K, M) for K, M in zip(K_list, M_list)]
         return _engine.TrainStepEngine(h, self._dev_f32(U_base), pairs, node_offsets, params, cfg,
                                        lam_target=lambda_target, mlp_mode=self.mlp_mode)
@@ -242,7 +247,7 @@ class MultigridGNN:
 
     def _forward_pass(self, x_feats, edge_index, A_norm):
         x_feats = x_feats.to(self.device)
-        if self.model_type == 'simple':
+        if self.model_type in ('simple', 'adaptive'):
             return self.model(x_feats, edge_index.to(self.device))
         return self.model(x_feats, A_norm)
 

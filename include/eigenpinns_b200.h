@@ -216,6 +216,29 @@ EP_API int ep_scale_columns_rsqrt_f32(int n, int k, const float* U, int ldu, con
 EP_API int ep_axpy_out_f32(size_t n, float alpha, const float* alpha_dev, const float* a, const float* b,
                     float* out, ep_stream_t stream);
 
+/* ---- learnable per-mode scales and the smoothness of the correction -------------------------
+ * AdaptiveCorrector of delta_pinns_validation/multigrid_gnn_refine_fixed.ipynb cell 4: corr = c o s (c: raw MLP output,
+ * n x k; s: k scales, column scaling), U_pred = U_base + sigma corr, and the `train_gnn` term
+ *   L_sc = w / (n_global k) sum_ij corr_ij (K corr)_ij = w / (n_global k) sum_j s_j^2 P_j,  P_j = sum_i c_ij (K c)_ij
+ * (K symmetric, K (c o s) = (K c) o s: only K c is formed, with ep_spmm_csr_f32).  k <= 256.
+ * Forward: U_pred = U_base + sigma * (c o s), rounded product by product (c s, then sigma (c s), then the sum; with
+ * s == NULL bit-identical to ep_axpy_out_f32).  s == NULL means unit scales; sigma_dev (device float, may be NULL)
+ * overrides sigma (graph-capturable ramp).  16-byte accesses when k % 4 == 0 and rows are 16-byte aligned. */
+EP_API int ep_mode_scale_fwd_f32(int n, int k, const float* c, int ldc, const float* U_base, int ldb, const float* s,
+                          float sigma, const float* sigma_dev, float* U_pred, int ldu, ep_stream_t stream);
+/* Backward, per level.  dcorr holds g = dL/dcorr from the eigen-loss backward (sigma already applied) and is rewritten
+ * in place to dL/dc, with w2 = 2 w_smooth_corr / (n_global k):
+ *   dcorr_ij <- s_j g_ij + w2 s_j^2 (K c)_ij
+ *   grad_s_j  = sum_i c_ij g_ij + w2 s_j P_j          (accumulate = 0: "=", first level of a step; 1: "+=")
+ *   loss_acc[8] and loss_acc[5] += L_sc
+ * Kc == NULL (w_smooth_corr = 0) skips the smoothness part; s == NULL means unit scales, grad_s must then be NULL.
+ * One streaming pass writes per-CTA fp64 column sums to the workspace (ep_mode_scale_bwd_workspace_bytes(k)), one CTA
+ * reduces them in a fixed order: deterministic, no host synchronisation (graph-capturable).  2 launches. */
+EP_API size_t ep_mode_scale_bwd_workspace_bytes(int k);
+EP_API int ep_mode_scale_bwd_f32(int n, int k, double n_global, const float* c, int ldc, const float* Kc, int ldkc,
+                          const float* s, float w_smooth_corr, float* dcorr, int ldd, float* grad_s, int accumulate,
+                          double* loss_acc, void* workspace, size_t workspace_bytes, ep_stream_t stream);
+
 /* ---- corrector MLP, fp32 SIMT path ("parity mode"): corrector_model.py:12-21,31 ---------
  * Y = act(X W^T + b), W: out x in row-major (nn.Linear layout), act: 0 none, 1 ReLU. */
 EP_API int ep_linear_fwd_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* b,
