@@ -13,7 +13,7 @@ Package layout
 """
 from . import _cabi
 
-__version__ = "0.3.0"
+__version__ = "0.4.0"
 
 
 def library_version():

@@ -38,7 +38,6 @@ SIGNATURES = {
                                       c_p]),
     "ep_loss_add_sum_f64": (c_int, [c_int, c_p, c_d, c_int, c_p, c_p]),
     "ep_eigen_bwd_prepare_f32": (c_int, [c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_p, c_p, c_p, c_p]),
-    "ep_eigen_bwd_fused_sym_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_f, c_p, c_p, c_int, c_p]),
     "ep_eigen_bwd_fused_sym_rows_f32": (c_int, [c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_f, c_p, c_p,
                                                 c_int, c_p]),
     "ep_eigen_bwd_gram_term_tf32x3": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_f, c_p, c_p, c_int, c_p]),
@@ -103,7 +102,7 @@ _lib = None
 # kernels launched by one call of each entry point (for bench.py's "gpu_launches" claim)
 KERNELS_PER_CALL = {
     "ep_spmm_csr_f32": 1, "ep_spmm2_csr_f32": 1, "ep_spmm2_sum_csr_f32": 1, "ep_neighbor_mean_concat_f32": 1,
-    "ep_spmm_concat_f32": 2, "ep_eigen_partials_f32": 2, "ep_eigen_finalize_f32": 1, "ep_loss_add_sum_f64": 1, "ep_eigen_bwd_prepare_f32": 1, "ep_eigen_bwd_fused_sym_f32": 1, "ep_eigen_bwd_fused_sym_rows_f32": 1, "ep_eigen_bwd_gram_term_tf32x3": 1, "ep_eigen_bwd_gather_sym_rows_f32": 1,
+    "ep_spmm_concat_f32": 2, "ep_eigen_partials_f32": 2, "ep_eigen_finalize_f32": 1, "ep_loss_add_sum_f64": 1, "ep_eigen_bwd_prepare_f32": 1, "ep_eigen_bwd_fused_sym_rows_f32": 1, "ep_eigen_bwd_gram_term_tf32x3": 1, "ep_eigen_bwd_gather_sym_rows_f32": 1,
     "ep_scale_columns_rsqrt_f32": 1, "ep_axpy_out_f32": 1, "ep_linear_fwd_f32": 1, "ep_linear_bwd_f32": 5,
     "ep_grad_sqnorm_f32": 2, "ep_adam_clip_step_f32": 1, "ep_fps_f64": 1, "ep_bounds_f64": 2,
     "ep_voxel_select_f64": 6, "ep_gather_rows_f32": 1, "ep_knn_grid_f64": 1, "ep_fem_elements_f64": 1, "ep_fem_segment_sum_f64": 1, "ep_scatter_add_rows_f32": 1,

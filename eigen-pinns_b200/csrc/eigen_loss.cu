@@ -9,6 +9,7 @@
 // The Gram matrix is accumulated in fp32 for at most four 32-row tiles and then folded into fp64.
 // Algorithmic traffic of the partials kernel: 12 n k bytes read, flops 2 n k^2 + 8 n k.
 #include "ep_common.cuh"
+#include "eigen_coef.cuh"
 
 namespace {
 
@@ -323,31 +324,28 @@ eigen_finalize_kernel(int k, double n_global, const double* __restrict__ P, floa
   const double ord_sum = block_sum_256(ordr, scratch);
   const double eig_sum = block_sum_256(eig, scratch);
   const double c_res = 2.0 * (double)w_res / (n_global * (double)k);
-  float* c_lam = coef + 1;
-  float* c_num = c_lam + k;
-  float* c_den = c_num + k;
-  float* c_G = c_den + k;
+  const ep::Coef<float> cf(coef, k);
   double den_bar_j = 0.0;
   if (tid < k) {
     double lam_bar = -c_res * (sKM[tid] - lam_j * sMM[tid]) + extra_bar;
     if (lam_bar_extra != nullptr) lam_bar += (double)lam_bar_extra[tid];
     const double num_bar = lam_bar / den_j + (double)w_smooth / (n_global * (double)k);
     den_bar_j = -lam_bar * lam_j / den_j;
-    c_lam[tid] = (float)lam_j;
-    c_num[tid] = (float)num_bar;
-    c_den[tid] = (float)den_bar_j;
+    cf.lam[tid] = (float)lam_j;
+    cf.num_bar[tid] = (float)num_bar;
+    cf.den_bar[tid] = (float)den_bar_j;
     if (lam_out) lam_out[tid] = (float)lam_j;
     // dL/d(MU)_ij of the zero-mean term is the same for every row i: g_j = 2 w_mean (1^T M u_j) / (k - 1)
-    coef[1 + 3 * k + k * k + tid] = (tid >= 1 && k > 1) ? (float)(2.0 * (double)w_mean * sMU[tid] / (double)(k - 1)) : 0.f;
+    cf.g_mean[tid] = (tid >= 1 && k > 1) ? (float)(2.0 * (double)w_mean * sMU[tid] / (double)(k - 1)) : 0.f;
   }
   __syncthreads();
   const double go = 2.0 * (double)w_orth / (double)k;
   for (int e = tid; e < k * k; e += 256) {
     const int a = e / k, b = e - a * k;
-    c_G[e] = (float)(go * (G[e] - (a == b ? 1.0 : 0.0)));   // den_bar is applied separately (coef)
+    cf.G_bar[e] = (float)(go * (G[e] - (a == b ? 1.0 : 0.0)));   // den_bar is applied separately (coef)
   }
   if (tid == 0) {
-    coef[0] = (float)c_res;
+    *cf.c_res = (float)c_res;
     const double t0 = (double)w_res * L_res, t1 = (double)w_orth * L_orth;
     const double t2 = (double)w_trace * tr_sum, t3 = (double)w_order * ord_sum, t4 = (double)w_eigen * eig_sum;
     const double t7 = (double)w_mean * mean_sum, t8 = (double)w_smooth * smooth_sum;
@@ -381,25 +379,21 @@ eigen_bwd_prepare_kernel(int n, int k, const float* __restrict__ U, int ldu, con
   float* s_lam = MUs + R * TP;                  // KP
   float* s_a = s_lam + KP;                      // KP   (num_bar)
   const int tid = threadIdx.x;
-  const float c_res = coef[0];
-  const float* c_lam = coef + 1;
-  const float* c_num = c_lam + k;
-  const float* c_den = c_num + k;
-  const float* c_G = c_den + k;
-  const float* c_mean = c_G + k * k;
+  const ep::Coef<const float> cf(coef, k);
+  const float c_res = *cf.c_res;
   for (int e = tid; e < KP * KP; e += 256) {
     const int a = e / KP, b = e - a * KP;
     float g = 0.f;
     if (a < k && b < k) {
-      g = c_G[a * k + b];
-      if (a == b) g += c_den[a];
+      g = cf.G_bar[a * k + b];
+      if (a == b) g += cf.den_bar[a];
     }
     Gs[a * GP + b] = g;
     GTs[b * GP + a] = g;
   }
   for (int e = tid; e < KP; e += 256) {
-    s_lam[e] = e < k ? c_lam[e] : 0.f;
-    s_a[e] = e < k ? c_num[e] : 0.f;
+    s_lam[e] = e < k ? cf.lam[e] : 0.f;
+    s_a[e] = e < k ? cf.num_bar[e] : 0.f;
   }
   constexpr int CG = KP / 4;                    // column groups
   const int tc = tid % CG, tr = tid / CG;       // tr in [0, R/4)
@@ -448,7 +442,7 @@ eigen_bwd_prepare_kernel(int n, int k, const float* __restrict__ U, int ldu, con
         const float lam = s_lam[c], a = s_a[c];
         const float rbar = c_res * (ku - lam * mu);
         KU_bar[(size_t)row * ld + c] = rbar + a * u;
-        MU_bar[(size_t)row * ld + c] = acc1[i][j] - lam * rbar + c_mean[c];
+        MU_bar[(size_t)row * ld + c] = acc1[i][j] - lam * rbar + cf.g_mean[c];
         D[(size_t)row * ld + c] = fmaf(a, ku, acc2[i][j]);
       }
     }
@@ -476,19 +470,10 @@ eigen_bwd_fused_sym_kernel(int row0, int n, int k, int lpr_shift, const int32_t*
   float* S = fsm;                 // k x k
   float* s_lam = S + k * k;       // k
   float* s_a2 = s_lam + k;        // k
-  const float c_res = coef[0];
-  const float* c_lam = coef + 1;
-  const float* c_num = c_lam + k;
-  const float* c_den = c_num + k;
-  const float* c_G = c_den + k;
-  for (int e = threadIdx.x; e < k * k; e += blockDim.x) {
-    const int m = e / k, j = e - m * k;
-    float v = c_G[e] + c_G[j * k + m];
-    if (m == j) v += 2.f * c_den[m];
-    S[e] = v;
-  }
-  const float* c_mean = c_G + k * k;
-  for (int e = threadIdx.x; e < k; e += blockDim.x) { s_lam[e] = c_lam[e]; s_a2[e] = 2.f * c_num[e]; }
+  const ep::Coef<const float> cf(coef, k);
+  const float c_res = *cf.c_res;
+  for (int e = threadIdx.x; e < k * k; e += blockDim.x) S[e] = ep::coef_sym_entry(cf, k, e);
+  for (int e = threadIdx.x; e < k; e += blockDim.x) { s_lam[e] = cf.lam[e]; s_a2[e] = 2.f * cf.num_bar[e]; }
   __syncthreads();
 
   const int lpr = 1 << lpr_shift;
@@ -498,7 +483,8 @@ eigen_bwd_fused_sym_kernel(int row0, int n, int k, int lpr_shift, const int32_t*
   const int cofs = active ? 4 * lane_r : 0;
   const float4 lam4 = *reinterpret_cast<const float4*>(s_lam + cofs);
   const float4 a24 = *reinterpret_cast<const float4*>(s_a2 + cofs);
-  const float4 gm4 = make_float4(__ldg(c_mean + cofs), __ldg(c_mean + cofs + 1), __ldg(c_mean + cofs + 2), __ldg(c_mean + cofs + 3));
+  const float4 gm4 = make_float4(__ldg(cf.g_mean + cofs), __ldg(cf.g_mean + cofs + 1), __ldg(cf.g_mean + cofs + 2),
+                                 __ldg(cf.g_mean + cofs + 3));
   const long long groups_per_grid = ((long long)gridDim.x * blockDim.x) >> lpr_shift;
   for (long long ri = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> lpr_shift;
        ri < (long long)((n + groups_per_grid - 1) / groups_per_grid) * groups_per_grid; ri += groups_per_grid) {
@@ -646,7 +632,7 @@ size_t ep_eigen_partials_workspace_bytes(int k) {
   return sizeof(double) * (size_t)partials_len(k) * (size_t)(ep::sm_count() * 4);
 }
 
-size_t ep_eigen_coef_len(int k) { return k > 0 ? (size_t)(1 + 4 * k + k * k) : 0; }
+size_t ep_eigen_coef_len(int k) { return k > 0 ? (size_t)ep::coef_len(k) : 0; }
 
 int ep_eigen_partials_f32(int n, int k, const float* U, int ldu, const float* KU, const float* MU, int ld,
                           double* out, void* workspace, size_t workspace_bytes, ep_stream_t stream) {
@@ -730,13 +716,6 @@ int ep_eigen_bwd_prepare_f32(int n, int k, const float* U, int ldu, const float*
   if (k <= 32) return launch_bwd_prepare<32>(n, k, U, ldu, KU, MU, ld, coef, KU_bar, MU_bar, D, st);
   if (k <= 64) return launch_bwd_prepare<64>(n, k, U, ldu, KU, MU, ld, coef, KU_bar, MU_bar, D, st);
   return launch_bwd_prepare<128>(n, k, U, ldu, KU, MU, ld, coef, KU_bar, MU_bar, D, st);
-}
-
-int ep_eigen_bwd_fused_sym_f32(int n, int k, const int32_t* rowptr, const int32_t* col, const float* valK,
-                               const float* valM, const float* KU, const float* MU, int ld, const float* coef,
-                               float out_scale, const float* out_scale_dev, float* dU, int ldo, ep_stream_t stream) {
-  return ep_eigen_bwd_fused_sym_rows_f32(0, n, k, rowptr, col, valK, valM, KU, MU, ld, coef, out_scale, out_scale_dev,
-                                         dU, ldo, stream);
 }
 
 int ep_eigen_bwd_fused_sym_rows_f32(int row0, int n, int k, const int32_t* rowptr, const int32_t* col,

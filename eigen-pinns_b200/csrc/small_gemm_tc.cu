@@ -10,7 +10,10 @@
 // accumulated in fp32 in TMEM.  One 128-vertex tile per CTA iteration: rows are loaded from HBM coalesced, split and
 // written to shared memory in the canonical no-swizzle K-major layout (8 rows x 16 B core matrices, the same layout
 // mlp_tc.cu uses with 2-byte elements), 3 k/8 MMAs, accumulator drained row-per-thread.  HBM-bound: 8 n k bytes.
+// Built for k = 64 only: at k = 32 the SIMT product of the one-pass backward hides behind its gather (B200, 1 M
+// vertices: 0.45 ms for the one-pass kernel against 0.54 ms for this kernel + the gather pass).
 #include "tc_common.cuh"
+#include "eigen_coef.cuh"
 
 namespace {
 
@@ -29,26 +32,18 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
       "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
 }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-        "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 __device__ __forceinline__ float tf32_hi(float x) { return __uint_as_float(__float_as_uint(x) & 0xFFFFE000u); }
 
-// K = number of columns of X = order of S (multiple of 16, <= 64); one CTA handles tiles blockIdx.x, + gridDim.x, ...
+// K = number of columns of X = order of S; one CTA handles tiles blockIdx.x, + gridDim.x, ...
 template <int K>
 __global__ void __launch_bounds__(SG_THREADS)
 rows_times_sym_tf32x3_kernel(int row0, int n, const float* __restrict__ X, int ldx, const float* __restrict__ coef,
                              float out_scale_v, const float* __restrict__ out_scale_dev, float* __restrict__ T, int ldt) {
+  static_assert(K == 64, "the drain reads 32 accumulator columns per half");
   constexpr int KC = K / 4;                          // 16-byte chunks (4 fp32) along K
   constexpr uint32_t A_BYTES = TILE_M * K * 4;
   constexpr uint32_t B_BYTES = K * K * 4;
-  constexpr uint32_t TM_COLS = K <= 32 ? 32 : 64;    // power of two >= 32
+  constexpr uint32_t TM_COLS = K;                    // power of two >= 32
   extern __shared__ __align__(128) uint8_t smem[];
   uint8_t* A_hi = smem;
   uint8_t* A_lo = A_hi + A_BYTES;
@@ -62,18 +57,14 @@ rows_times_sym_tf32x3_kernel(int row0, int n, const float* __restrict__ X, int l
   if (threadIdx.x == 0) { mbar_init(done, 1); fence_barrier_init(); }
   if (warp == 0) tmem_alloc(tmem_slot, TM_COLS);
   // S = Gp + Gp^T from the finalize coefficients; B[n][kk] = S[kk][n] = S[n][kk], K-major, chunk-major in shared memory
-  {
-    const float* c_den = coef + 1 + 2 * K;
-    const float* c_G = c_den + K;
-    for (int e = threadIdx.x; e < K * K; e += SG_THREADS) {
-      const int nn = e / K, kk = e - nn * K;
-      float v = __ldg(c_G + nn * K + kk) + __ldg(c_G + kk * K + nn);
-      if (nn == kk) v += 2.f * __ldg(c_den + nn);
-      const float hi = tf32_hi(v);
-      const uint32_t off = (uint32_t)(kk >> 2) * (K * 16) + (uint32_t)nn * 16 + (uint32_t)(kk & 3) * 4;
-      *reinterpret_cast<float*>(B_hi + off) = hi;
-      *reinterpret_cast<float*>(B_lo + off) = v - hi;
-    }
+  const ep::Coef<const float> cf(coef, K);
+  for (int e = threadIdx.x; e < K * K; e += SG_THREADS) {
+    const int nn = e / K, kk = e - nn * K;
+    const float v = ep::coef_sym_entry(cf, K, e);
+    const float hi = tf32_hi(v);
+    const uint32_t off = (uint32_t)(kk >> 2) * (K * 16) + (uint32_t)nn * 16 + (uint32_t)(kk & 3) * 4;
+    *reinterpret_cast<float*>(B_hi + off) = hi;
+    *reinterpret_cast<float*>(B_lo + off) = v - hi;
   }
   tc_fence_before();
   __syncthreads();
@@ -120,27 +111,16 @@ rows_times_sym_tf32x3_kernel(int row0, int n, const float* __restrict__ X, int l
     {
       const int q = warp & 3, half = warp >> 2;
       const long long row = (long long)tile * TILE_M + q * 32 + lane;
-      constexpr int CPH = K / 2;                       // columns per half: 8, 16, 24 or 32
+      constexpr int CPH = K / 2;                       // columns per half
       const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(half * CPH);
       float* dst = T + (size_t)(row0 + row) * ldt + half * CPH;
-      if constexpr (CPH == 32) {
-        uint32_t v[32];
-        tmem_ld32(t_addr, v);
-        if (row < n) {
+      uint32_t v[32];
+      tmem_ld32(t_addr, v);
+      if (row < n) {
 #pragma unroll
-          for (int j = 0; j < 8; ++j)
-            reinterpret_cast<float4*>(dst)[j] = make_float4(out_scale * __uint_as_float(v[4 * j]), out_scale * __uint_as_float(v[4 * j + 1]),
-                                                            out_scale * __uint_as_float(v[4 * j + 2]), out_scale * __uint_as_float(v[4 * j + 3]));
-        }
-      } else {
-        uint32_t v[16];
-        tmem_ld16(t_addr, v);                          // CPH = 8 / 16 (24 is not instantiated): extra columns are ignored
-        if (row < n) {
-#pragma unroll
-          for (int j = 0; j < CPH / 4; ++j)
-            reinterpret_cast<float4*>(dst)[j] = make_float4(out_scale * __uint_as_float(v[4 * j]), out_scale * __uint_as_float(v[4 * j + 1]),
-                                                            out_scale * __uint_as_float(v[4 * j + 2]), out_scale * __uint_as_float(v[4 * j + 3]));
-        }
+        for (int j = 0; j < 8; ++j)
+          reinterpret_cast<float4*>(dst)[j] = make_float4(out_scale * __uint_as_float(v[4 * j]), out_scale * __uint_as_float(v[4 * j + 1]),
+                                                          out_scale * __uint_as_float(v[4 * j + 2]), out_scale * __uint_as_float(v[4 * j + 3]));
       }
     }
     tc_fence_before();
@@ -160,8 +140,7 @@ int launch_rows_times_sym(int row0, int n, const float* X, int ldx, const float*
     configured = true;
   }
   const int n_tiles = (n + TILE_M - 1) / TILE_M;
-  const int per_sm = K <= 16 ? 6 : (K <= 32 ? 4 : 2);            // resident CTAs per SM (shared memory / TMEM columns)
-  int grid = ep::sm_count() * per_sm;
+  int grid = ep::sm_count() * 2;                                  // resident CTAs per SM (shared memory / TMEM columns)
   if (grid > n_tiles) grid = n_tiles;
   rows_times_sym_tf32x3_kernel<K><<<grid, SG_THREADS, smem, st>>>(row0, n, X, ldx, coef, scale, scale_dev, T, ldt);
   EP_LAUNCH_CHECK("rows_times_sym_tf32x3_kernel");
@@ -177,14 +156,11 @@ int ep_eigen_bwd_gram_term_tf32x3(int row0, int n_rows, int k, const float* MU, 
   EP_REQUIRE(n_rows >= 0 && row0 >= 0 && k > 0, "bad size");
   if (n_rows == 0) return EP_OK;
   EP_REQUIRE(MU && coef && dU, "null pointer");
-  if ((k != 16 && k != 32 && k != 64) || ld % 4 != 0 || ldo % 4 != 0 || !ep::aligned16(MU) || !ep::aligned16(dU)) {
-    ep::set_error("ep_eigen_bwd_gram_term_tf32x3: k must be 16, 32 or 64 and rows 16-byte aligned");
+  if (k != 64 || ld % 4 != 0 || ldo % 4 != 0 || !ep::aligned16(MU) || !ep::aligned16(dU)) {
+    ep::set_error("ep_eigen_bwd_gram_term_tf32x3: k must be 64 and rows 16-byte aligned");
     return EP_ERR_UNSUPPORTED;
   }
-  cudaStream_t st = ep::as_stream(stream);
-  if (k == 16) return launch_rows_times_sym<16>(row0, n_rows, MU, ld, coef, out_scale, out_scale_dev, dU, ldo, st);
-  if (k == 32) return launch_rows_times_sym<32>(row0, n_rows, MU, ld, coef, out_scale, out_scale_dev, dU, ldo, st);
-  return launch_rows_times_sym<64>(row0, n_rows, MU, ld, coef, out_scale, out_scale_dev, dU, ldo, st);
+  return launch_rows_times_sym<64>(row0, n_rows, MU, ld, coef, out_scale, out_scale_dev, dU, ldo, ep::as_stream(stream));
 }
 
 }  // extern "C"

@@ -187,6 +187,10 @@ class ShardedTrainStepEngine(TrainStepEngine):
         self.overlap_grads = self.n_mlp >= 1_000_000
         self.dCorr.zero_()                      # halo rows never receive a gradient on this rank
 
+    def add_projection_term(self, level, P, U_coarse, w_proj):
+        raise NotImplementedError("the vertex-sharded step has no projection term: it would need the rank-local rows of "
+                                  "the prolongation and its transpose; use the single-GPU TrainStepEngine")
+
     def _mlp_rows(self):
         # single level: rows are [owned | halo], and the corrector is only needed on the owned ones (the halo rows
         # of U_pred arrive through the exchange).  Stacked levels interleave owned and halo blocks: evaluate all.
@@ -245,17 +249,14 @@ class ShardedTrainStepEngine(TrainStepEngine):
         gradient of the interior rows is computed while it is in flight."""
         for li, (pl, pair) in enumerate(zip(self.plans, self.pairs)):
             s = self._level_slices(li)
-            if not ops.eigen_bwd_fused_ok(pair, self.k, self.KU[s], self.MU[s], self.dCorr[s]):
-                raise NotImplementedError("the vertex-sharded backward uses the fused symmetric kernel: k must be a "
-                                          "multiple of 4 (<= 128)")
             pending = self.halo[li].start(self._ext(self.KUMU, li), pl.n_own)
             a, b = pl.interior if self.overlap else (0, 0)
-            args = (pair, self.KU[s], self.MU[s], self.coefs[li], scale, self.dCorr[s], scale_dev)
-            ops.eigen_bwd_fused(*args, rows=(a, b))
+            args = (pair, self.U_pred[s], self.KU[s], self.MU[s], self.coefs[li], scale, self.dCorr[s], scale_dev)
+            ops.eigen_loss_bwd(*args, rows=(a, b))
             for w in pending:
                 w.wait()
-            ops.eigen_bwd_fused(*args, rows=(0, a))
-            ops.eigen_bwd_fused(*args, rows=(b, pl.n_own))
+            ops.eigen_loss_bwd(*args, rows=(0, a))
+            ops.eigen_loss_bwd(*args, rows=(b, pl.n_own))
 
 
 def shard_rows(global_rows, plans, global_offsets):

@@ -170,7 +170,6 @@ class TrainStepEngine:
                 self.Kc = torch.empty((self.n_mlp, k), **f32)
         self.launches_per_step = None
         self.use_graph, self._graph, self.hyper = False, None, None
-        self.fused_bwd = True          # symmetric operators: one-pass analytic backward
 
     # ---- pieces (also used one by one by the tests)
     def add_projection_term(self, level, P, U_coarse, w_proj):
@@ -240,20 +239,18 @@ class TrainStepEngine:
         for li, term in self.projections.items():
             term.forward(self.U_pred[self._level_slices(li)], self.loss_acc)
 
+    def _bwd_scratch_rows(self, s):
+        """KU_bar, MU_bar, D rows of level slice s for the general backward, allocated on first use."""
+        if self._bwd_scratch is None:                 # same row stride as KU / MU (halves of the interleaved rows)
+            two = torch.empty_like(self.KUMU)
+            self._bwd_scratch = [two[:, :self.k], two[:, self.k:], torch.empty_like(self.KUMU)[:, :self.k]]
+        return [t[s] for t in self._bwd_scratch]
+
     def loss_backward(self, scale, scale_dev=None):
         for li, pair in enumerate(self.pairs):
             s = self._level_slices(li)
-            if self.fused_bwd and ops.eigen_bwd_fused_ok(pair, self.k, self.KU[s], self.MU[s], self.dCorr[s]):
-                ops.eigen_bwd_fused(pair, self.KU[s], self.MU[s], self.coefs[li], scale, self.dCorr[s], scale_dev)
-                if li in self.projections:
-                    self.projections[li].backward(self.dCorr[s], scale, scale_dev)
-                continue
-            if self._bwd_scratch is None:             # same row stride as KU / MU (halves of the interleaved rows)
-                two = torch.empty_like(self.KUMU)
-                self._bwd_scratch = [two[:, :self.k], two[:, self.k:], torch.empty_like(self.KUMU)[:, :self.k]]
-            KU_bar, MU_bar, D = self._bwd_scratch
-            ops.eigen_bwd_prepare(self.U_pred[s], self.KU[s], self.MU[s], self.coefs[li], KU_bar[s], MU_bar[s], D[s])
-            ops.spmm2_sum(pair.KT, pair.MT, KU_bar[s], MU_bar[s], D[s], scale, out=self.dCorr[s], scale_dev=scale_dev)
+            ops.eigen_loss_bwd(pair, self.U_pred[s], self.KU[s], self.MU[s], self.coefs[li], scale, self.dCorr[s],
+                               scale_dev, scratch=lambda: self._bwd_scratch_rows(s))
             if li in self.projections:
                 self.projections[li].backward(self.dCorr[s], scale, scale_dev)
         if self.adaptive:

@@ -209,42 +209,38 @@ def eigen_bwd_prepare(U, KU, MU, coef, KU_bar=None, MU_bar=None, D=None):
     return KU_bar, MU_bar, D
 
 
-# k x k term of the backward on the tensor cores (tcgen05 kind::tf32, 3 passes) instead of SIMT shuffles, for
-# k >= TENSOR_CORE_GRAM_MIN_K; below it the one-kernel SIMT form runs
-TENSOR_CORE_GRAM = True
-# measured on B200: at k = 32 the SIMT product hides behind the gather (0.45 vs 0.54 ms at 1 M vertices), at k = 64 the
-# tensor-core form wins (15.8 vs 16.4 ms at 16.7 M vertices; 21.6 ms before KU / MU were interleaved)
-TENSOR_CORE_GRAM_MIN_K = 64
-
-
-def eigen_bwd_fused_ok(pair, k, *tensors):
-    return (pair.symmetric and k % 4 == 0 and k <= 128
-            and all(t.stride(0) % 4 == 0 and t.data_ptr() % 16 == 0 for t in tensors))
-
-
-def eigen_bwd_fused(pair, KU, MU, coef, scale, out, scale_dev=None, rows=None):
-    """dL/dU for symmetric (K, M) in one gather pass (see ep_eigen_bwd_fused_sym_f32).  KU / MU hold every row the
-    pattern references (owned and halo); rows=(a, b) restricts the OUTPUT rows (interior / boundary split)."""
+def eigen_loss_bwd(pair, U, KU, MU, coef, scale, out, scale_dev=None, rows=None, scratch=None):
+    """out = scale * dL/dU of one level (scale_dev: device scalar that overrides scale) from K U, M U and the coefficients
+    of eigen_finalize.  Symmetric (K, M), k % 4 == 0, k <= 128 and 16-byte aligned rows of KU, MU and out: one gather
+    pass over the pattern, reading every row of KU / MU the pattern references (owned and halo).  Otherwise
+    eigen_bwd_prepare + the transposed dual SpMM; scratch, if given, is called on that path only and returns the
+    (KU_bar, MU_bar, D) buffers to use (default: new ones per call).  rows=(a, b) restricts the OUTPUT rows to that range
+    (one-pass form only): the sharded engine computes the interior rows while the halo rows of KU / MU are in flight."""
     k = KU.shape[1]
-    n = out.shape[0]
     assert KU.stride(0) == MU.stride(0)
-    a, b = (0, n) if rows is None else rows
+    if not (pair.symmetric and k % 4 == 0 and k <= 128
+            and all(t.stride(0) % 4 == 0 and t.data_ptr() % 16 == 0 for t in (KU, MU, out))):
+        if rows is not None:
+            raise NotImplementedError("a row range needs the one-pass backward: symmetric K, M and k a multiple of 4 "
+                                      "(<= 128)")
+        KU_bar, MU_bar, D = eigen_bwd_prepare(U, KU, MU, coef, *(scratch() if scratch is not None else ()))
+        return spmm2_sum(pair.KT, pair.MT, KU_bar, MU_bar, D, scale, out=out, scale_dev=scale_dev)
+    a, b = (0, out.shape[0]) if rows is None else rows
     if b <= a:
         return out
-    # the kernel reads row i of KU / MU for output row i: shift those base pointers together with the output;
-    # gathered neighbours are addressed from the unshifted bases through absolute column indices, so the shifted
-    # call passes the column-relative bases explicitly (gather base = row 0)
-    if TENSOR_CORE_GRAM and k in (16, 32, 64) and k >= TENSOR_CORE_GRAM_MIN_K:
-        # k x k product on the tensor cores (TF32 x 3, fp32 accuracy), then the gather pass adds the sparse terms
+    # the kernels read row i of KU / MU for output row i and gather neighbours through absolute column indices, so all
+    # pointers keep their row-0 bases and the range is passed as (row0, n_rows)
+    gather = (a, b - a, k, _ptr(pair.K.rowptr), _ptr(pair.K.col), _ptr(pair.K.val), _ptr(pair.M.val), _ptr(KU),
+              _ptr(MU), KU.stride(0), _ptr(coef), float(scale), _ptr(scale_dev), _ptr(out), out.stride(0))
+    if k == 64:
+        # k x k product on the tensor cores (TF32 x 3, fp32 accuracy), then the gather pass adds the sparse terms.
+        # Measured on B200: at k = 64 this wins (15.8 vs 16.4 ms at 16.7 M vertices); at k = 32 the SIMT product of the
+        # one-kernel form hides behind the gather (0.45 vs 0.54 ms at 1 M vertices)
         call("ep_eigen_bwd_gram_term_tf32x3", a, b - a, k, _ptr(MU), MU.stride(0), _ptr(coef), float(scale),
              _ptr(scale_dev), _ptr(out), out.stride(0), _stream())
-        call("ep_eigen_bwd_gather_sym_rows_f32", a, b - a, k, _ptr(pair.K.rowptr), _ptr(pair.K.col), _ptr(pair.K.val),
-             _ptr(pair.M.val), _ptr(KU), _ptr(MU), KU.stride(0), _ptr(coef), float(scale), _ptr(scale_dev), _ptr(out),
-             out.stride(0), 1, _stream())
-        return out
-    call("ep_eigen_bwd_fused_sym_rows_f32", a, b - a, k, _ptr(pair.K.rowptr), _ptr(pair.K.col), _ptr(pair.K.val),
-         _ptr(pair.M.val), _ptr(KU), _ptr(MU), KU.stride(0), _ptr(coef), float(scale), _ptr(scale_dev), _ptr(out),
-         out.stride(0), _stream())
+        call("ep_eigen_bwd_gather_sym_rows_f32", *gather, 1, _stream())
+    else:
+        call("ep_eigen_bwd_fused_sym_rows_f32", *gather, _stream())
     return out
 
 
@@ -392,12 +388,7 @@ class _EigenLossFn(torch.autograd.Function):
             U = U_pred[off:off + pair.n]
             extra = g_lams[li].contiguous() if (li < len(g_lams) and g_lams[li] is not None) else None
             _, coef = eigen_finalize(k, pair.n, P, w_res * gr, w_orth * go, scratch_acc, lam_bar_extra=extra)
-            dst = dU[off:off + pair.n]
-            if eigen_bwd_fused_ok(pair, k, KU, MU, dst):
-                eigen_bwd_fused(pair, KU, MU, coef, 1.0, dst)
-            else:
-                KU_bar, MU_bar, D = eigen_bwd_prepare(U, KU, MU, coef)
-                spmm2_sum(pair.KT, pair.MT, KU_bar, MU_bar, D, 1.0, out=dst)
+            eigen_loss_bwd(pair, U, KU, MU, coef, 1.0, dU[off:off + pair.n])
         return dU, None, None, None, None
 
 

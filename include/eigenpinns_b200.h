@@ -180,14 +180,10 @@ EP_API int ep_eigen_bwd_prepare_f32(int n, int k, const float* U, int ldu, const
  *   dU = out_scale * [ c_res * sum_j (K_ij - lam M_ij)(KU_j - lam MU_j) + 2 num_bar KU_i + MU_i (Gp + Gp^T)
  *                      + (sum_j M_ij) g_mean ]
  * with Gp = G_bar + diag(den_bar).  Algebraically equal to prepare + ep_spmm2_sum_csr_f32 when K = K^T,
- * M = M^T.  Needs k % 4 == 0, k <= 128, 16-byte aligned rows (EP_ERR_UNSUPPORTED otherwise). */
-EP_API int ep_eigen_bwd_fused_sym_f32(int n, int k, const int32_t* rowptr, const int32_t* col, const float* valK,
-                               const float* valM, const float* KU, const float* MU, int ld, const float* coef,
-                               float out_scale, const float* out_scale_dev, float* dU, int ldo,
-                               ep_stream_t stream);
-
-/* Same, for the output rows [row0, row0 + n_rows) only (all pointers keep their row-0 bases).  The vertex-sharded step
- * computes the interior rows while the halo rows of KU / MU are in flight, then the boundary rows. */
+ * M = M^T.  Needs k % 4 == 0, k <= 128, 16-byte aligned rows (EP_ERR_UNSUPPORTED otherwise).
+ * Only the output rows [row0, row0 + n_rows) are written (row0 = 0, n_rows = n: all); every pointer keeps its row-0
+ * base.  The vertex-sharded step computes the interior rows while the halo rows of KU / MU are in flight, then the
+ * boundary rows. */
 EP_API int ep_eigen_bwd_fused_sym_rows_f32(int row0, int n_rows, int k, const int32_t* rowptr, const int32_t* col,
                                     const float* valK, const float* valM, const float* KU, const float* MU, int ld,
                                     const float* coef, float out_scale, const float* out_scale_dev, float* dU, int ldo,
@@ -195,9 +191,10 @@ EP_API int ep_eigen_bwd_fused_sym_rows_f32(int row0, int n_rows, int k, const in
 
 /* Two-kernel form of the same backward with the dense k x k product on the TENSOR CORES (tcgen05 kind::tf32, 3-pass
  * hi/lo split = fp32 accuracy, accumulators in TMEM):
- *   1. ep_eigen_bwd_gram_term_tf32x3     dU[row0 .. row0+n) = out_scale * MU_i (Gp + Gp^T)          (k = 16, 32 or 64)
+ *   1. ep_eigen_bwd_gram_term_tf32x3     dU[row0 .. row0+n) = out_scale * MU_i (Gp + Gp^T)          (k = 64 only)
  *   2. ep_eigen_bwd_gather_sym_rows_f32  with gram_in_out = 1: dU += out_scale * (gathered terms), product skipped
- * The one-kernel form spends 53 % (k = 32) to 75 % (k = 64) of its time issuing that product with shuffles. */
+ * The one-kernel form spends 53 % (k = 32) to 75 % (k = 64) of its time issuing that product with shuffles, yet at
+ * k = 32 it is still the faster one: step 1 is built for k = 64 only and returns EP_ERR_UNSUPPORTED for any other k. */
 EP_API int ep_eigen_bwd_gram_term_tf32x3(int row0, int n_rows, int k, const float* MU, int ld, const float* coef,
                                   float out_scale, const float* out_scale_dev, float* dU, int ldo, ep_stream_t stream);
 EP_API int ep_eigen_bwd_gather_sym_rows_f32(int row0, int n_rows, int k, const int32_t* rowptr, const int32_t* col,

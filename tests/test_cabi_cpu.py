@@ -50,6 +50,16 @@ def test_sizes_without_gpu():
     assert cabi.query("ep_eigen_coef_len", 64) == 1 + 4 * 64 + 64 * 64         # c_res | lam | num_bar | den_bar | G_bar | g_mean
 
 
+@pytest.mark.parametrize("k", [k for k in range(4, 129, 4) if k != 64])
+def test_gram_term_tf32x3_accepts_k_64_only(k):
+    """The tensor-core k x k term of the loss backward is built for k = 64 alone: any other k returns EP_ERR_UNSUPPORTED
+    before anything is launched (so no GPU is needed; the pointers are never dereferenced)."""
+    cabi = importlib.import_module("eigen-pinns_b200._cabi")
+    fake = ctypes.c_void_p(256)
+    with pytest.raises(cabi.EpError, match=r"status -3\).*k must be 64"):
+        cabi.call("ep_eigen_bwd_gram_term_tf32x3", 0, 1000, k, fake, 2 * k, fake, 1.0, None, fake, k, None)
+
+
 def test_ops_reject_cpu_tensors():
     import torch
     ops = importlib.import_module("eigen-pinns_b200.ops")

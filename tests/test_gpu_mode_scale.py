@@ -145,7 +145,9 @@ def test_kernel_argument_errors():
 @pytest.mark.parametrize("fused", [True, False])
 def test_loss_level_against_autograd(fused):
     """Mode scales, both smoothness parts, the projection term, fused and unfused eigen-loss backward, on the coarse +
-    bunny pair: loss slots 5 and 8, dL/dc and dL/ds against fp64 autograd."""
+    bunny pair: loss slots 5 and 8, dL/dc and dL/ds against fp64 autograd.  For the unfused (general) backward the same
+    matrices, declared non-symmetric, replace the pairs after construction: the constructor refuses w_smooth_corr on a
+    non-symmetric pair, and since these matrices are symmetric the gradient it protects still holds."""
     import scipy.sparse as sp
     from sklearn.neighbors import NearestNeighbors
     sparse, engine = pkg("sparse"), pkg("engine")
@@ -193,7 +195,8 @@ def test_loss_level_against_autograd(fused):
     eng = engine.TrainStepEngine(h, U_base.to(dev()), [sparse.OperatorPair(Kc, Mc, dev()), sparse.OperatorPair(K, M, dev())],
                                  [0, nc], params, cfg)
     assert eng.adaptive and eng.Kc is not None
-    eng.fused_bwd = fused
+    if not fused:
+        eng.pairs = [sparse.OperatorPair(a, b, dev(), assume_symmetric=False) for a, b in ((Kc, Mc), (K, M))]
     eng.add_projection_term(1, P, U_c, w_proj)
     eng.corr_raw.copy_(c.to(dev()))
     eng.mode_scale_forward(sigma)

@@ -179,20 +179,21 @@ def test_large_mesh_properties():
 
 @pytest.mark.parametrize("k", [16, 32, 64, 128])
 def test_fused_symmetric_backward_equals_general_path(k):
-    """One-pass backward (symmetric K, M) against prepare + transposed dual SpMM, and partials for every tiling."""
+    """One-pass backward (symmetric K, M) against prepare + transposed dual SpMM (the same matrices declared
+    non-symmetric), and partials for every tiling."""
     ops, sparse, engine = pkg("ops"), pkg("sparse"), pkg("engine")
     fem, (K, M), _ = bunny_levels()
-    pair = sparse.OperatorPair(K, M, dev())
+    pairs = [sparse.OperatorPair(K, M, dev()), sparse.OperatorPair(K, M, dev(), assume_symmetric=False)]
+    assert pairs[0].symmetric and not pairs[1].symmetric
     n = K.shape[0]
     g = torch.Generator().manual_seed(k)
     U = (0.3 * torch.randn(n, k, generator=g)).to(dev())
     cfg = engine.StepConfig(w_trace=0.5, w_order=2.0, w_eigen=3.0)
     outs = []
-    for fused in (True, False):
+    for pair in pairs:                                 # one-pass form, then the general path
         eng = engine.TrainStepEngine(torch.zeros(n, 4, device=dev()), U, [pair], [0],
                                      engine.FlatParams([torch.zeros(k, 4)], [torch.zeros(k)], dev()), cfg,
                                      lam_target=torch.linspace(0, 2, k).to(dev()))
-        eng.fused_bwd = fused
         eng.U_pred.copy_(U)
         eng.loss_forward()
         eng.loss_backward(0.7)
@@ -209,11 +210,12 @@ def test_fused_symmetric_backward_equals_general_path(k):
     assert (outs[0][0].cpu() - gref).abs().max().item() <= 5e-5 * gref.abs().max().item()
 
 
-@pytest.mark.parametrize("fused", [True, False])
-def test_notebook_variant_terms_against_autograd(fused):
+@pytest.mark.parametrize("symmetric", [True, False])
+def test_notebook_variant_terms_against_autograd(symmetric):
     """Zero-mean, smoothness and projection terms (SURVEY 8a-bis; notebooks multigrid_gnn_farthest_point_sampling cell 0,
     multigrid_gnn_refine_fixed cells 0 and 4) as flags of the engine's eigen-loss: loss terms and dL/dU against a
-    torch-autograd (fp64) restatement of the notebook formulas on the coarse + bunny pair."""
+    torch-autograd (fp64) restatement of the notebook formulas on the coarse + bunny pair.  symmetric=False declares the
+    operators non-symmetric, so the backward takes the general path instead of the one-pass form."""
     import scipy.sparse as sp
     ops, sparse, engine = pkg("ops"), pkg("sparse"), pkg("engine")
     from sklearn.neighbors import NearestNeighbors
@@ -254,9 +256,10 @@ def test_notebook_variant_terms_against_autograd(fused):
     h = torch.zeros(nc + n, 4, device=dev())
     params = engine.FlatParams([torch.zeros(8, 4), torch.zeros(k, 8)], [torch.zeros(8), torch.zeros(k)], dev())
     cfg = engine.StepConfig(w_res=w_res, w_orth=w_orth, w_mean=w_mean, w_smooth=w_smooth)
-    eng = engine.TrainStepEngine(h, U.to(dev()), [sparse.OperatorPair(Kc, Mc, dev()), sparse.OperatorPair(K, M, dev())],
-                                 [0, nc], params, cfg)
-    eng.fused_bwd = fused
+    assume = None if symmetric else False
+    pairs = [sparse.OperatorPair(a, b, dev(), assume_symmetric=assume) for a, b in ((Kc, Mc), (K, M))]
+    assert all(p.symmetric == symmetric for p in pairs)
+    eng = engine.TrainStepEngine(h, U.to(dev()), pairs, [0, nc], params, cfg)
     eng.add_projection_term(1, P, U_c, w_proj)
     eng.U_pred.copy_(U.to(dev()))
     eng.loss_forward()
@@ -270,10 +273,11 @@ def test_notebook_variant_terms_against_autograd(fused):
     assert err <= 3e-5 * np.abs(gref).max(), err
 
 
-@pytest.mark.parametrize("k", [16, 32, 64])
+@pytest.mark.parametrize("k", [64])
 @pytest.mark.parametrize("n", [1, 127, 2503, 40001])
 def test_tensor_core_gram_term_matches_fp64(n, k):
-    """ep_eigen_bwd_gram_term_tf32x3: dU = s * MU (Gp + Gp^T) on tcgen05 (TF32 x 3) against fp64, strided inputs."""
+    """ep_eigen_bwd_gram_term_tf32x3: dU = s * MU (Gp + Gp^T) on tcgen05 (TF32 x 3) against fp64, strided inputs.  It is
+    built for k = 64 only; tests/test_cabi_cpu.py checks that every other k is rejected."""
     import ctypes
     cabi, ops = pkg("_cabi"), pkg("ops")
     g = torch.Generator().manual_seed(100 * k + n % 97)
@@ -294,27 +298,28 @@ def test_tensor_core_gram_term_matches_fp64(n, k):
     assert (got - ref).abs().max().item() <= 4e-6 * ref.abs().max().item() * np.sqrt(k / 16.0)
 
 
-def test_tensor_core_backward_equals_simt_backward():
-    """Two-kernel form (tensor-core k x k term + gather) against the one-kernel SIMT form, incl. a row range."""
-    ops, sparse, engine = pkg("ops"), pkg("sparse"), pkg("engine")
+def test_one_pass_backward_row_ranges_and_general_path_at_k64():
+    """k = 64, where the k x k term runs on the tensor cores before the gather pass: the row ranges (0, 1000) + (1000, n)
+    give the whole-range result bit for bit, and that equals the general path (prepare + transposed dual SpMM, which
+    takes no row range)."""
+    ops, sparse = pkg("ops"), pkg("sparse")
     fem, (K, M), _ = bunny_levels()
     pair = sparse.OperatorPair(K, M, dev())
-    n = K.shape[0]
-    for k in (16, 32, 64):
-        U = (0.3 * torch.randn(n, k, generator=torch.Generator().manual_seed(k))).to(dev())
-        KUMU = torch.empty(n, 2 * k, device=dev())
-        KU, MU = KUMU[:, :k], KUMU[:, k:]
-        ops.spmm2(pair, U, out_K=KU, out_M=MU)
-        Pp = ops.eigen_partials(U, KU, MU)
-        acc = torch.zeros(ops.N_LOSS_TERMS, dtype=torch.float64, device=dev())
-        _, coef = ops.eigen_finalize(k, n, Pp, 1000.0, 10.0, acc, w_mean=2.0, w_smooth=1.5)
-        outs = []
-        min_k, ops.TENSOR_CORE_GRAM_MIN_K = ops.TENSOR_CORE_GRAM_MIN_K, 16
-        for tc in (False, True):
-            ops.TENSOR_CORE_GRAM = tc
-            d = torch.zeros(n, k, device=dev())
-            ops.eigen_bwd_fused(pair, KU, MU, coef, 0.7, d, rows=(0, 1000))
-            ops.eigen_bwd_fused(pair, KU, MU, coef, 0.7, d, rows=(1000, n))
-            outs.append(d)
-        ops.TENSOR_CORE_GRAM, ops.TENSOR_CORE_GRAM_MIN_K = True, min_k
-        assert (outs[0] - outs[1]).abs().max().item() <= 1e-5 * outs[0].abs().max().item()
+    general = sparse.OperatorPair(K, M, dev(), assume_symmetric=False)
+    n, k = K.shape[0], 64
+    U = (0.3 * torch.randn(n, k, generator=torch.Generator().manual_seed(k))).to(dev())
+    KUMU = torch.empty(n, 2 * k, device=dev())
+    KU, MU = KUMU[:, :k], KUMU[:, k:]
+    ops.spmm2(pair, U, out_K=KU, out_M=MU)
+    Pp = ops.eigen_partials(U, KU, MU)
+    acc = torch.zeros(ops.N_LOSS_TERMS, dtype=torch.float64, device=dev())
+    _, coef = ops.eigen_finalize(k, n, Pp, 1000.0, 10.0, acc, w_mean=2.0, w_smooth=1.5)
+    whole = ops.eigen_loss_bwd(pair, U, KU, MU, coef, 0.7, torch.zeros(n, k, device=dev()))
+    split = torch.zeros(n, k, device=dev())
+    ops.eigen_loss_bwd(pair, U, KU, MU, coef, 0.7, split, rows=(0, 1000))
+    ops.eigen_loss_bwd(pair, U, KU, MU, coef, 0.7, split, rows=(1000, n))
+    ref = ops.eigen_loss_bwd(general, U, KU, MU, coef, 0.7, torch.zeros(n, k, device=dev()))
+    assert torch.equal(split, whole)
+    assert (whole - ref).abs().max().item() <= 1e-5 * ref.abs().max().item()
+    with pytest.raises(NotImplementedError):
+        ops.eigen_loss_bwd(general, U, KU, MU, coef, 0.7, split, rows=(0, 1000))

@@ -123,3 +123,12 @@ def test_sharded_engine_refuses_mode_scales_and_correction_smoothness():
     gnn = types.SimpleNamespace(model=types.SimpleNamespace(net=model.net), w_smooth_corr=1.0)
     with pytest.raises(NotImplementedError):
         dist_engine.make_sharded_engine(gnn, None, None, None, None, None, None, None, 0, 2)
+
+
+def test_sharded_engine_refuses_projection_terms():
+    """The sharded forward and backward have no projection term, so adding one raises instead of being ignored."""
+    import scipy.sparse as sp
+    dist_engine = pkg("dist_engine")
+    eng = object.__new__(dist_engine.ShardedTrainStepEngine)          # the refusal needs no engine state
+    with pytest.raises(NotImplementedError):
+        eng.add_projection_term(0, sp.eye(4, 2, format="csr"), torch.zeros(2, 3), 1.0)

@@ -106,9 +106,9 @@ def test_mixed_dtypes_cpu_tensors_and_large_k_are_refused():
         cabi.call("ep_eigen_partials_f64", 10, 129, fake, 129, fake, fake, 129, fake, fake, 1 << 20, None)
 
 
-def test_fp64_entries_are_declared_and_sized():
+def test_library_version_and_fp64_entries():
     cabi = pkg("_cabi")
-    assert cabi.query("ep_version") == 300
+    assert cabi.query("ep_version") == 400
     for name in ("ep_spmm_csr_f64", "ep_spmm2_csr_f64", "ep_spmm2_sum_csr_f64", "ep_eigen_partials_f64",
                  "ep_linear_fwd_f64", "ep_linear_bwd_f64"):
         assert name in cabi.SIGNATURES and name in cabi.KERNELS_PER_CALL
