@@ -10,7 +10,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libeigenpinns_b200.so")
 
-c_int, c_i64, c_sz = ctypes.c_int, ctypes.c_int64, ctypes.c_size_t
+c_int, c_i64, c_sz, c_u64 = ctypes.c_int, ctypes.c_int64, ctypes.c_size_t, ctypes.c_uint64
 c_f, c_d, c_p = ctypes.c_float, ctypes.c_double, ctypes.c_void_p
 
 # name -> (restype, argtypes); mirrors the header one to one
@@ -69,6 +69,16 @@ SIGNATURES = {
     "ep_tc_linear_dx_bf16": (c_int, [c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p]),
     "ep_tc_chain_fwd_bf16": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_f, c_p, c_p,
                                      c_int, c_p]),
+    "ep_dropout_keep_mask_u8": (c_int, [c_i64, c_int, c_f, c_u64, c_int, c_p, c_int, c_i64, c_p, c_p]),
+    "ep_linear_fwd_dropout_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_f, c_u64, c_int, c_p,
+                                          c_int, c_i64, c_p]),
+    "ep_linear_bwd_dropout_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_int, c_f, c_p, c_p,
+                                          c_p, c_sz, c_p]),
+    "ep_tc_linear_fwd_dropout_bf16": (c_int, [c_int, c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_f, c_u64, c_int,
+                                              c_p, c_int, c_i64, c_p]),
+    "ep_tc_linear_dx_dropout_bf16": (c_int, [c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_f, c_int, c_p]),
+    "ep_tc_chain_fwd_dropout_bf16": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_int, c_p, c_f, c_p,
+                                             c_p, c_int, c_p, c_f, c_u64, c_int, c_p, c_i64, c_p]),
     "ep_tc_dw_workspace_bytes": (c_sz, []),
     "ep_tc_linear_dw_bf16": (c_int, [c_int, c_int, c_int, c_int, c_int, c_p, c_p, c_p, c_p, c_p, c_sz, c_int, c_p]),
     "ep_grad_sqnorm_f32": (c_int, [c_sz, c_p, c_p, c_p]),
@@ -112,6 +122,8 @@ KERNELS_PER_CALL = {
     "ep_spmm_csr_f64": 1, "ep_spmm2_csr_f64": 1, "ep_spmm2_sum_csr_f64": 1, "ep_eigen_partials_f64": 2,
     "ep_linear_fwd_f64": 1, "ep_linear_bwd_f64": 5,
     "ep_mode_scale_fwd_f32": 1, "ep_mode_scale_bwd_f32": 2,
+    "ep_dropout_keep_mask_u8": 1, "ep_linear_fwd_dropout_f32": 1, "ep_linear_bwd_dropout_f32": 5,
+    "ep_tc_linear_fwd_dropout_bf16": 1, "ep_tc_linear_dx_dropout_bf16": 1, "ep_tc_chain_fwd_dropout_bf16": 1,
 }
 launch_counter = 0
 launch_by_entry = {}          # entry point -> kernels launched through it (bench.py reports the per-step table)

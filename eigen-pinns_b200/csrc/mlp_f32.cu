@@ -12,6 +12,8 @@
 // bf16 tcgen05 kernel in mlp_tc.cu.  The same kernels instantiated for double (plain DFMA, same tiling)
 // serve the fp64 dense layers of the notebook variants (variants.py).
 #include "ep_common.cuh"
+#include <type_traits>
+#include "dropout.cuh"
 
 namespace {
 
@@ -95,6 +97,78 @@ gemm_kernel(int M, int N, int K, const T* __restrict__ A, long long sa_i, long l
   }
 }
 
+// gemm_kernel<float> (no split-K) for a hidden layer followed by dropout, kept apart so that gemm_kernel's code does not
+// change.  DROP_FWD (forward, A = X, B = W^T): y = keep ? relu(z) * s : 0 with the keep mask of dropout.cuh.
+// DROP_BWD (dX): dX = (dY W) * [X > 0] * s - X is the stored, dropped activation, so its sign pattern already carries
+// the keep mask.
+enum Drop { DROP_FWD = 1, DROP_BWD = 2 };
+
+template <bool A_KC, bool B_KC, int DROP>
+__global__ void __launch_bounds__(256)
+gemm_dropout_kernel(int M, int N, int K, const float* __restrict__ A, long long sa_i, long long sa_k,
+                    const float* __restrict__ B, long long sb_k, long long sb_j, float* __restrict__ C, int ldc,
+                    const float* __restrict__ bias, const float* __restrict__ mask, int ldm, const dropout::Params dp) {
+  using T = float;
+  __shared__ __align__(16) T As[BK][PITCH];
+  __shared__ __align__(16) T Bs[BK][PITCH];
+  const int tid = threadIdx.x;
+  const int ty = tid >> 4, tx = tid & 15;
+  const int i0 = blockIdx.y * BM, j0 = blockIdx.x * BN;
+  T acc[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[i][j] = T(0);
+
+  for (int k0 = 0; k0 < K; k0 += BK) {
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int e = tid + 256 * q;
+      int ai, ak, bk, bj;
+      if (A_KC) { ai = e >> 4; ak = e & 15; } else { ak = e >> 6; ai = e & 63; }
+      if (B_KC) { bj = e >> 4; bk = e & 15; } else { bk = e >> 6; bj = e & 63; }
+      const int gi = i0 + ai, gk = k0 + ak;
+      As[ak][ai] = (gi < M && gk < K) ? __ldg(A + gi * sa_i + gk * sa_k) : T(0);
+      const int gj = j0 + bj, gk2 = k0 + bk;
+      Bs[bk][bj] = (gj < N && gk2 < K) ? __ldg(B + gk2 * sb_k + gj * sb_j) : T(0);
+    }
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < BK; ++kk) {
+      T av[4], bv[4];
+      lds4(&As[kk][ty * 4], av);
+      lds4(&Bs[kk][tx * 4], bv);
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fma_t(av[i], bv[j], acc[i][j]);
+    }
+    __syncthreads();
+  }
+  const int step = DROP == DROP_FWD ? dropout::step_of(dp) : 0;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int gi = i0 + ty * 4 + i;
+    if (gi >= M) continue;
+    uint32_t keep = 0;                 // the thread's four columns lie in one 8-column chunk: one Philox call per row
+    if (DROP == DROP_FWD)
+      keep = dropout::keep_byte(dp.seed, step, dp.layer, dp.row0 + gi, (j0 + tx * 4) >> 3, dp.thr) >> ((tx & 1) * 4);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int gj = j0 + tx * 4 + j;
+      if (gj >= N) continue;
+      T v = acc[i][j];
+      if (DROP == DROP_FWD) {
+        if (bias) v += __ldg(bias + gj);
+        v = ((keep >> j) & 1u) ? relu_t(v) * dp.s : T(0);
+      } else {
+        v = (__ldg(mask + (size_t)gi * ldm + gj) > T(0)) ? v * dp.s : T(0);
+      }
+      C[(size_t)gi * ldc + gj] = v;
+    }
+  }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256)
 sum_splits_kernel(int n_split, size_t len, const T* __restrict__ parts, T* __restrict__ out) {
@@ -161,9 +235,10 @@ int linear_fwd(int n, int in, int out, const T* X, int ldx, const T* W, const T*
   return EP_OK;
 }
 
+// drop_s > 0: X is the output of a hidden layer with dropout, dX = (dY W) * [X > 0] * drop_s (fp32 only)
 template <typename T>
 int linear_bwd(int n, int in, int out, const T* X, int ldx, const T* W, const T* dY, int lddy, T* dX, int lddx,
-               int relu_mask, T* dW, T* db, void* workspace, cudaStream_t st) {
+               int relu_mask, T* dW, T* db, void* workspace, cudaStream_t st, float drop_s = 0.f) {
   BwdPlan p = plan_bwd(n, in, out);
   T* parts = static_cast<T*>(workspace);
   T* cs_parts = parts + (size_t)p.n_split * in * out;
@@ -190,11 +265,38 @@ int linear_bwd(int n, int in, int out, const T* X, int ldx, const T* W, const T*
     for (int r0 = 0; r0 < n; r0 += slab) {
       const int rows = (n - r0) < slab ? (n - r0) : slab;
       dim3 grid(ep::ceil_div(in, BN), ep::ceil_div(rows, BM), 1);
+      if constexpr (std::is_same<T, float>::value) {
+        if (drop_s > 0.f) {
+          dropout::Params d{};
+          d.s = drop_s;
+          gemm_dropout_kernel<true, false, DROP_BWD><<<grid, 256, 0, st>>>(
+              rows, in, out, dY + (size_t)r0 * lddy, lddy, 1, W, in, 1, dX + (size_t)r0 * lddx, lddx, nullptr,
+              X + (size_t)r0 * ldx, ldx, d);
+          EP_LAUNCH_CHECK("gemm_dropout_kernel<dX>");
+          continue;
+        }
+      }
       gemm_kernel<T, true, false><<<grid, 256, 0, st>>>(
           rows, in, out, dY + (size_t)r0 * lddy, lddy, 1, W, in, 1, dX + (size_t)r0 * lddx, lddx, 0, nullptr, 0,
           relu_mask ? X + (size_t)r0 * ldx : nullptr, ldx, out);
       EP_LAUNCH_CHECK("gemm_kernel<dX>");
     }
+  }
+  return EP_OK;
+}
+
+// forward of a hidden layer followed by dropout: Y = keep ? relu(X W^T + b) * s : 0
+int linear_fwd_dropout(int n, int in, int out, const float* X, int ldx, const float* W, const float* b, float* Y, int ldy,
+                       dropout::Params dp, cudaStream_t st) {
+  const int slab = 65535 * BM;
+  for (int r0 = 0; r0 < n; r0 += slab) {
+    const int rows = (n - r0) < slab ? (n - r0) : slab;
+    dim3 grid(ep::ceil_div(out, BN), ep::ceil_div(rows, BM), 1);
+    dropout::Params d = dp;
+    d.row0 += r0;
+    gemm_dropout_kernel<true, true, DROP_FWD><<<grid, 256, 0, st>>>(
+        rows, out, in, X + (size_t)r0 * ldx, ldx, 1, W, 1, in, Y + (size_t)r0 * ldy, ldy, b, nullptr, 0, d);
+    EP_LAUNCH_CHECK("gemm_dropout_kernel<fwd>");
   }
   return EP_OK;
 }
@@ -246,6 +348,36 @@ int ep_linear_bwd_f32(int n, int in, int out, const float* X, int ldx, const flo
     return EP_ERR_WORKSPACE;
   }
   return linear_bwd(n, in, out, X, ldx, W, dY, lddy, dX, lddx, relu_mask, dW, db, workspace, ep::as_stream(stream));
+}
+
+int ep_linear_fwd_dropout_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* b,
+                              float* Y, int ldy, float p, unsigned long long seed, int step, const int* step_dev,
+                              int layer, long long row0, ep_stream_t stream) {
+  EP_REQUIRE(n >= 0 && in > 0 && out > 0, "bad size");
+  if (n == 0) return EP_OK;
+  EP_REQUIRE(X && W && Y, "null pointer");
+  EP_REQUIRE(ldx >= in && ldy >= out, "leading dimension too small");
+  EP_REQUIRE(ep::ceil_div(n, BM) <= 65535 * 1024, "n too large");
+  dropout::Params dp{};
+  if (int rc = dropout::host_params("ep_linear_fwd_dropout_f32", p, &dp.thr, &dp.s)) return rc;
+  dp.seed = seed; dp.row0 = row0; dp.step_dev = step_dev; dp.step = step; dp.layer = layer;
+  return linear_fwd_dropout(n, in, out, X, ldx, W, b, Y, ldy, dp, ep::as_stream(stream));
+}
+
+int ep_linear_bwd_dropout_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* dY,
+                              int lddy, float* dX, int lddx, float p, float* dW, float* db, void* workspace,
+                              size_t workspace_bytes, ep_stream_t stream) {
+  EP_REQUIRE(n > 0 && in > 0 && out > 0, "bad size");
+  EP_REQUIRE(X && W && dY && dX && dW && db && workspace, "null pointer");
+  EP_REQUIRE(ldx >= in && lddy >= out && lddx >= in, "leading dimension too small");
+  if (workspace_bytes < ep_linear_bwd_workspace_bytes(n, in, out)) {
+    ep::set_error("ep_linear_bwd_dropout_f32: workspace too small");
+    return EP_ERR_WORKSPACE;
+  }
+  uint32_t thr;
+  float s;
+  if (int rc = dropout::host_params("ep_linear_bwd_dropout_f32", p, &thr, &s)) return rc;
+  return linear_bwd(n, in, out, X, ldx, W, dY, lddy, dX, lddx, 1, dW, db, workspace, ep::as_stream(stream), s);
 }
 
 int ep_linear_bwd_f64(int n, int in, int out, const double* X, int ldx, const double* W, const double* dY,

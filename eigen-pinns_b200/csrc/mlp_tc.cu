@@ -35,6 +35,8 @@
 namespace tc {
 
 enum LinearMode { MODE_HIDDEN = 0, MODE_DX = 1, MODE_FINAL = 2 };
+// DROP (tc_linear_dropout_kernel): MODE_HIDDEN applies the dropout of dropout.cuh before the bf16 pack, MODE_DX scales
+// the masked gradient by s (its mask was built from the dropped activation).
 
 struct LinearArgs {
   const uint8_t* A;          // packed input tiles, KC chunks each
@@ -50,8 +52,8 @@ struct LinearArgs {
   int n_rows, n_out;
 };
 
-template <int MODE>
-__global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs a) {
+template <int MODE, bool DROP>
+__device__ __forceinline__ void tc_linear_body(const LinearArgs& a, const dropout::Params& dp) {
   extern __shared__ __align__(128) uint8_t smem[];
   const int KC = a.KC, N = a.N;
   uint8_t* Bs = smem;                                           // KC * N * 16 bytes
@@ -139,6 +141,7 @@ __global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs
     const int ncb = N / 32;                              // 32-column blocks (<= 8)
     int acc = 0; uint32_t acc_phase = 0;
     const float scale = (MODE == MODE_FINAL && a.scale_dev) ? *a.scale_dev : a.scale;
+    const int drop_step = (DROP && MODE == MODE_HIDDEN) ? dropout::step_of(dp) : 0;
     float* stg = stage_f + (size_t)q * 32 * 33;           // MODE_FINAL: per-warp 32 x 33 transpose buffer
     for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
       const long long row = (long long)tile * TILE_M + r;
@@ -193,8 +196,14 @@ __global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs
               float4 b4[8];
 #pragma unroll
               for (int j = 0; j < 8; ++j) b4[j] = *reinterpret_cast<const float4*>(bias_s + cb * 32 + 4 * j);
-              bits = epi_block_fwd(v, b4, w);
+              if constexpr (DROP) {
+                const uint32_t keep = keep_block32(dp.seed, drop_step, dp.layer, dp.row0 + row, cb * 4, dp.thr);
+                bits = epi_block_fwd_drop(v, b4, keep, dp.s, w);
+              } else {
+                bits = epi_block_fwd(v, b4, w);
+              }
             }
+            else if constexpr (DROP) epi_block_dx_scaled(v, mw[cb], dp.s, w);
             else epi_block_dx(v, mw[cb], w);
 #pragma unroll
             for (int g = 0; g < 4; ++g)                       // 4 chunks of 8 columns
@@ -213,6 +222,17 @@ __global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs
   tc_fence_before();
   __syncthreads();
   if (warp == 1) { tc_fence_after(); tmem_dealloc(tmem_base, TMEM_COLS); }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_kernel(LinearArgs a) {
+  tc_linear_body<MODE, false>(a, dropout::Params{});
+}
+
+// MODE_HIDDEN / MODE_DX of a hidden layer followed by dropout
+template <int MODE>
+__global__ void __launch_bounds__(LINEAR_THREADS, 1) tc_linear_dropout_kernel(LinearArgs a, const dropout::Params dp) {
+  tc_linear_body<MODE, true>(a, dp);
 }
 
 // ------------------------------------------------------------------------------------------- layer chain
@@ -282,6 +302,15 @@ struct ChainArgs {
   int n_rows, n_out, relu;
   unsigned long long* trace;   // optional timing trace of CTA 0 (clock64 stamps), experiments only
 };
+// dropout after the ReLU of every hidden layer l (tc_chain2_dropout_kernel); layer index = l, thr[l] = 0 keeps all
+struct ChainDropout {
+  unsigned long long seed;
+  long long row0;
+  const int* step_dev;
+  int step, pad_;
+  uint32_t thr[CH_MAX_LAYERS];
+  float s[CH_MAX_LAYERS];
+};
 
 constexpr int C2_PRODUCERS = 3;               // weight-issuing warps: 0, 10, 11
 constexpr int C2_THREADS = 384;               // + warp 1: MMA issuer (leader) / forwarder (peer), warps 2..9: epilogue.
@@ -323,298 +352,14 @@ __device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols));
 }
 
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C2_THREADS, 1)
-tc_chain2_kernel(const __grid_constant__ ChainArgs a) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  uint8_t* act0 = smem;                                   // operand tile of slot P
-  uint8_t* act1 = smem + CH_ACT_BYTES;                    // operand tile of slot Q
-  uint8_t* ring = smem + 2 * CH_ACT_BYTES;
-  float* bias_s = reinterpret_cast<float*>(ring + C2_STAGES * C2_SLOT_BYTES);          // [CH_MAX_LAYERS][256]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(bias_s + CH_MAX_LAYERS * 256);
-  uint64_t* wempty = bars;                         // [C2_STAGES]
-  uint64_t* landed = wempty + C2_STAGES;           // [2]
-  uint64_t* in_full = landed + 2;                  // [2]
-  uint64_t* acc_full = in_full + 2;                // [2]
-  uint64_t* act_ready = acc_full + 2;              // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + C2_N_BARRIERS);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int L = a.n_layers;
-  const int rank = (int)cluster_ctarank();
-  const bool leader = rank == 0;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < C2_STAGES; ++s) mbar_init(&wempty[s], 1);
-    for (int u = 0; u < 2; ++u) {
-      mbar_init(&landed[u], C2_PRODUCERS + (leader ? 1 : 0));
-      mbar_init(&in_full[u], leader ? 2 : 1);
-      mbar_init(&acc_full[u], 1);
-      mbar_init(&act_ready[u], 512);
-    }
-    fence_barrier_init();
-  }
-  for (int i = threadIdx.x; i < L * 256; i += blockDim.x) {
-    const int l = i >> 8, c = i & 255;
-    bias_s[i] = (a.L[l].bias && c < a.L[l].n_bias) ? a.L[l].bias[c] : 0.f;
-  }
-  if (warp == 1) tmem_alloc2(tmem_slot, TMEM_COLS);
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                 // both CTAs' barriers and TMEM exist before anything crosses over
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int n_units = (a.n_tiles + 1) >> 1;
-  const int n_clusters = (int)gridDim.x >> 1;
-  const int cluster_id = (int)blockIdx.x >> 1;
-  const int my_units = cluster_id < n_units ? (n_units - cluster_id + n_clusters - 1) / n_clusters : 0;
-  auto unit_of = [&](int j) { return cluster_id + j * n_clusters; };
-  const uint32_t in_bytes = (uint32_t)a.L[0].KC * CHUNK_BYTES;
-
-  if (warp == 0 || warp >= 10) {
-    // ---- weights: this CTA's N/2 output columns of every K = 32 slab, each layer once per unit pair; the slabs of the
-    //      whole sequence are dealt round-robin to the C2_PRODUCERS issuing warps
-    if (lane == 0) {
-      const int me = warp == 0 ? 0 : warp - 9;
-      uint32_t gs = 0;                               // slab counter over the whole sequence
-      uint32_t lc = 0;                               // layer counter over the whole sequence
-      for (int j = 0; j < my_units; j += 2) {
-        for (int l = 0; l < L; ++l, ++lc) {
-          const int N = a.L[l].N;
-          const uint32_t half_bytes = (uint32_t)(N >> 1) * 64u;          // 4 chunks x N/2 columns x 16 B
-          const int n_slabs = a.L[l].KC >> 2;
-          const uint8_t* src = a.L[l].B + (size_t)a.L[l].KC * N * 16 + (size_t)rank * half_bytes;    // the "pair" copy
-          // Every producer announces the bytes of ITS slabs of this layer with one arrive.expect_tx (so the transaction
-          // count never goes negative) - after the barrier's previous phase (layer lc - 2) is complete.
-          {
-            int mine = 0;
-            for (int s = 0; s < n_slabs; ++s) mine += ((gs + s) % C2_PRODUCERS) == (uint32_t)me ? 1 : 0;
-            if (lc >= 2) mbar_wait(&landed[lc & 1], ((lc - 2) >> 1) & 1);
-            if (mine) mbar_expect_tx(&landed[lc & 1], (uint32_t)mine * half_bytes);
-            else mbar_arrive(&landed[lc & 1]);
-          }
-          for (int s = 0; s < n_slabs; ++s, ++gs) {
-            if ((int)(gs % C2_PRODUCERS) != me) continue;
-            const uint32_t stage = gs % C2_STAGES, phase = (gs / C2_STAGES) & 1;
-            mbar_wait(&wempty[stage], phase ^ 1);
-            bulk_g2s(ring + stage * C2_SLOT_BYTES, src + (size_t)s * 2 * half_bytes, half_bytes, &landed[lc & 1]);
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0 && !leader) {
-      // ---- peer: tell the leader when a layer's weights / the input tile of a slot have landed here (or that there is
-      //      no tile); the two event streams interleave, so poll both
-      const uint32_t remote_w[2] = {map_to_cta(&landed[0], 0), map_to_cta(&landed[1], 0)};
-      const uint32_t remote_i[2] = {map_to_cta(&in_full[0], 0), map_to_cta(&in_full[1], 0)};
-      const uint32_t n_layers_total = (uint32_t)((my_units + 1) >> 1) * (uint32_t)L;
-      uint32_t lc = 0, nu[2] = {0, 0};
-      int j = 0;
-      for (uint32_t spin = 0; lc < n_layers_total || j < my_units; ++spin) {
-        if (lc < n_layers_total && mbar_test(&landed[lc & 1], (lc >> 1) & 1)) { mbar_arrive_remote(remote_w[lc & 1]); ++lc; spin = 0; }
-        if (j < my_units) {
-          const int u = j & 1;
-          if (2 * unit_of(j) + rank >= a.n_tiles || mbar_test(&in_full[u], nu[u] & 1)) {
-            mbar_arrive_remote(remote_i[u]); ++nu[u]; ++j; spin = 0;
-          }
-        }
-        if (spin > (1u << 28)) { printf("eigenpinns_b200: forwarder timed out (block %d)\n", blockIdx.x); __trap(); }
-      }
-    } else if (lane == 0) {
-      // ---- leader: every MMA of the pair
-      uint32_t stage = 0;
-      uint32_t lc = 0;
-      uint32_t gl[2] = {0, 0};                       // layers completed per slot
-      uint32_t nu[2] = {0, 0};                       // units started per slot
-      const uint32_t abase[2] = {smem_u32(act0), smem_u32(act1)};
-      for (int j = 0; j < my_units; j += 2) {
-        const bool has_q = (j + 1) < my_units;
-        for (int l = 0; l < L; ++l, ++lc) {
-          const int N = a.L[l].N;
-          const uint32_t idesc = make_idesc(256, N, false, false);
-          const uint32_t b_lbo = (uint32_t)(N >> 1) * 16;
-          const int n_slabs = a.L[l].KC >> 2;
-          for (int u = 0; u < (has_q ? 2 : 1); ++u) {
-            if (l == 0) mbar_wait_spin(&in_full[u], nu[u] & 1);
-            if (u == 0) mbar_wait_spin(&landed[lc & 1], (lc >> 1) & 1);
-            if (gl[u] > 0) mbar_wait_spin(&act_ready[u], (gl[u] - 1) & 1);
-            tc_fence_after();
-            const uint32_t tg = gl[0] + gl[1];
-            if (a.trace && blockIdx.x == 0 && tg < 64) a.trace[tg * 8 + 0] = clock64();      // operands ready
-            const bool releases = (u == 1) || !has_q;       // last reader of the layer's slots
-            for (int s = 0; s < n_slabs; ++s) {
-              uint32_t slot = stage + s;
-              if (slot >= C2_STAGES) slot -= C2_STAGES;
-              const uint32_t b_base = smem_u32(ring + slot * C2_SLOT_BYTES);
-#pragma unroll
-              for (int jj = 0; jj < 2; ++jj) {
-                const uint64_t bdesc = make_desc(b_base + (uint32_t)(jj * 2) * b_lbo, b_lbo, 128);
-                const uint64_t adesc = make_desc(abase[u] + (uint32_t)(s * 4 + jj * 2) * CHUNK_BYTES, CHUNK_BYTES, 128);
-                umma2_bf16(tmem_base + (uint32_t)u * 256u, adesc, bdesc, idesc, (s | jj) != 0 ? 1u : 0u);
-              }
-              if (releases) umma2_commit_pair(&wempty[slot]);
-            }
-            umma2_commit_pair(&acc_full[u]);
-            if (a.trace && blockIdx.x == 0 && tg < 64) a.trace[tg * 8 + 1] = clock64();      // all MMAs issued
-            ++gl[u];
-          }
-          stage += n_slabs;
-          if (stage >= C2_STAGES) stage -= C2_STAGES;
-        }
-        ++nu[0]; ++nu[1];
-      }
-    }
-  } else {
-    // ---- epilogue: 8 warps on ONE tile (slot u of the current step); TMEM lane quadrant q, column half hf
-    const int q = warp & 3;
-    const int hf = (warp - 2) >> 2;
-    const int r = q * 32 + lane;
-    const bool elected = (warp == 2 && lane == 0);
-    const uint32_t ready_remote[2] = {map_to_cta(&act_ready[0], 0), map_to_cta(&act_ready[1], 0)};
-    auto issue_input = [&](int j) {                    // input tile of this CTA for its j-th unit -> slot j & 1
-      const int u = j & 1;
-      const int tile = 2 * unit_of(j) + rank;
-      if (tile < a.n_tiles) {
-        mbar_expect_tx(&in_full[u], in_bytes);
-        bulk_g2s(u ? act1 : act0, a.A0 + (size_t)tile * in_bytes, in_bytes, &in_full[u]);
-      }
-    };
-    if (elected) { if (my_units > 0) issue_input(0); if (my_units > 1) issue_input(1); }
-    const float scale = a.scale_dev ? *a.scale_dev : a.scale;
-    const bool vec_out = ((a.ldc | a.ldu | a.n_out) & 3) == 0 &&
-                         ((reinterpret_cast<uintptr_t>(a.corr) | reinterpret_cast<uintptr_t>(a.U_base) |
-                           reinterpret_cast<uintptr_t>(a.U_pred)) & 15u) == 0;
-    uint32_t gl[2] = {0, 0};
-    for (int j = 0; j < my_units; j += 2) {
-      const bool has_q = (j + 1) < my_units;
-      for (int l = 0; l < L; ++l) {
-        const int N = a.L[l].N, ncb = N >> 5;
-        const int my_cb = min(4, ncb - 4 * hf);           // 32-column blocks of this warp (<= 0: none)
-        uint8_t* const out_packed = a.L[l].out_packed;
-        uint32_t* const mask_ptr = a.L[l].mask;
-        const float* bl = bias_s + l * 256 + hf * 128;
-        const bool last = (l == L - 1);
-        for (int u = 0; u < (has_q ? 2 : 1); ++u) {
-          const int tile = 2 * unit_of(j + u) + rank;
-          const bool valid = tile < a.n_tiles;
-          const bool work = valid && my_cb > 0;
-          const long long row = (long long)tile * TILE_M + r;
-          uint8_t* act = u ? act1 : act0;
-          const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)u * 256u + (uint32_t)hf * 128u;
-          float4 ub[8];
-          const bool final_rows = last && work && row < a.n_rows;
-          if (final_rows && vec_out && a.U_pred) {
-#pragma unroll
-            for (int jj = 0; jj < 8; ++jj) {
-              const int col = hf * 128 + 4 * jj;
-              ub[jj] = col < a.n_out ? __ldg(reinterpret_cast<const float4*>(a.U_base + (size_t)row * a.ldu + col))
-                                     : make_float4(0.f, 0.f, 0.f, 0.f);
-            }
-          }
-          mbar_wait(&acc_full[u], gl[u] & 1);
-          tc_fence_after();
-          const uint32_t tg = gl[0] + gl[1];
-          if (a.trace && blockIdx.x == 0 && tg < 64 && threadIdx.x == 64) a.trace[tg * 8 + 2] = clock64();   // accumulator ready
-          if (last && elected && (j + u + 2) < my_units) issue_input(j + u + 2);     // slot u's operand tile is free
-          if (work) {
-            if (last) {
-              const bool in_rows = row < a.n_rows;
-              for (int cb = 0; cb < my_cb; ++cb) {
-                const int col0 = hf * 128 + cb * 32;
-                if (cb > 0 && vec_out && in_rows && a.U_pred) {
-#pragma unroll
-                  for (int jj = 0; jj < 8; ++jj) {
-                    const int col = col0 + 4 * jj;
-                    ub[jj] = col < a.n_out ? __ldg(reinterpret_cast<const float4*>(a.U_base + (size_t)row * a.ldu + col))
-                                           : make_float4(0.f, 0.f, 0.f, 0.f);
-                  }
-                }
-                uint32_t v[32];
-                tmem_ld32(t_addr + cb * 32, v);
-                if (in_rows) {
-                  if (vec_out) {
-#pragma unroll
-                    for (int jj = 0; jj < 8; ++jj) {
-                      const int col = col0 + 4 * jj;
-                      if (col < a.n_out) {
-                        const float4 bj = *reinterpret_cast<const float4*>(bl + cb * 32 + 4 * jj);
-                        float4 c;
-                        c.x = __uint_as_float(v[4 * jj]) + bj.x;     c.y = __uint_as_float(v[4 * jj + 1]) + bj.y;
-                        c.z = __uint_as_float(v[4 * jj + 2]) + bj.z; c.w = __uint_as_float(v[4 * jj + 3]) + bj.w;
-                        if (a.corr) *reinterpret_cast<float4*>(a.corr + (size_t)row * a.ldc + col) = c;
-                        if (a.U_pred) {
-                          float4 uu;
-                          uu.x = __fadd_rn(ub[jj].x, __fmul_rn(scale, c.x)); uu.y = __fadd_rn(ub[jj].y, __fmul_rn(scale, c.y));
-                          uu.z = __fadd_rn(ub[jj].z, __fmul_rn(scale, c.z)); uu.w = __fadd_rn(ub[jj].w, __fmul_rn(scale, c.w));
-                          *reinterpret_cast<float4*>(a.U_pred + (size_t)row * a.ldu + col) = uu;
-                        }
-                      }
-                    }
-                  } else {
-#pragma unroll
-                    for (int jj = 0; jj < 32; ++jj) {
-                      const int col = col0 + jj;
-                      if (col < a.n_out) {
-                        const float c = __uint_as_float(v[jj]) + bl[cb * 32 + jj];
-                        if (a.corr) a.corr[(size_t)row * a.ldc + col] = c;
-                        if (a.U_pred)
-                          a.U_pred[(size_t)row * a.ldu + col] =
-                              __fadd_rn(__ldg(a.U_base + (size_t)row * a.ldu + col), __fmul_rn(scale, c));
-                      }
-                    }
-                  }
-                }
-              }
-            } else {
-              const size_t tile_off = (size_t)tile * (N >> 3) * CHUNK_BYTES + (size_t)r * 16;
-              const bool to_smem = !last;
-              uint32_t bits[4];
-              uint32_t va[32], vb[32];                     // two accumulator blocks: the load of block cb + 1 flies
-              tmem_ld32_issue(t_addr, va);                 // while block cb is converted and stored
-#pragma unroll
-              for (int cb = 0; cb < 4; ++cb) {
-                if (cb < my_cb) {
-                  uint32_t (&v)[32] = (cb & 1) ? vb : va;
-                  tmem_ld32_wait(v);
-                  if (cb + 1 < my_cb) tmem_ld32_issue(t_addr + (cb + 1) * 32, (cb & 1) ? va : vb);
-                  uint32_t w[16];
-                  bits[cb] = epi_block_fwd_sb(v, bl + cb * 32, w);
-#pragma unroll
-                  for (int g4 = 0; g4 < 4; ++g4) {
-                    const uint4 o = make_uint4(w[4 * g4], w[4 * g4 + 1], w[4 * g4 + 2], w[4 * g4 + 3]);
-                    const size_t c_off = (size_t)((hf * 4 + cb) * 4 + g4) * CHUNK_BYTES;
-                    if (to_smem) *reinterpret_cast<uint4*>(act + c_off + (size_t)r * 16) = o;
-                    if (out_packed) *reinterpret_cast<uint4*>(out_packed + tile_off + c_off) = o;
-                  }
-                } else {
-                  bits[cb] = 0u;
-                }
-              }
-              if (mask_ptr) {
-                uint32_t* mrow = mask_ptr + (size_t)row * ncb + 4 * hf;
-                if (my_cb == 4) {
-                  *reinterpret_cast<uint4*>(mrow) = make_uint4(bits[0], bits[1], bits[2], bits[3]);
-                } else {
-#pragma unroll
-                  for (int cb = 0; cb < 4; ++cb) if (cb < my_cb) mrow[cb] = bits[cb];
-                }
-              }
-            }
-          }
-          if (a.trace && blockIdx.x == 0 && tg < 64 && threadIdx.x == 64) a.trace[tg * 8 + 3] = clock64();   // drained
-          if (!last) fence_proxy_async_smem();           // generic-proxy writes -> visible to the tensor core of this SM
-          tc_fence_before();
-          mbar_arrive_remote(ready_remote[u]);         // the leader's barrier, whichever CTA this is
-          if (a.trace && blockIdx.x == 0 && tg < 64 && threadIdx.x == 64) a.trace[tg * 8 + 4] = clock64();   // arrived
-          ++gl[u];
-        }
-      }
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                 // neither CTA leaves (or frees TMEM) while the other may still signal it
-  if (warp == 1) { tc_fence_after(); tmem_dealloc2(tmem_base, TMEM_COLS); }
-}
+#define CHAIN2_DROPOUT 0
+#include "chain2_kernel.cuh"
+#undef CHAIN2_DROPOUT
+// the chain with dropout after every hidden ReLU (ChainDropout): a separate kernel, so that the epilogue of the one
+// above - the forward's limiter - carries no dropout code
+#define CHAIN2_DROPOUT 1
+#include "chain2_kernel.cuh"
+#undef CHAIN2_DROPOUT
 
 // ------------------------------------------------------------------------------------------- dW
 constexpr int DW_THREADS = 192;
@@ -902,17 +647,30 @@ using namespace tc;
 namespace {
 
 template <int MODE>
-int launch_linear(const LinearArgs& a, cudaStream_t st, int max_ctas = 0) {
+int launch_linear(const LinearArgs& a, cudaStream_t st, int max_ctas = 0, const dropout::Params* dp = nullptr) {
   const size_t smem = (size_t)a.KC * a.N * 16 + (size_t)N_STAGES * STAGE_BYTES + 8 * (2 * N_STAGES + 5) + 16 +
                       sizeof(float) * a.N + (MODE == MODE_FINAL ? sizeof(float) * 4 * 32 * 33 : 0) + 128;
+  int grid = ep::sm_count();
+  if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
+  if (grid > a.n_tiles) grid = a.n_tiles;
+  if constexpr (MODE != MODE_FINAL) {
+    if (dp) {
+      static size_t configured_drop = 0;
+      if (smem > configured_drop) {
+        EP_CUDA_CHECK(cudaFuncSetAttribute(tc_linear_dropout_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)smem));
+        configured_drop = smem;
+      }
+      tc_linear_dropout_kernel<MODE><<<grid, LINEAR_THREADS, smem, st>>>(a, *dp);
+      EP_LAUNCH_CHECK("tc_linear_dropout_kernel");
+      return EP_OK;
+    }
+  }
   static size_t configured = 0;
   if (smem > configured) {
     EP_CUDA_CHECK(cudaFuncSetAttribute(tc_linear_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = smem;
   }
-  int grid = ep::sm_count();
-  if (max_ctas > 0 && grid > max_ctas) grid = max_ctas;
-  if (grid > a.n_tiles) grid = a.n_tiles;
   tc_linear_kernel<MODE><<<grid, LINEAR_THREADS, smem, st>>>(a);
   EP_LAUNCH_CHECK("tc_linear_kernel");
   return EP_OK;
@@ -920,19 +678,29 @@ int launch_linear(const LinearArgs& a, cudaStream_t st, int max_ctas = 0) {
 
 bool dims_ok(int kp, int np) { return kp % 32 == 0 && np % 32 == 0 && kp >= 32 && np >= 32 && kp <= 256 && np <= 256; }
 
-int launch_chain(const ChainArgs& a, cudaStream_t st) {
+int launch_chain(const ChainArgs& a, cudaStream_t st, const ChainDropout* dp = nullptr) {
   // one cluster of two CTAs per unit of two tiles, at most one CTA per SM
   const size_t smem = 2 * (size_t)CH_ACT_BYTES + (size_t)C2_STAGES * C2_SLOT_BYTES + sizeof(float) * CH_MAX_LAYERS * 256 +
                       8 * C2_N_BARRIERS + 16 + 128;
+  const int n_pairs = (a.n_tiles + 1) / 2;
+  int clusters = ep::sm_count() / 2;
+  if (clusters > n_pairs) clusters = n_pairs;
+  ChainArgs b = a;
+  if (dp) {
+    static bool configured_drop = false;
+    if (!configured_drop) {
+      EP_CUDA_CHECK(cudaFuncSetAttribute(tc_chain2_dropout_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      configured_drop = true;
+    }
+    tc_chain2_dropout_kernel<<<2 * clusters, C2_THREADS, smem, st>>>(b, *dp);
+    EP_LAUNCH_CHECK("tc_chain2_dropout_kernel");
+    return EP_OK;
+  }
   static bool configured = false;
   if (!configured) {
     EP_CUDA_CHECK(cudaFuncSetAttribute(tc_chain2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     configured = true;
   }
-  const int n_pairs = (a.n_tiles + 1) / 2;
-  int clusters = ep::sm_count() / 2;
-  if (clusters > n_pairs) clusters = n_pairs;
-  ChainArgs b = a;
   b.trace = reinterpret_cast<unsigned long long*>(((uintptr_t)(uint32_t)ep::tune_flag(4) << 32) | (uint32_t)ep::tune_flag(3));
   tc_chain2_kernel<<<2 * clusters, C2_THREADS, smem, st>>>(b);
   EP_LAUNCH_CHECK("tc_chain2_kernel");
@@ -1021,6 +789,37 @@ int ep_tc_linear_final_bf16(int n, int in_padded, int out, int out_padded, const
   return launch_linear<MODE_FINAL>(a, ep::as_stream(stream));
 }
 
+int ep_tc_linear_fwd_dropout_bf16(int n, int in_padded, int out, int out_padded, const void* A_packed, const void* Wp,
+                                  const float* bias, void* out_packed, void* relu_mask_out, float p,
+                                  unsigned long long seed, int step, const int* step_dev, int layer, long long row0,
+                                  ep_stream_t stream) {
+  EP_REQUIRE(n > 0 && A_packed && Wp && out_packed, "bad argument");
+  if (!dims_ok(in_padded, out_padded)) { ep::set_error("ep_tc_linear_fwd_dropout_bf16: padded dims must be multiples of 32 in [32, 256]"); return EP_ERR_UNSUPPORTED; }
+  dropout::Params dp{};
+  if (int rc = dropout::host_params("ep_tc_linear_fwd_dropout_bf16", p, &dp.thr, &dp.s)) return rc;
+  dp.seed = seed; dp.row0 = row0; dp.step_dev = step_dev; dp.step = step; dp.layer = layer;
+  LinearArgs a{};
+  a.A = static_cast<const uint8_t*>(A_packed); a.B = static_cast<const uint8_t*>(Wp);
+  a.n_tiles = n_tiles_for(n); a.KC = in_padded / 8; a.N = out_padded; a.bias = bias; a.n_bias = out; a.relu = 1;
+  a.out_packed = static_cast<uint8_t*>(out_packed); a.mask_out = static_cast<uint32_t*>(relu_mask_out);
+  a.n_rows = n; a.n_out = out_padded;
+  return launch_linear<MODE_HIDDEN>(a, ep::as_stream(stream), 0, &dp);
+}
+
+int ep_tc_linear_dx_dropout_bf16(int n, int out_padded, int in_padded, const void* dZ_packed, const void* WTp,
+                                 const void* relu_mask, void* dZprev_packed, float p, int max_ctas, ep_stream_t stream) {
+  EP_REQUIRE(n > 0 && dZ_packed && WTp && relu_mask && dZprev_packed, "bad argument");
+  if (!dims_ok(out_padded, in_padded)) { ep::set_error("ep_tc_linear_dx_dropout_bf16: unsupported dims"); return EP_ERR_UNSUPPORTED; }
+  dropout::Params dp{};
+  if (int rc = dropout::host_params("ep_tc_linear_dx_dropout_bf16", p, &dp.thr, &dp.s)) return rc;
+  LinearArgs a{};
+  a.A = static_cast<const uint8_t*>(dZ_packed); a.B = static_cast<const uint8_t*>(WTp);
+  a.n_tiles = n_tiles_for(n); a.KC = out_padded / 8; a.N = in_padded;
+  a.out_packed = static_cast<uint8_t*>(dZprev_packed); a.mask_in = static_cast<const uint32_t*>(relu_mask);
+  a.n_rows = n; a.n_out = in_padded;
+  return launch_linear<MODE_DX>(a, ep::as_stream(stream), max_ctas, &dp);
+}
+
 int ep_tc_linear_dx_bf16(int n, int out_padded, int in_padded, const void* dZ_packed, const void* WTp,
                          const void* relu_mask, void* dZprev_packed, int max_ctas, ep_stream_t stream) {
   EP_REQUIRE(n > 0 && dZ_packed && WTp && relu_mask && dZprev_packed, "bad argument");
@@ -1033,13 +832,17 @@ int ep_tc_linear_dx_bf16(int n, int out_padded, int in_padded, const void* dZ_pa
   return launch_linear<MODE_DX>(a, ep::as_stream(stream), max_ctas);
 }
 
-int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, const int* dims_out, const void* A0_packed,
-                         const void* const* Wp, const float* const* bias, void* const* act_out,
-                         void* const* relu_mask_out, float* corr, int ldc, const float* U_base, float scale,
-                         const float* scale_dev, float* U_pred, int ldu, ep_stream_t stream) {
+}  // extern "C"
+
+namespace {
+
+int chain_fwd(const char* who, int n, int n_layers, const int* dims_padded, const int* dims_out, const void* A0_packed,
+              const void* const* Wp, const float* const* bias, void* const* act_out, void* const* relu_mask_out,
+              float* corr, int ldc, const float* U_base, float scale, const float* scale_dev, float* U_pred, int ldu,
+              const ChainDropout* dp, ep_stream_t stream) {
   EP_REQUIRE(n > 0 && A0_packed && Wp && bias && dims_out, "bad argument");
   EP_REQUIRE(n_layers >= 2, "the forward chain needs at least one hidden layer");
-  if (int rc = chain_dims_ok("ep_tc_chain_fwd_bf16", n_layers, dims_padded)) return rc;
+  if (int rc = chain_dims_ok(who, n_layers, dims_padded)) return rc;
   const int k = dims_out[n_layers - 1];
   EP_REQUIRE(k > 0 && k <= dims_padded[n_layers], "bad output width");
   EP_REQUIRE((U_base == nullptr) == (U_pred == nullptr) && (!U_pred || ldu >= k) && (!corr || ldc >= k),
@@ -1059,7 +862,35 @@ int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, const int*
   }
   a.corr = corr; a.ldc = ldc; a.U_base = U_base; a.U_pred = U_pred; a.ldu = ldu; a.scale = scale; a.scale_dev = scale_dev;
   a.n_rows = n; a.n_out = k; a.relu = 1;
-  return launch_chain(a, ep::as_stream(stream));
+  return launch_chain(a, ep::as_stream(stream), dp);
+}
+
+}  // namespace
+
+extern "C" {
+
+int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, const int* dims_out, const void* A0_packed,
+                         const void* const* Wp, const float* const* bias, void* const* act_out,
+                         void* const* relu_mask_out, float* corr, int ldc, const float* U_base, float scale,
+                         const float* scale_dev, float* U_pred, int ldu, ep_stream_t stream) {
+  return chain_fwd("ep_tc_chain_fwd_bf16", n, n_layers, dims_padded, dims_out, A0_packed, Wp, bias, act_out,
+                   relu_mask_out, corr, ldc, U_base, scale, scale_dev, U_pred, ldu, nullptr, stream);
+}
+
+int ep_tc_chain_fwd_dropout_bf16(int n, int n_layers, const int* dims_padded, const int* dims_out, const void* A0_packed,
+                                 const void* const* Wp, const float* const* bias, void* const* act_out,
+                                 void* const* relu_mask_out, float* corr, int ldc, const float* U_base, float scale,
+                                 const float* scale_dev, float* U_pred, int ldu, const float* p_layers, float p,
+                                 unsigned long long seed, int step, const int* step_dev, long long row0,
+                                 ep_stream_t stream) {
+  ChainDropout dp{};
+  dp.seed = seed; dp.row0 = row0; dp.step_dev = step_dev; dp.step = step;
+  EP_REQUIRE(n_layers >= 2 && n_layers <= CH_MAX_LAYERS, "1 <= hidden layers < 8");
+  for (int l = 0; l + 1 < n_layers; ++l)
+    if (int rc = dropout::host_params("ep_tc_chain_fwd_dropout_bf16", p_layers ? p_layers[l] : p, &dp.thr[l], &dp.s[l]))
+      return rc;
+  return chain_fwd("ep_tc_chain_fwd_dropout_bf16", n, n_layers, dims_padded, dims_out, A0_packed, Wp, bias, act_out,
+                   relu_mask_out, corr, ldc, U_base, scale, scale_dev, U_pred, ldu, &dp, stream);
 }
 
 size_t ep_tc_dw_workspace_bytes(void) { return sizeof(float) * (size_t)ep::sm_count() * (256 * 256 + 256); }

@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_bf16.h>
 #include "ep_common.cuh"
+#include "dropout.cuh"
 
 namespace tc {
 
@@ -186,6 +187,57 @@ __device__ __forceinline__ void epi_block_dx(const uint32_t (&v)[32], uint32_t m
 #pragma unroll
   for (int i = 0; i < 16; ++i)
     w[i] = relu_mask_apply(pack_bf16x2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), mask_word, i);
+}
+
+// ---- dropout forms (dropout.cuh) ------------------------------------------------------------------------------
+// Keep bits of a 32-column block (bit j = feature 8 * chunk0 + j kept): four Philox calls, chunks chunk0 .. chunk0 + 3.
+__device__ __forceinline__ uint32_t keep_block32(unsigned long long seed, int step, int layer, long long row, int chunk0,
+                                                 uint32_t thr) {
+  uint32_t k = 0;
+#pragma unroll
+  for (int g = 0; g < 4; ++g) k |= dropout::keep_byte(seed, step, layer, row, chunk0 + g, thr) << (8 * g);
+  return k;
+}
+// z = v + bias, scaled by s where kept and zeroed where dropped, then ReLU + bf16 as in epi_block_fwd; the ReLU mask is
+// built from the packed value, so it is "kept and z > 0" and the backward needs nothing else to know the dropped units
+__device__ __forceinline__ float drop_scale(float z, uint32_t keep, int j, float s) { return ((keep >> j) & 1u) ? z * s : 0.f; }
+__device__ __forceinline__ uint32_t epi_mask_bits(const uint32_t (&w)[16]) {
+  uint32_t acc[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+  for (int i = 0; i < 16; ++i)
+    acc[i & 3] |= ((w[i] + 0x7FFF7FFFu) >> (15 - i)) & (0x00010001u << i);
+  return (acc[0] | acc[1]) | (acc[2] | acc[3]);
+}
+__device__ __forceinline__ uint32_t epi_block_fwd_drop(const uint32_t (&v)[32], const float4 (&b)[8], uint32_t keep,
+                                                       float s, uint32_t (&w)[16]) {
+#pragma unroll
+  for (int g4 = 0; g4 < 8; ++g4) {
+    const int j = 4 * g4;
+    w[2 * g4] = pack_relu_bf16x2(drop_scale(__uint_as_float(v[j]) + b[g4].x, keep, j, s),
+                                 drop_scale(__uint_as_float(v[j + 1]) + b[g4].y, keep, j + 1, s));
+    w[2 * g4 + 1] = pack_relu_bf16x2(drop_scale(__uint_as_float(v[j + 2]) + b[g4].z, keep, j + 2, s),
+                                     drop_scale(__uint_as_float(v[j + 3]) + b[g4].w, keep, j + 3, s));
+  }
+  return epi_mask_bits(w);
+}
+__device__ __forceinline__ uint32_t epi_block_fwd_drop_sb(const uint32_t (&v)[32], const float* bias_smem, uint32_t keep,
+                                                          float s, uint32_t (&w)[16]) {
+#pragma unroll
+  for (int g4 = 0; g4 < 8; ++g4) {
+    const float4 b = *reinterpret_cast<const float4*>(bias_smem + 4 * g4);
+    const int j = 4 * g4;
+    w[2 * g4] = pack_relu_bf16x2(drop_scale(__uint_as_float(v[j]) + b.x, keep, j, s),
+                                 drop_scale(__uint_as_float(v[j + 1]) + b.y, keep, j + 1, s));
+    w[2 * g4 + 1] = pack_relu_bf16x2(drop_scale(__uint_as_float(v[j + 2]) + b.z, keep, j + 2, s),
+                                     drop_scale(__uint_as_float(v[j + 3]) + b.w, keep, j + 3, s));
+  }
+  return epi_mask_bits(w);
+}
+// dX of a layer whose input had dropout: w_i = bf16x2(v * s) & mask (multiplied in fp32, rounded once)
+__device__ __forceinline__ void epi_block_dx_scaled(const uint32_t (&v)[32], uint32_t mask_word, float s, uint32_t (&w)[16]) {
+#pragma unroll
+  for (int i = 0; i < 16; ++i)
+    w[i] = relu_mask_apply(pack_bf16x2(__uint_as_float(v[2 * i]) * s, __uint_as_float(v[2 * i + 1]) * s), mask_word, i);
 }
 
 }  // namespace tc

@@ -156,11 +156,18 @@ def _refuse_mode_scales(has_scales, w_smooth_corr):
                                   "and an all-reduce of the scale gradient; use the single-GPU TrainStepEngine")
 
 
+def _refuse_dropout(p):
+    if float(p) > 0.0:
+        raise NotImplementedError("the vertex-sharded step does not support dropout (got %g): use the single-GPU "
+                                  "TrainStepEngine, or dropout = 0.0" % float(p))
+
+
 class ShardedTrainStepEngine(TrainStepEngine):
     def __init__(self, h_local, U_base_local, plans, params: FlatParams, cfg: StepConfig, lam_target=None,
                  mlp_mode="fp32", group=None, symmetric=True, pairs=None):
         dev = h_local.device
         _refuse_mode_scales(params.mode_scales is not None, cfg.w_smooth_corr)
+        _refuse_dropout(cfg.dropout)
         if not symmetric:
             raise NotImplementedError("the vertex-sharded step needs symmetric K, M (FEM / tufted Laplacians): the "
                                       "transposed products of a non-symmetric operator would need a halo scatter-add")
@@ -273,6 +280,7 @@ def make_sharded_engine(gnn, x_feats, edge_index, U_base, K, M, lam_target, opti
     vertex range, and builds the rank-local engine."""
     import torch.nn as nn
     _refuse_mode_scales(hasattr(gnn.model, "mode_scales"), getattr(gnn, "w_smooth_corr", 0.0))
+    _refuse_dropout(getattr(gnn, "dropout", 0.0) or 0.0)
     dev = gnn.device
     h_global = gnn.model.corrector_input(x_feats.to(dev), edge_index.to(dev))
     plan = resolve_send_lists(LevelPlan(K, M, rank, world), group)

@@ -71,20 +71,26 @@ class FlatParams:
 
 
 class Fp32Mlp:
-    """Layer-wise fp32 forward / backward with saved activations."""
+    """Layer-wise fp32 forward / backward with saved activations.  dropout (ops.Dropout or None): dropout after every
+    hidden ReLU, hidden layer l drawing the masks of layer index l at the step passed to forward()."""
 
-    def __init__(self, n, params: FlatParams, device):
+    def __init__(self, n, params: FlatParams, device, dropout=None):
         self.p = params
+        self.dropout = dropout
         dims = params.dims
         self.acts = [torch.empty((n, d), dtype=torch.float32, device=device) for d in dims[1:]]
         wmax = max(dims[1:-1]) if len(dims) > 2 else dims[0]
         self.dx = [torch.empty((n, wmax), dtype=torch.float32, device=device) for _ in range(2)]
 
-    def forward(self, h, U_base=None, scale=0.0, U_pred=None, scale_dev=None):
+    def forward(self, h, U_base=None, scale=0.0, U_pred=None, scale_dev=None, step=0, step_dev=None):
         x = h
         L = len(self.p.W)
         for l in range(L):
-            ops.linear_fwd(x, self.p.W[l], self.p.b[l], relu=(l < L - 1), out=self.acts[l])
+            if self.dropout is not None and l < L - 1:
+                ops.linear_fwd_dropout(x, self.p.W[l], self.p.b[l], self.dropout, step, l, step_dev=step_dev,
+                                       out=self.acts[l])
+            else:
+                ops.linear_fwd(x, self.p.W[l], self.p.b[l], relu=(l < L - 1), out=self.acts[l])
             x = self.acts[l]
         if U_pred is not None:
             ops.axpy_out(U_base, x, scale, out=U_pred, alpha_dev=scale_dev)
@@ -99,7 +105,11 @@ class Fp32Mlp:
             x = self.acts[l - 1] if l > 0 else h
             need_dx = l > 0
             dx = self.dx[l & 1][:, :x.shape[1]] if need_dx else None
-            ops.linear_bwd(x, self.p.W[l], dy, need_dx, relu_mask=need_dx, dW=self.p.dW[l], db=self.p.db[l], dX=dx)
+            if need_dx and self.dropout is not None:
+                ops.linear_bwd_dropout(x, self.p.W[l], dy, self.dropout, dW=self.p.dW[l], db=self.p.db[l], dX=dx)
+            else:
+                ops.linear_bwd(x, self.p.W[l], dy, need_dx, relu_mask=need_dx, dW=self.p.dW[l], db=self.p.db[l],
+                               dX=dx)
             if on_layer_grads is not None:
                 on_layer_grads(l)
             dy = dx
@@ -108,7 +118,11 @@ class Fp32Mlp:
 class StepConfig:
     def __init__(self, lr=1e-3, weight_decay=1e-5, corr_scale=10.0, w_res=1000.0, w_orth=10.0, w_trace=0.0,
                  w_order=0.0, w_eigen=0.0, grad_clip=10.0, beta1=0.9, beta2=0.999, eps=1e-8, ramp_epochs=5000.0,
-                 w_mean=0.0, w_smooth=0.0, w_smooth_corr=0.0):
+                 w_mean=0.0, w_smooth=0.0, w_smooth_corr=0.0, dropout=0.0, dropout_seed=None):
+        # dropout: probability of the nn.Dropout after every hidden ReLU (parameters.yml `dropout`), in [0, 1);
+        # dropout_seed: 64-bit key of the keep masks (None: one draw from torch's generator when the engine is built)
+        self.dropout = ops.check_dropout_p(dropout)
+        self.dropout_seed = dropout_seed
         # w_mean / w_smooth: per-level zero-mean and smoothness terms of the notebook variants (SURVEY 8a-bis);
         # w_smooth_corr: the smoothness of the correction, w sum corr o (K corr) / (n k) per level
         self.w_mean, self.w_smooth, self.w_smooth_corr = w_mean, w_smooth, w_smooth_corr
@@ -146,11 +160,17 @@ class TrainStepEngine:
         self.lam_target = lam_target.to(**f32).contiguous() if lam_target is not None else None
         self.mlp_mode = mlp_mode
         self.n_mlp = self._mlp_rows()                  # rows the corrector is evaluated on (all, unless sharded)
+        self.dropout = None
+        if cfg.dropout > 0.0:
+            seed = cfg.dropout_seed
+            if seed is None:
+                seed = int(torch.randint(0, 2 ** 63 - 1, (1,)).item())
+            self.dropout = ops.Dropout(cfg.dropout, seed)
         if mlp_mode == "fp32":
-            self.mlp = Fp32Mlp(self.n_mlp, params, self.dev)
+            self.mlp = Fp32Mlp(self.n_mlp, params, self.dev, dropout=self.dropout)
         elif mlp_mode == "bf16":
             from .mlp_tc import TcMlp
-            self.mlp = TcMlp(self.n_mlp, params, self.dev, h[:self.n_mlp])
+            self.mlp = TcMlp(self.n_mlp, params, self.dev, h[:self.n_mlp], dropout=self.dropout)
             self.mlp.want_corr = False
         else:
             raise ValueError("mlp_mode must be 'fp32' or 'bf16'")
@@ -184,12 +204,15 @@ class TrainStepEngine:
     def scale_for(self, epoch):
         return self.cfg.corr_scale * min(1.0, epoch / self.cfg.ramp_epochs)
 
-    def forward(self, scale, scale_dev=None):
+    def forward(self, scale, scale_dev=None, step_dev=None):
+        """step_dev (device int32, graph replay) or else params.step_count + 1: the Adam step this forward feeds, which
+        selects the dropout masks."""
         m = self.n_mlp
+        step = self.params.step_count + 1
         if not self.adaptive:
             return self.mlp.forward(self.h[:m], U_base=self.U_base[:m], scale=scale, U_pred=self.U_pred[:m],
-                                    scale_dev=scale_dev)
-        self.mlp.forward(self.h[:m])
+                                    scale_dev=scale_dev, step=step, step_dev=step_dev)
+        self.mlp.forward(self.h[:m], step=step, step_dev=step_dev)
         self.mode_scale_forward(scale, scale_dev)
         return self.corr_raw
 
@@ -322,7 +345,7 @@ class TrainStepEngine:
 
     def _step_body_dev(self):
         sd = self.hyper[0:1]
-        self.forward(0.0, scale_dev=sd)
+        self.forward(0.0, scale_dev=sd, step_dev=self.hyper.view(torch.int32)[2:3])
         self.loss_forward()
         self.loss_backward(0.0, scale_dev=sd)
         self.mlp_backward()

@@ -46,8 +46,9 @@ class TcMlp:
     top: the dW kernel of layer l (side stream) and the dX kernel that produces dZ of layer l - 1 (main stream) run
     concurrently on two disjoint shares of the SMs; layer 0 needs no dX, so its dW kernel takes the whole GPU."""
 
-    def __init__(self, n, params, device, h=None, chain_fwd=True):
+    def __init__(self, n, params, device, h=None, chain_fwd=True, dropout=None):
         self.p, self.n, self.dev = params, n, device
+        self.dropout = dropout                                # ops.Dropout after every hidden ReLU, or None
         self.chain_fwd = bool(chain_fwd)
         dims = params.dims                                    # [in, h1, ..., out]
         L = len(dims) - 1
@@ -95,20 +96,30 @@ class TcMlp:
             call("ep_tc_pack_weight_bf16", W.shape[0], W.shape[1], self.pd[l + 1], self.pd[l], _p(W), _p(self.Wp[l]),
                  _p(self.WTp[l]) if l > 0 else None, _stream())
 
-    def forward(self, h, U_base=None, scale=0.0, U_pred=None, scale_dev=None):
+    def forward(self, h, U_base=None, scale=0.0, U_pred=None, scale_dev=None, step=0, step_dev=None):
+        """step / step_dev (device int32, overrides step): the Adam step that selects the dropout masks."""
         if self._packed_version != (h.data_ptr(), h._version):
             self.input_changed(h)
         self._pack_weights()
+        d = self.dropout
         if self.chain_fwd:
             corr = self.corr if (self.want_corr or U_pred is None) else None
-            call("ep_tc_chain_fwd_bf16", self.n, self.L, self._t_pd, self._t_out, _p(self.x0), self._t_Wp, self._t_b,
-                 self._t_acts, self._t_masks, _p(corr), self.corr.stride(0), _p(U_base), float(scale), _p(scale_dev),
-                 _p(U_pred), U_pred.stride(0) if U_pred is not None else 0, _stream())
+            args = (self.n, self.L, self._t_pd, self._t_out, _p(self.x0), self._t_Wp, self._t_b, self._t_acts,
+                    self._t_masks, _p(corr), self.corr.stride(0), _p(U_base), float(scale), _p(scale_dev), _p(U_pred),
+                    U_pred.stride(0) if U_pred is not None else 0)
+            if d is None:
+                call("ep_tc_chain_fwd_bf16", *args, _stream())
+            else:
+                call("ep_tc_chain_fwd_dropout_bf16", *args, None, d.p, d.seed, int(step), _p(step_dev), 0, _stream())
             return self.corr
         x = self.x0
         for l in range(self.L - 1):
-            call("ep_tc_linear_fwd_bf16", self.n, self.pd[l], self.dims[l + 1], self.pd[l + 1], _p(x), _p(self.Wp[l]),
-                 _p(self.p.b[l]), 1, _p(self.acts[l]), _p(self.masks[l]), _stream())
+            args = (self.n, self.pd[l], self.dims[l + 1], self.pd[l + 1], _p(x), _p(self.Wp[l]), _p(self.p.b[l]))
+            if d is None:
+                call("ep_tc_linear_fwd_bf16", *args, 1, _p(self.acts[l]), _p(self.masks[l]), _stream())
+            else:
+                call("ep_tc_linear_fwd_dropout_bf16", *args, _p(self.acts[l]), _p(self.masks[l]), d.p, d.seed, int(step),
+                     _p(step_dev), l, 0, _stream())
             x = self.acts[l]
         l = self.L - 1
         call("ep_tc_linear_final_bf16", self.n, self.pd[l], self.dims[-1], self.pd[-1], _p(x), _p(self.Wp[l]),
@@ -138,8 +149,12 @@ class TcMlp:
                     call("ep_tc_linear_dw_bf16", self.n, self.dims[l + 1], self.dims[l], dz_w, self.pd[l], _p(dz), _p(act),
                          _p(self.p.dW[l]), _p(self.p.db[l]), _p(self.ws), self.ws_bytes, n_dw, _stream())
                 nxt = self.dz[l & 1]
-                call("ep_tc_linear_dx_bf16", self.n, dz_w, self.pd[l], _p(dz), _p(self.WTp[l]), _p(self.masks[l - 1]),
-                     _p(nxt), n_dx, _stream())
+                if self.dropout is None:
+                    call("ep_tc_linear_dx_bf16", self.n, dz_w, self.pd[l], _p(dz), _p(self.WTp[l]), _p(self.masks[l - 1]),
+                         _p(nxt), n_dx, _stream())
+                else:
+                    call("ep_tc_linear_dx_dropout_bf16", self.n, dz_w, self.pd[l], _p(dz), _p(self.WTp[l]),
+                         _p(self.masks[l - 1]), _p(nxt), self.dropout.p, n_dx, _stream())
                 main.wait_stream(side)
                 dz, dz_w = nxt, self.pd[l]
             else:

@@ -10,6 +10,7 @@ operands (OperatorPair(..., dtype=torch.float64)).  Nothing is cast implicitly.
 """
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _cabi
@@ -444,6 +445,67 @@ def linear_bwd(X, W, dY, need_dX, relu_mask, dW=None, db=None, dX=None):
     call("ep_linear_bwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(dY), dY.stride(0),
          _ptr(dX) if need_dX else None, dX.stride(0) if need_dX else 0, 1 if relu_mask else 0, _ptr(dW), _ptr(db),
          _ptr(buf), need, _stream())
+    return dX, dW, db
+
+
+class Dropout:
+    """Dropout after every hidden ReLU of the fused step (nn.Dropout(p) of corrector_model.py::_build_net in training
+    mode).  Keep masks are a pure function of (seed, step, layer, row, col) (csrc/dropout.cuh), regenerated by every
+    kernel; they are NOT torch's RNG stream, so a dropout run matches the reference in distribution only."""
+
+    def __init__(self, p, seed):
+        self.p = check_dropout_p(p)
+        self.seed = int(seed) % (1 << 64)
+
+    @property
+    def thr(self):
+        return round(float(self.p) * 65536.0)
+
+    @property
+    def scale(self):
+        """s = 1 / (1 - thr / 65536) in fp32, as the kernels use it."""
+        return float(np.float32(1.0) / (np.float32(1.0) - np.float32(self.thr) / np.float32(65536.0)))
+
+
+def check_dropout_p(p):
+    """p as the kernels see it (fp32); raises ValueError unless 0 <= p < 1 with round(p * 65536) < 65536."""
+    p32 = float(np.float32(p))
+    if not (0.0 <= p32 < 1.0) or round(p32 * 65536.0) >= 65536:
+        raise ValueError("dropout must lie in [0, 1) (got %r)" % (p,))
+    return p32
+
+
+def dropout_keep_mask(n, width, drop, step, layer, row0=0, device="cuda"):
+    """(n, width) uint8 keep mask of hidden layer `layer` at Adam step `step` (1 = kept)."""
+    out = torch.empty((n, width), dtype=torch.uint8, device=device)
+    call("ep_dropout_keep_mask_u8", n, width, drop.p, drop.seed, int(step), None, int(layer), int(row0), _ptr(out),
+         _stream())
+    return out
+
+
+def linear_fwd_dropout(X, W, b, drop, step, layer, step_dev=None, out=None):
+    """Y = keep ? relu(X W^T + b) * s : 0 (fp32); step_dev (device int32) overrides step."""
+    X, W = _check(_rowmajor(X)), _check(W)
+    n, d_in = X.shape
+    d_out = W.shape[0]
+    assert W.is_contiguous() and W.shape[1] == d_in
+    Y = out if out is not None else torch.empty((n, d_out), device=X.device, dtype=torch.float32)
+    call("ep_linear_fwd_dropout_f32", n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(b), _ptr(Y), Y.stride(0),
+         drop.p, drop.seed, int(step), _ptr(step_dev), int(layer), 0, _stream())
+    return Y
+
+
+def linear_bwd_dropout(X, W, dY, drop, dW=None, db=None, dX=None):
+    """linear_bwd for a layer whose input X came out of a hidden layer with dropout: dX = (dY W) * [X > 0] * s."""
+    X, W, dY = _check(_rowmajor(X)), _check(W), _check(_rowmajor(dY))
+    n, d_in = X.shape
+    d_out = W.shape[0]
+    dW = dW if dW is not None else torch.empty_like(W)
+    db = db if db is not None else torch.empty(d_out, device=X.device, dtype=torch.float32)
+    dX = dX if dX is not None else torch.empty((n, d_in), device=X.device, dtype=torch.float32)
+    buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device)
+    call("ep_linear_bwd_dropout_f32", n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(dY), dY.stride(0), _ptr(dX),
+         dX.stride(0), drop.p, _ptr(dW), _ptr(db), _ptr(buf), need, _stream())
     return dX, dW, db
 
 

@@ -177,8 +177,6 @@ class MultigridGNN:
     # ------------------------------------------------------------------ hot loop
     def _make_engine(self, x_feats, edge_index, A_norm, U_base, K_list, M_list, lambda_target, node_offsets,
                      optimizer):
-        if self.dropout and self.dropout > 0.0:
-            raise NotImplementedError("the fused training step supports dropout = 0.0 (the reference default)")
         x_feats = self._dev_f32(x_feats)
         if self.model_type in ('simple', 'adaptive'):
             h = self.model.corrector_input(x_feats, edge_index.to(self.device))
@@ -191,7 +189,8 @@ class MultigridGNN:
                                  w_res=self.w_res, w_orth=self.w_orth, w_trace=self.w_trace, w_order=self.w_order,
                                  w_eigen=self.w_eigen, grad_clip=self.grad_clip, beta1=group['betas'][0],
                                  beta2=group['betas'][1], eps=group['eps'], w_smooth=self.w_smooth,
-                                 w_smooth_corr=self.w_smooth_corr)
+                                 w_smooth_corr=self.w_smooth_corr, dropout=float(self.dropout or 0.0),
+                                 dropout_seed=self.seed)
         pairs = [self._pair(K, M) for K, M in zip(K_list, M_list)]
         return _engine.TrainStepEngine(h, self._dev_f32(U_base), pairs, node_offsets, params, cfg,
                                        lam_target=lambda_target, mlp_mode=self.mlp_mode)

@@ -250,6 +250,30 @@ EP_API int ep_linear_bwd_f32(int n, int in, int out, const float* X, int ldx, co
                       const float* dY, int lddy, float* dX, int lddx, int relu_mask,
                       float* dW, float* db, void* workspace, size_t workspace_bytes,
                       ep_stream_t stream);
+
+/* ---- dropout after a hidden ReLU (the nn.Dropout(p) of corrector_model.py::_build_net in training mode) ----------
+ * Keep masks are regenerated, never stored: unit (row, col) of hidden layer `layer` is kept iff the 16-bit lane of
+ * Philox4x32-10(key = seed, counter = (row0 + row, col / 8, layer, step)) that belongs to col is >= thr, with
+ * thr = round(p * 65536) (0 <= p, thr < 65536, else EP_ERR_INVALID); kept units are scaled by s = 1 / (1 - thr / 65536)
+ * (fp32), so E[y] = relu(z).  Lane of feature 8c + 2j: low half of output word j; 8c + 2j + 1: its high half.  `row`
+ * is the row of the MLP input, `col` the output feature, `step` the Adam step t the forward feeds; step_dev (device,
+ * may be NULL) overrides step so a captured graph draws fresh masks each replay.  Not torch's RNG stream: dropout
+ * runs match the reference in distribution, not bit for bit.  Both MLP modes draw identical masks.
+ * The backward needs no mask: the stored activation is non-zero exactly where the unit is kept and z > 0.
+ * ep_dropout_keep_mask_u8: keep[r * width + c] = 1 / 0 for rows 0..n-1 (tests, hosts that apply the mask themselves). */
+EP_API int ep_dropout_keep_mask_u8(long long n, int width, float p, unsigned long long seed, int step,
+                                   const int* step_dev, int layer, long long row0, unsigned char* keep,
+                                   ep_stream_t stream);
+/* Y = keep ? relu(X W^T + b) * s : 0  (ep_linear_fwd_f32 with act = 1, then nn.Dropout) */
+EP_API int ep_linear_fwd_dropout_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* b,
+                              float* Y, int ldy, float p, unsigned long long seed, int step,
+                              const int* step_dev, int layer, long long row0, ep_stream_t stream);
+/* ep_linear_bwd_f32 for a layer whose input X is the output of a hidden layer with dropout p:
+ * dX = (dY W) * [X > 0] * s;  dW, db, workspace as there. */
+EP_API int ep_linear_bwd_dropout_f32(int n, int in, int out, const float* X, int ldx, const float* W,
+                              const float* dY, int lddy, float* dX, int lddx, float p,
+                              float* dW, float* db, void* workspace, size_t workspace_bytes,
+                              ep_stream_t stream);
 /* fp64 forms (plain DFMA, same tiling and fixed-order split-K): the dense layers of the notebook networks in double -
  * `MLP` of scripts/simplified_loss.ipynb cell 0 and scripts/loss_with_rigid_body.ipynb cell 0, `EigenfunctionNN` of
  * delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1. */
@@ -315,6 +339,24 @@ EP_API int ep_tc_chain_fwd_bf16(int n, int n_layers, const int* dims_padded, con
                          const void* const* Wp, const float* const* bias, void* const* act_out,
                          void* const* relu_mask_out, float* corr, int ldc, const float* U_base, float scale,
                          const float* scale_dev, float* U_pred, int ldu, ep_stream_t stream);
+/* Dropout forms of the bf16 path (masks and scale as for ep_linear_fwd_dropout_f32; corrector_model.py::_build_net,
+ * nn.Dropout after every hidden ReLU).  The forward scales by s and zeroes dropped units before the bf16 pack, so the
+ * ReLU bit mask it writes is "kept and > 0"; the dX form multiplies by s in fp32 and rounds once.
+ * Chain: hidden layer l uses layer index l and p_layers[l] (HOST array of n_layers - 1 entries) or, when p_layers is
+ * NULL, p for every hidden layer.  Bit-identical to the layer-by-layer dropout entry points. */
+EP_API int ep_tc_linear_fwd_dropout_bf16(int n, int in_padded, int out, int out_padded, const void* A_packed,
+                                  const void* Wp, const float* bias, void* out_packed, void* relu_mask_out, float p,
+                                  unsigned long long seed, int step, const int* step_dev, int layer, long long row0,
+                                  ep_stream_t stream);
+EP_API int ep_tc_linear_dx_dropout_bf16(int n, int out_padded, int in_padded, const void* dZ_packed, const void* WTp,
+                                 const void* relu_mask, void* dZprev_packed, float p, int max_ctas,
+                                 ep_stream_t stream);
+EP_API int ep_tc_chain_fwd_dropout_bf16(int n, int n_layers, const int* dims_padded, const int* dims_out,
+                                 const void* A0_packed, const void* const* Wp, const float* const* bias,
+                                 void* const* act_out, void* const* relu_mask_out, float* corr, int ldc,
+                                 const float* U_base, float scale, const float* scale_dev, float* U_pred, int ldu,
+                                 const float* p_layers, float p, unsigned long long seed, int step,
+                                 const int* step_dev, long long row0, ep_stream_t stream);
 /* dW = dZ^T act (fp32 [out x in]) and db = column sums of dZ; deterministic two-stage reduction. */
 EP_API size_t ep_tc_dw_workspace_bytes(void);
 EP_API int ep_tc_linear_dw_bf16(int n, int out, int in, int out_padded, int in_padded, const void* dZ_packed,
