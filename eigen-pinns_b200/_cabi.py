@@ -57,6 +57,12 @@ SIGNATURES = {
     "ep_linear_bwd_workspace_bytes_f64": (c_sz, [c_int, c_int, c_int]),
     "ep_linear_bwd_f64": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_int, c_p, c_int, c_int,
                                   c_p, c_p, c_p, c_sz, c_p]),
+    "ep_linear_act_fwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_p, c_int, c_int, c_p]),
+    "ep_linear_act_fwd_f64": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_p, c_p, c_int, c_p, c_int, c_int, c_p]),
+    "ep_linear_act_bwd_f32": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_int, c_int, c_p, c_p, c_int, c_p, c_int,
+                                      c_p, c_p, c_p, c_sz, c_p]),
+    "ep_linear_act_bwd_f64": (c_int, [c_int, c_int, c_int, c_p, c_int, c_p, c_int, c_int, c_p, c_p, c_int, c_p, c_int,
+                                      c_p, c_p, c_p, c_sz, c_p]),
     "ep_tc_pad_features": (c_int, [c_int, c_int]),
     "ep_tc_packed_rows_bytes": (c_sz, [c_int, c_int]),
     "ep_tc_packed_weight_bytes": (c_sz, [c_int, c_int]),
@@ -121,6 +127,7 @@ KERNELS_PER_CALL = {
     "ep_halo_exchange_f32": 1,
     "ep_spmm_csr_f64": 1, "ep_spmm2_csr_f64": 1, "ep_spmm2_sum_csr_f64": 1, "ep_eigen_partials_f64": 2,
     "ep_linear_fwd_f64": 1, "ep_linear_bwd_f64": 5,
+    "ep_linear_act_fwd_f32": 1, "ep_linear_act_fwd_f64": 1, "ep_linear_act_bwd_f32": 5, "ep_linear_act_bwd_f64": 5,
     "ep_mode_scale_fwd_f32": 1, "ep_mode_scale_bwd_f32": 2,
     "ep_dropout_keep_mask_u8": 1, "ep_linear_fwd_dropout_f32": 1, "ep_linear_bwd_dropout_f32": 5,
     "ep_tc_linear_fwd_dropout_bf16": 1, "ep_tc_linear_dx_dropout_bf16": 1, "ep_tc_chain_fwd_dropout_bf16": 1,

@@ -169,6 +169,110 @@ gemm_dropout_kernel(int M, int N, int K, const float* __restrict__ A, long long 
   }
 }
 
+// Activation epilogues of the notebook networks (variants.py), ep_linear_act_{fwd,bwd}_*.  Accurate libm math (expf / exp,
+// sinf / sin, cosf / cos, tanhf / tanh), no fast-math intrinsics.
+enum Act { ACT_NONE = 0, ACT_RELU = 1, ACT_SILU = 2, ACT_SIN = 3, ACT_TANH = 4 };
+
+__device__ __forceinline__ float exp_t(float v) { return expf(v); }
+__device__ __forceinline__ double exp_t(double v) { return exp(v); }
+__device__ __forceinline__ float sin_t(float v) { return sinf(v); }
+__device__ __forceinline__ double sin_t(double v) { return sin(v); }
+__device__ __forceinline__ float cos_t(float v) { return cosf(v); }
+__device__ __forceinline__ double cos_t(double v) { return cos(v); }
+__device__ __forceinline__ float tanh_t(float v) { return tanhf(v); }
+__device__ __forceinline__ double tanh_t(double v) { return tanh(v); }
+
+template <int ACT, typename T>
+__device__ __forceinline__ T act_fwd(T z) {
+  if (ACT == ACT_RELU) return relu_t(z);
+  if (ACT == ACT_SILU) return z / (T(1) + exp_t(-z));
+  if (ACT == ACT_SIN) return sin_t(z);
+  if (ACT == ACT_TANH) return tanh_t(z);
+  return z;
+}
+
+// act'(z) from what the backward reads: z for SiLU (s (1 + z (1 - s)), s = sigmoid z) and sin (cos z); the activation
+// x = tanh z itself for tanh (1 - x^2)
+template <int ACT, typename T>
+__device__ __forceinline__ T act_grad(T v) {
+  if (ACT == ACT_SILU) {
+    const T s = T(1) / (T(1) + exp_t(-v));
+    return s * (T(1) + v * (T(1) - s));
+  }
+  if (ACT == ACT_SIN) return cos_t(v);
+  return T(1) - v * v;
+}
+
+// The tile and main loop of gemm_kernel<T, true, !DX> (no split-K), kept apart so that gemm_kernel's code does not
+// change, with an activation epilogue:
+//   forward (DX = false, A = X, B = W^T):  z = X W^T + b, Z = z if Z != NULL, C = act(z)   (ACT: any Act)
+//   dX      (DX = true,  A = dY, B = W):   C = (dY W) * act'(aux), aux = Z of the layer that produced X (SiLU, sin) or
+//                                          X itself (tanh)
+// Three CTAs per SM (at most 85 registers): left to its default, ptxas gives the fp32 sin dX form 64 registers and
+// spills one of them in the main loop.
+template <typename T, int ACT, bool DX>
+__global__ void __launch_bounds__(256, 3)
+gemm_act_kernel(int M, int N, int K, const T* __restrict__ A, long long sa_i, long long sa_k, const T* __restrict__ B,
+                long long sb_k, long long sb_j, T* __restrict__ C, int ldc, const T* __restrict__ bias,
+                const T* __restrict__ aux, int ld_aux, T* __restrict__ Z, int ldz) {
+  constexpr bool A_KC = true, B_KC = !DX;
+  __shared__ __align__(16) T As[BK][PITCH];
+  __shared__ __align__(16) T Bs[BK][PITCH];
+  const int tid = threadIdx.x;
+  const int ty = tid >> 4, tx = tid & 15;
+  const int i0 = blockIdx.y * BM, j0 = blockIdx.x * BN;
+  T acc[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) acc[i][j] = T(0);
+
+  for (int k0 = 0; k0 < K; k0 += BK) {
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int e = tid + 256 * q;
+      int ai, ak, bk, bj;
+      if (A_KC) { ai = e >> 4; ak = e & 15; } else { ak = e >> 6; ai = e & 63; }
+      if (B_KC) { bj = e >> 4; bk = e & 15; } else { bk = e >> 6; bj = e & 63; }
+      const int gi = i0 + ai, gk = k0 + ak;
+      As[ak][ai] = (gi < M && gk < K) ? __ldg(A + gi * sa_i + gk * sa_k) : T(0);
+      const int gj = j0 + bj, gk2 = k0 + bk;
+      Bs[bk][bj] = (gj < N && gk2 < K) ? __ldg(B + gk2 * sb_k + gj * sb_j) : T(0);
+    }
+    __syncthreads();
+#pragma unroll
+    for (int kk = 0; kk < BK; ++kk) {
+      T av[4], bv[4];
+      lds4(&As[kk][ty * 4], av);
+      lds4(&Bs[kk][tx * 4], bv);
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fma_t(av[i], bv[j], acc[i][j]);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int gi = i0 + ty * 4 + i;
+    if (gi >= M) continue;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int gj = j0 + tx * 4 + j;
+      if (gj >= N) continue;
+      T v = acc[i][j];
+      if (DX) {
+        v *= act_grad<ACT>(__ldg(aux + (size_t)gi * ld_aux + gj));
+      } else {
+        if (bias) v += __ldg(bias + gj);
+        if (Z) Z[(size_t)gi * ldz + gj] = v;
+        v = act_fwd<ACT>(v);
+      }
+      C[(size_t)gi * ldc + gj] = v;
+    }
+  }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256)
 sum_splits_kernel(int n_split, size_t len, const T* __restrict__ parts, T* __restrict__ out) {
@@ -307,6 +411,93 @@ size_t bwd_workspace_bytes(int n, int in, int out, size_t elem) {
   return elem * ((size_t)p.n_split * in * out + (size_t)p.cs_blocks * out);
 }
 
+// Y = act(X W^T + b), Z = X W^T + b (if Z != NULL); row slabs of 65535 tiles as in linear_fwd
+template <typename T, int ACT>
+int linear_act_fwd(int n, int in, int out, const T* X, int ldx, const T* W, const T* b, T* Y, int ldy, T* Z, int ldz,
+                   cudaStream_t st) {
+  const int slab = 65535 * BM;
+  for (int r0 = 0; r0 < n; r0 += slab) {
+    const int rows = (n - r0) < slab ? (n - r0) : slab;
+    dim3 grid(ep::ceil_div(out, BN), ep::ceil_div(rows, BM), 1);
+    gemm_act_kernel<T, ACT, false><<<grid, 256, 0, st>>>(
+        rows, out, in, X + (size_t)r0 * ldx, ldx, 1, W, 1, in, Y + (size_t)r0 * ldy, ldy, b, nullptr, 0,
+        Z ? Z + (size_t)r0 * ldz : nullptr, ldz);
+    EP_LAUNCH_CHECK("gemm_act_kernel<fwd>");
+  }
+  return EP_OK;
+}
+
+// dX = (dY W) * act'(aux)
+template <typename T, int ACT>
+int linear_act_dx(int n, int in, int out, const T* aux, int ld_aux, const T* W, const T* dY, int lddy, T* dX, int lddx,
+                  cudaStream_t st) {
+  const int slab = 65535 * BM;
+  for (int r0 = 0; r0 < n; r0 += slab) {
+    const int rows = (n - r0) < slab ? (n - r0) : slab;
+    dim3 grid(ep::ceil_div(in, BN), ep::ceil_div(rows, BM), 1);
+    gemm_act_kernel<T, ACT, true><<<grid, 256, 0, st>>>(
+        rows, in, out, dY + (size_t)r0 * lddy, lddy, 1, W, in, 1, dX + (size_t)r0 * lddx, lddx, nullptr,
+        aux + (size_t)r0 * ld_aux, ld_aux, nullptr, 0);
+    EP_LAUNCH_CHECK("gemm_act_kernel<dX>");
+  }
+  return EP_OK;
+}
+
+// EP_REQUIRE with the entry point's name in the message
+#define ACT_REQUIRE(cond, msg)                                                  \
+  do {                                                                          \
+    if (!(cond)) { ep::set_error("%s: %s", name, msg); return EP_ERR_INVALID; } \
+  } while (0)
+
+template <typename T>
+int act_fwd_entry(const char* name, int n, int in, int out, const T* X, int ldx, const T* W, const T* b, T* Y, int ldy, T* Z, int ldz,
+                  int act, ep_stream_t stream) {
+  ACT_REQUIRE(n >= 0 && in > 0 && out > 0, "bad size");
+  ACT_REQUIRE(act >= ACT_NONE && act <= ACT_TANH, "unknown activation (0 none, 1 ReLU, 2 SiLU, 3 sin, 4 tanh)");
+  if (n == 0) return EP_OK;
+  ACT_REQUIRE(X && W && Y, "null pointer");
+  ACT_REQUIRE(ldx >= in && ldy >= out && (!Z || ldz >= out), "leading dimension too small");
+  ACT_REQUIRE(ep::ceil_div(n, BM) <= 65535 * 1024, "n too large");
+  cudaStream_t st = ep::as_stream(stream);
+  switch (act) {
+    case ACT_NONE: return linear_act_fwd<T, ACT_NONE>(n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, st);
+    case ACT_RELU: return linear_act_fwd<T, ACT_RELU>(n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, st);
+    case ACT_SILU: return linear_act_fwd<T, ACT_SILU>(n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, st);
+    case ACT_SIN: return linear_act_fwd<T, ACT_SIN>(n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, st);
+    default: return linear_act_fwd<T, ACT_TANH>(n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, st);
+  }
+}
+
+// act_x 0 / 1: dX through linear_bwd's gemm_kernel (no mask / [X > 0]); 2 - 4: dW, db there, dX by gemm_act_kernel
+template <typename T>
+int act_bwd_entry(const char* name, int n, int in, int out, const T* X, int ldx, const T* Zx, int ldzx, int act_x, const T* W,
+                  const T* dY, int lddy, T* dX, int lddx, T* dW, T* db, void* workspace, size_t workspace_bytes,
+                  ep_stream_t stream) {
+  ACT_REQUIRE(n > 0 && in > 0 && out > 0, "bad size");
+  ACT_REQUIRE(act_x >= ACT_NONE && act_x <= ACT_TANH, "unknown activation (0 none, 1 ReLU, 2 SiLU, 3 sin, 4 tanh)");
+  ACT_REQUIRE(X && W && dY && dW && db && workspace, "null pointer");
+  const bool needs_z = dX && (act_x == ACT_SILU || act_x == ACT_SIN);
+  ACT_REQUIRE(!needs_z || Zx, "Zx is NULL but the activation of X (SiLU or sin) needs its pre-activation");
+  ACT_REQUIRE(ldx >= in && lddy >= out && (!dX || lddx >= in) && (!needs_z || ldzx >= in),
+             "leading dimension too small");
+  if (workspace_bytes < bwd_workspace_bytes(n, in, out, sizeof(T))) {
+    ep::set_error("%s: workspace too small", name);
+    return EP_ERR_WORKSPACE;
+  }
+  cudaStream_t st = ep::as_stream(stream);
+  const bool plain_dx = act_x <= ACT_RELU;
+  int rc = linear_bwd(n, in, out, X, ldx, W, dY, lddy, plain_dx ? dX : nullptr, lddx, act_x == ACT_RELU, dW, db,
+                      workspace, st);
+  if (rc != EP_OK || plain_dx || !dX) return rc;
+  switch (act_x) {
+    case ACT_SILU: return linear_act_dx<T, ACT_SILU>(n, in, out, Zx, ldzx, W, dY, lddy, dX, lddx, st);
+    case ACT_SIN: return linear_act_dx<T, ACT_SIN>(n, in, out, Zx, ldzx, W, dY, lddy, dX, lddx, st);
+    default: return linear_act_dx<T, ACT_TANH>(n, in, out, X, ldx, W, dY, lddy, dX, lddx, st);
+  }
+}
+
+#undef ACT_REQUIRE
+
 }  // namespace
 
 extern "C" {
@@ -391,6 +582,30 @@ int ep_linear_bwd_f64(int n, int in, int out, const double* X, int ldx, const do
     return EP_ERR_WORKSPACE;
   }
   return linear_bwd(n, in, out, X, ldx, W, dY, lddy, dX, lddx, relu_mask, dW, db, workspace, ep::as_stream(stream));
+}
+
+int ep_linear_act_fwd_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* b, float* Y,
+                          int ldy, float* Z, int ldz, int act, ep_stream_t stream) {
+  return act_fwd_entry("ep_linear_act_fwd_f32", n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, act, stream);
+}
+
+int ep_linear_act_fwd_f64(int n, int in, int out, const double* X, int ldx, const double* W, const double* b, double* Y,
+                          int ldy, double* Z, int ldz, int act, ep_stream_t stream) {
+  return act_fwd_entry("ep_linear_act_fwd_f64", n, in, out, X, ldx, W, b, Y, ldy, Z, ldz, act, stream);
+}
+
+int ep_linear_act_bwd_f32(int n, int in, int out, const float* X, int ldx, const float* Zx, int ldzx, int act_x,
+                          const float* W, const float* dY, int lddy, float* dX, int lddx, float* dW, float* db,
+                          void* workspace, size_t workspace_bytes, ep_stream_t stream) {
+  return act_bwd_entry("ep_linear_act_bwd_f32", n, in, out, X, ldx, Zx, ldzx, act_x, W, dY, lddy, dX, lddx, dW, db,
+                       workspace, workspace_bytes, stream);
+}
+
+int ep_linear_act_bwd_f64(int n, int in, int out, const double* X, int ldx, const double* Zx, int ldzx, int act_x,
+                          const double* W, const double* dY, int lddy, double* dX, int lddx, double* dW, double* db,
+                          void* workspace, size_t workspace_bytes, ep_stream_t stream) {
+  return act_bwd_entry("ep_linear_act_bwd_f64", n, in, out, X, ldx, Zx, ldzx, act_x, W, dY, lddy, dX, lddx, dW, db,
+                       workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

@@ -448,6 +448,98 @@ def linear_bwd(X, W, dY, need_dX, relu_mask, dW=None, db=None, dX=None):
     return dX, dW, db
 
 
+ACTIVATIONS = {"none": 0, "relu": 1, "silu": 2, "sin": 3, "tanh": 4}     # the `act` codes of ep_linear_act_*
+_NEEDS_Z = ("silu", "sin")                      # act' is read from the pre-activation; relu and tanh read the output
+
+
+def linear_act_fwd(X, W, b, act, Y=None, Z=None):
+    """Y = act(X W^T + b) with act one of ACTIVATIONS; Z (optional) receives X W^T + b.  fp32 or fp64 by X's dtype."""
+    dtype = _layer_dtype(X)
+    X, W = _check(_rowmajor(X), dtype), _check(W, dtype)
+    if b is not None:
+        _check(b, dtype)
+    n, d_in = X.shape
+    d_out = W.shape[0]
+    assert W.is_contiguous() and W.shape[1] == d_in and (b is None or (b.is_contiguous() and b.numel() == d_out))
+    Y = Y if Y is not None else torch.empty((n, d_out), device=X.device, dtype=dtype)
+    call("ep_linear_act_fwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(W), _ptr(b), _ptr(_check(Y, dtype)),
+         Y.stride(0), _ptr(Z if Z is None else _check(Z, dtype)), Z.stride(0) if Z is not None else 0, ACTIVATIONS[act],
+         _stream())
+    return Y
+
+
+def linear_act_bwd(X, Zx, act_x, W, dY, need_dX, dW=None, db=None, dX=None):
+    """Backward of one layer whose input is X = act_x(Zx) ("none" for the network input): dX = (dY W) * act_x' (if
+    need_dX; the gradient w.r.t. the layer below's pre-activation), dW = dY^T X, db = colsum(dY).  Zx: the
+    pre-activation saved by linear_act_fwd, needed for silu and sin."""
+    dtype = _layer_dtype(X)
+    X, W, dY = _check(_rowmajor(X), dtype), _check(W, dtype), _check(_rowmajor(dY), dtype)
+    n, d_in = X.shape
+    d_out = W.shape[0]
+    assert W.is_contiguous() and W.shape[1] == d_in and dY.shape == (n, d_out)
+    dW = dW if dW is not None else torch.empty_like(W)
+    db = db if db is not None else torch.empty(d_out, device=X.device, dtype=dtype)
+    if need_dX and dX is None:
+        dX = torch.empty((n, d_in), device=X.device, dtype=dtype)
+    if Zx is not None:
+        _check(Zx, dtype)
+    buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device, dtype)
+    call("ep_linear_act_bwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(Zx),
+         Zx.stride(0) if Zx is not None else 0, ACTIVATIONS[act_x], _ptr(W), _ptr(dY), dY.stride(0),
+         _ptr(dX) if need_dX else None, dX.stride(0) if need_dX else 0, _ptr(dW), _ptr(db), _ptr(buf), need, _stream())
+    return (dX if need_dX else None), dW, db
+
+
+class _MlpActFn(torch.autograd.Function):
+    """x -> L_{m-1}(act(... act(L_0(x)))) with L_i(h) = h W_i^T + b_i: one ep_linear_act_fwd per layer; the backward is
+    one ep_linear_act_bwd per layer with act' of the layer below folded into its dX, so no element-wise pass and no
+    n x h temporary beyond the saved outputs (and pre-activations for silu / sin)."""
+
+    @staticmethod
+    def forward(ctx, act, x, *params):
+        m = len(params) // 2
+        Ws = [W.contiguous() for W in params[:m]]
+        bs = [b.contiguous() for b in params[m:]]
+        keep_z = act in _NEEDS_Z
+        h, hs, zs = x, [], []
+        for i in range(m):
+            hidden = i < m - 1
+            z = torch.empty((h.shape[0], Ws[i].shape[0]), device=x.device, dtype=x.dtype) if hidden and keep_z else None
+            h = linear_act_fwd(h, Ws[i], bs[i], act if hidden else "none", Z=z)
+            if hidden:
+                hs.append(h)
+                zs.append(z)
+        ctx.act, ctx.m, ctx.keep_z = act, m, keep_z
+        ctx.save_for_backward(x, *Ws, *hs, *(zs if keep_z else ()))
+        return h
+
+    @staticmethod
+    def backward(ctx, g):
+        m, act = ctx.m, ctx.act
+        saved = ctx.saved_tensors
+        x, Ws, hs = saved[0], saved[1:1 + m], saved[1 + m:2 * m]
+        zs = saved[2 * m:] if ctx.keep_z else (None,) * (m - 1)
+        dWs, dbs = [None] * m, [None] * m
+        g = g.contiguous()
+        for i in reversed(range(m)):
+            if i > 0:
+                g, dWs[i], dbs[i] = linear_act_bwd(hs[i - 1], zs[i - 1], act, Ws[i], g, True)
+            else:
+                g, dWs[i], dbs[i] = linear_act_bwd(x, None, "none", Ws[i], g, ctx.needs_input_grad[1])
+        return (None, g, *dWs, *dbs)
+
+
+def mlp_act(x, weights, biases, act):
+    """The network x -> L_{m-1}(act(... act(L_0(x)))), L_i(h) = h W_i^T + b_i (last layer linear), differentiable in x,
+    the weights and the biases; act in {"none", "relu", "silu", "sin", "tanh"}.  x's dtype selects the fp32 / fp64
+    kernels."""
+    if act not in ACTIVATIONS:
+        raise ValueError("activation must be one of %s (got %r)" % (sorted(ACTIVATIONS), act))
+    if len(weights) != len(biases) or not weights:
+        raise ValueError("need one bias per weight and at least one layer")
+    return _MlpActFn.apply(act, _rowmajor(x), *weights, *biases)
+
+
 class Dropout:
     """Dropout after every hidden ReLU of the fused step (nn.Dropout(p) of corrector_model.py::_build_net in training
     mode).  Keep masks are a pure function of (seed, step, layer, row, col) (csrc/dropout.cuh), regenerated by every

@@ -20,7 +20,8 @@ the C ABI and writes each notebook's functional on top of them with torch for th
 
 Every piece runs in fp32 (fp64 accumulation in the Gram partials) or, as the notebooks train, in fp64: the dtype of
 the tensors selects the kernels.  For fp64 build the operators with OperatorPair(K, M, device, dtype=torch.float64)
-and call .double() on the networks; activations stay torch element-wise in either precision.  Parity with the
+and call .double() on the networks.  The networks run on ops.mlp_act in either precision: SiLU, sin, tanh and ReLU are
+epilogues of the layer GEMMs, forward and backward (ep_linear_act_fwd_* / ep_linear_act_bwd_*).  Parity with the
 restated formulas (oracle/variants_port.py, fp64) is checked to fp32 tolerances in tests/test_gpu_variants.py and
 on the unrounded operators to fp64 tolerances in tests/test_gpu_variants_f64.py.
 Operators must be symmetric (FEM K and M are): the backward uses K^T = K.
@@ -196,7 +197,8 @@ _ACTIVATIONS = {"silu": nn.SiLU, "sin": Sin, "relu": nn.ReLU, "tanh": nn.Tanh}
 class CoordinateMLP(nn.Module):
     """x (n x in_dim) -> U (n x out_dim): Linear + activation per hidden width, then Linear.  `net` is a Sequential
     with the reference's indexing (state_dict keys net.<2i>.weight / .bias), scripts/simplified_loss.ipynb cell 0
-    `MLP`, scripts/loss_with_rigid_body.ipynb cell 0 `MLP`."""
+    `MLP`, scripts/loss_with_rigid_body.ipynb cell 0 `MLP`.  forward runs the whole network as ops.mlp_act: the
+    activation is the epilogue of each hidden layer's GEMM, and act' that of the dX GEMM above it."""
 
     def __init__(self, in_dim=3, out_dim=50, hidden=(256, 256, 128), activation="silu"):
         super().__init__()
@@ -206,14 +208,19 @@ class CoordinateMLP(nn.Module):
             last = h
         layers.append(KernelLinear(last, out_dim))
         self.net = nn.Sequential(*layers)
+        self.activation = activation
 
     def forward(self, x):
-        return self.net(x)
+        linear = self.net[::2]
+        return ops.mlp_act(x, [m.weight for m in linear], [m.bias for m in linear], self.activation)
 
 
 class EigenfunctionNN(nn.Module):
     """delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1: u(x) with sin activations and a learnable
-    eigenvalue lambda = |w| that is appended to the input of every layer.  forward -> (u (n x 1), lambda (1 x 1))."""
+    eigenvalue lambda = |w| that is appended to the input of every layer.  forward -> (u (n x 1), lambda (1 x 1)).
+    The appended column is folded into the bias, layer(h (+) lambda) = h W[:, :d]^T + (b + lambda W[:, d]), so the
+    four layers run as one ops.mlp_act with sin and no n x (d + 1) concatenation is formed; autograd on the k-sized
+    bias pieces gives d lambda and dW[:, d]."""
 
     def __init__(self, hidden_dim=64, input_dim=3, initial_eigenvalue=0.0):
         super().__init__()
@@ -228,8 +235,7 @@ class EigenfunctionNN(nn.Module):
 
     def forward(self, x):
         eigenvalue = torch.abs(self.eigenvalue_layer.weight).reshape(1, 1)
-        lam = eigenvalue.expand(x.shape[0], 1)
-        h = self.activation(self.fc1(torch.cat([x, lam], dim=1)))
-        h = self.activation(self.fc2(torch.cat([h, lam], dim=1)))
-        h = self.activation(self.fc3(torch.cat([h, lam], dim=1)))
-        return self.fc4(torch.cat([h, lam], dim=1)), eigenvalue
+        lam = eigenvalue.reshape(())
+        fcs = (self.fc1, self.fc2, self.fc3, self.fc4)
+        u = ops.mlp_act(x, [fc.weight[:, :-1] for fc in fcs], [fc.bias + lam * fc.weight[:, -1] for fc in fcs], "sin")
+        return u, eigenvalue

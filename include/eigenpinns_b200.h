@@ -284,6 +284,29 @@ EP_API int ep_linear_bwd_f64(int n, int in, int out, const double* X, int ldx, c
                       const double* dY, int lddy, double* dX, int lddx, int relu_mask,
                       double* dW, double* db, void* workspace, size_t workspace_bytes,
                       ep_stream_t stream);
+/* Dense layers with an activation epilogue: the SiLU / sin / tanh networks of the notebooks (CoordinateMLP,
+ * EigenfunctionNN in variants.py), same tiling and summation order as ep_linear_{fwd,bwd}_*, accurate libm math
+ * (expf / exp, sinf / sin, cosf / cos, tanhf / tanh).  act: 0 none, 1 ReLU, 2 SiLU z / (1 + e^-z), 3 sin, 4 tanh;
+ * any other value is EP_ERR_INVALID.
+ * Forward: z = X W^T + b (b may be NULL), Y = act(z); Z (may be NULL) receives z.  The backward of the next layer needs
+ * Z when act is SiLU or sin; Z may be NULL when no backward follows or act is 0, 1 or 4. */
+EP_API int ep_linear_act_fwd_f32(int n, int in, int out, const float* X, int ldx, const float* W, const float* b,
+                                 float* Y, int ldy, float* Z, int ldz, int act, ep_stream_t stream);
+EP_API int ep_linear_act_fwd_f64(int n, int in, int out, const double* X, int ldx, const double* W, const double* b,
+                                 double* Y, int ldy, double* Z, int ldz, int act, ep_stream_t stream);
+/* Backward of one layer whose input X = act_x(Zx) is the output of the layer below (act_x = 0 for the network input).
+ * dY: n x out, the gradient w.r.t. this layer's pre-activation.
+ *   dX = (dY W) * act_x'   if dX != NULL: the gradient w.r.t. the pre-activation of the layer below.
+ *        act_x' = [X > 0] (ReLU), sigmoid(z) (1 + z (1 - sigmoid(z))) (SiLU), cos z (sin) with z read from Zx, and
+ *        1 - X^2 (tanh); act_x = 0 gives dX = dY W.  Zx (ldzx) must be non-NULL when dX is and act_x is 2 or 3.
+ *   dW = dY^T X (out x in), db = column sums of dY, exactly as ep_linear_bwd_*.
+ * workspace: ep_linear_bwd_workspace_bytes(n, in, out) bytes (_f64 for the double form). */
+EP_API int ep_linear_act_bwd_f32(int n, int in, int out, const float* X, int ldx, const float* Zx, int ldzx, int act_x,
+                                 const float* W, const float* dY, int lddy, float* dX, int lddx, float* dW, float* db,
+                                 void* workspace, size_t workspace_bytes, ep_stream_t stream);
+EP_API int ep_linear_act_bwd_f64(int n, int in, int out, const double* X, int ldx, const double* Zx, int ldzx,
+                                 int act_x, const double* W, const double* dY, int lddy, double* dX, int lddx,
+                                 double* dW, double* db, void* workspace, size_t workspace_bytes, ep_stream_t stream);
 
 /* ---- corrector MLP, bf16 tcgen05 path ("perf mode") --------------------------------------
  * Same Linear / ReLU network, evaluated layer by layer on the 5th-generation tensor cores:
