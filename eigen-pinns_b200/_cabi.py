@@ -90,6 +90,19 @@ SIGNATURES = {
     "ep_grad_sqnorm_f32": (c_int, [c_sz, c_p, c_p, c_p]),
     "ep_adam_clip_step_f32": (c_int, [c_sz, c_p, c_p, c_p, c_p, c_f, c_p, c_f, c_f, c_f, c_f, c_int, c_f,
                                       c_p, c_p]),
+    "ep_grad_sqnorm_f64": (c_int, [c_sz, c_p, c_p, c_p]),
+    "ep_adam_clip_step_f64": (c_int, [c_sz, c_p, c_p, c_p, c_p, c_d, c_p, c_d, c_d, c_d, c_d, c_int, c_d,
+                                      c_p, c_p]),
+    "ep_single_mode_max_prev": (c_int, []),
+    "ep_single_mode_workspace_bytes": (c_sz, [c_int]),
+    "ep_single_mode_fwd_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p, c_d, c_p, c_p, c_p, c_sz, c_p]),
+    "ep_single_mode_fwd_f64": (c_int, [c_int, c_int, c_p, c_p, c_p, c_p, c_int, c_p, c_d, c_p, c_p, c_p, c_sz, c_p]),
+    "ep_single_mode_bwd_f32": (c_int, [c_int, c_int, c_p, c_p, c_p, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ep_single_mode_bwd_f64": (c_int, [c_int, c_int, c_p, c_p, c_p, c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ep_single_mode_fold_fwd_f32": (c_int, [c_int, c_p, c_p, c_p, c_p]),
+    "ep_single_mode_fold_fwd_f64": (c_int, [c_int, c_p, c_p, c_p, c_p]),
+    "ep_single_mode_fold_bwd_f32": (c_int, [c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
+    "ep_single_mode_fold_bwd_f64": (c_int, [c_int, c_p, c_p, c_p, c_p, c_p, c_p]),
     "ep_fps_workspace_bytes": (c_sz, [c_i64]),
     "ep_fps_f64": (c_int, [c_i64, c_p, c_int, c_i64, c_p, c_p, c_sz, c_p]),
     "ep_fps_f64_host": (c_int, [c_i64, c_p, c_int, c_i64, c_p]),
@@ -131,6 +144,10 @@ KERNELS_PER_CALL = {
     "ep_mode_scale_fwd_f32": 1, "ep_mode_scale_bwd_f32": 2,
     "ep_dropout_keep_mask_u8": 1, "ep_linear_fwd_dropout_f32": 1, "ep_linear_bwd_dropout_f32": 5,
     "ep_tc_linear_fwd_dropout_bf16": 1, "ep_tc_linear_dx_dropout_bf16": 1, "ep_tc_chain_fwd_dropout_bf16": 1,
+    "ep_grad_sqnorm_f64": 2, "ep_adam_clip_step_f64": 1,
+    "ep_single_mode_fwd_f32": 2, "ep_single_mode_fwd_f64": 2, "ep_single_mode_bwd_f32": 1, "ep_single_mode_bwd_f64": 1,
+    "ep_single_mode_fold_fwd_f32": 1, "ep_single_mode_fold_fwd_f64": 1, "ep_single_mode_fold_bwd_f32": 1,
+    "ep_single_mode_fold_bwd_f64": 1,
 }
 launch_counter = 0
 launch_by_entry = {}          # entry point -> kernels launched through it (bench.py reports the per-step table)

@@ -468,10 +468,11 @@ def linear_act_fwd(X, W, b, act, Y=None, Z=None):
     return Y
 
 
-def linear_act_bwd(X, Zx, act_x, W, dY, need_dX, dW=None, db=None, dX=None):
+def linear_act_bwd(X, Zx, act_x, W, dY, need_dX, dW=None, db=None, dX=None, workspace=None):
     """Backward of one layer whose input is X = act_x(Zx) ("none" for the network input): dX = (dY W) * act_x' (if
     need_dX; the gradient w.r.t. the layer below's pre-activation), dW = dY^T X, db = colsum(dY).  Zx: the
-    pre-activation saved by linear_act_fwd, needed for silu and sin."""
+    pre-activation saved by linear_act_fwd, needed for silu and sin.  workspace: the caller's scratch of at least
+    ep_linear_bwd_workspace_bytes (default: the shared per-device buffer)."""
     dtype = _layer_dtype(X)
     X, W, dY = _check(_rowmajor(X), dtype), _check(W, dtype), _check(_rowmajor(dY), dtype)
     n, d_in = X.shape
@@ -483,7 +484,10 @@ def linear_act_bwd(X, Zx, act_x, W, dY, need_dX, dW=None, db=None, dX=None):
         dX = torch.empty((n, d_in), device=X.device, dtype=dtype)
     if Zx is not None:
         _check(Zx, dtype)
-    buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device, dtype)
+    if workspace is None:
+        buf, need = _linear_bwd_workspace(n, d_in, d_out, X.device, dtype)
+    else:
+        buf, need = workspace, workspace.numel()
     call("ep_linear_act_bwd_" + _scalar(X), n, d_in, d_out, _ptr(X), X.stride(0), _ptr(Zx),
          Zx.stride(0) if Zx is not None else 0, ACTIVATIONS[act_x], _ptr(W), _ptr(dY), dY.stride(0),
          _ptr(dX) if need_dX else None, dX.stride(0) if need_dX else 0, _ptr(dW), _ptr(db), _ptr(buf), need, _stream())
@@ -628,15 +632,110 @@ def linear(x, W, b, relu=False):
 
 # ------------------------------------------------------------------------------- optimiser
 def grad_sqnorm(g, out):
-    call("ep_grad_sqnorm_f32", g.numel(), _ptr(g), _ptr(out), _stream())
+    """out (fp64, device) = sum g^2; g fp32 or fp64."""
+    call("ep_grad_sqnorm_" + ("f64" if g.dtype == torch.float64 else "f32"), g.numel(), _ptr(g), _ptr(out), _stream())
     return out
 
 
 def adam_clip_step(p, g, m, v, lr, beta1, beta2, eps, weight_decay, step, max_norm, sq_norm, hyper_dev=None):
-    """hyper_dev: 8-byte device buffer {float lr, int32 step} overriding lr / step (graph replay)."""
+    """hyper_dev: device buffer overriding lr / step (graph replay): {float lr, int32 step} for fp32 p, {double lr,
+    double step} for fp64 p.  max_norm <= 0 or sq_norm None: no clipping."""
+    if p.dtype == torch.float64:
+        for t in (p, g, m, v):
+            _check(t, torch.float64)
+        call("ep_adam_clip_step_f64", p.numel(), _ptr(p), _ptr(g), _ptr(m), _ptr(v), float(lr), _ptr(hyper_dev),
+             float(beta1), float(beta2), float(eps), float(weight_decay), int(step), float(max_norm), _ptr(sq_norm),
+             _stream())
+        return
     call("ep_adam_clip_step_f32", p.numel(), _ptr(p), _ptr(g), _ptr(m), _ptr(v), float(lr), _ptr(hyper_dev),
          float(beta1), float(beta2), float(eps), float(weight_decay), int(step), float(max_norm), _ptr(sq_norm),
          _stream())
+
+
+# ------------------------------------------------------------------------------- single mode with learnable eigenvalue
+def single_mode_max_prev():
+    """Largest number of earlier modes P the single-mode kernels take."""
+    return query("ep_single_mode_max_prev")
+
+
+def single_mode_workspace(P, device):
+    """Device scratch of ep_single_mode_fwd_* for P earlier modes."""
+    if not 0 <= P <= single_mode_max_prev():
+        raise _cabi.EpError("P = %d earlier modes: the single-mode kernels take 0 .. %d" % (P, single_mode_max_prev()))
+    return torch.empty(query("ep_single_mode_workspace_bytes", P), dtype=torch.uint8, device=device)
+
+
+def _column(t, dtype, n):
+    _check(t, dtype)
+    if t.numel() != n or (t.dim() == 2 and t.shape[1] != 1) or not t.is_contiguous():
+        raise ValueError("expected a contiguous n x 1 column of %d values" % n)
+    return t
+
+
+def _prev_block(Q, dtype, n):
+    """(P, ldq) of the n x P block of the earlier modes' M u_p (None: P = 0)."""
+    if Q is None:
+        return 0, 1
+    _check(Q, dtype)
+    if Q.dim() != 2 or Q.shape[0] != n:
+        raise ValueError("Q must be n x P")
+    return Q.shape[1], Q.stride(0)
+
+
+def single_mode_fwd(u, Lu, Mu, Q, w, ortho_weight, loss, coef, workspace):
+    """loss[0:4] = [total, eig, norm, ortho] and coef[0:3+P] (fp64, device) of the single-mode functional
+    (include/eigenpinns_b200.h).  u, Lu, Mu: n x 1; Q: n x P (None for P = 0); w: the eigenvalue weight (1 value)."""
+    dtype = _layer_dtype(u)
+    n = u.shape[0]
+    u, Lu, Mu = (_column(t, dtype, n) for t in (u, Lu, Mu))
+    _check(w, dtype)
+    P, ldq = _prev_block(Q, dtype, n)
+    _check(loss, torch.float64)
+    _check(coef, torch.float64)
+    call("ep_single_mode_fwd_" + _scalar(u), n, P, _ptr(u), _ptr(Lu), _ptr(Mu), _ptr(Q), ldq, _ptr(w),
+         float(ortho_weight), _ptr(loss), _ptr(coef), _ptr(workspace), workspace.numel(), _stream())
+    return loss, coef
+
+
+def single_mode_bwd(Lu, Mu, Q, w, coef, gL, gM, D):
+    """gL = (2/n) r, gM = -(2/n) lambda r, D = 4 (u^T M u - 1) Mu + Q c from the coefficients of single_mode_fwd;
+    dL/du = spmm2_sum(L, M, gL, gM, D) for symmetric L, M."""
+    dtype = _layer_dtype(Lu)
+    n = Lu.shape[0]
+    Lu, Mu, gL, gM, D = (_column(t, dtype, n) for t in (Lu, Mu, gL, gM, D))
+    _check(w, dtype)
+    _check(coef, torch.float64)
+    P, ldq = _prev_block(Q, dtype, n)
+    call("ep_single_mode_bwd_" + _scalar(Lu), n, P, _ptr(Lu), _ptr(Mu), _ptr(Q), ldq, _ptr(w), _ptr(coef), _ptr(gL),
+         _ptr(gM), _ptr(D), _stream())
+    return gL, gM, D
+
+
+def _dims_array(dims):
+    return (ctypes.c_int * len(dims))(*[int(d) for d in dims])
+
+
+def single_mode_fold_fwd(dims, params, eff):
+    """eff = [W_l[:, :d] | b_l + lambda W_l[:, d]] per layer from the flat params [W_l | b_l ... | w]
+    (include/eigenpinns_b200.h); dims: the len(layers) + 1 widths, input first."""
+    dtype = _layer_dtype(params)
+    _check(params, dtype)
+    _check(eff, dtype)
+    call("ep_single_mode_fold_fwd_" + _scalar(params), len(dims) - 1, _dims_array(dims), _ptr(params), _ptr(eff),
+         _stream())
+    return eff
+
+
+def single_mode_fold_bwd(dims, params, grad_eff, dloss_dlam, grad):
+    """grad (layout of params) from grad_eff (layout of eff) and dL/dlambda of the loss (fp64 device scalar or None)."""
+    dtype = _layer_dtype(params)
+    for t in (params, grad_eff, grad):
+        _check(t, dtype)
+    if dloss_dlam is not None:
+        _check(dloss_dlam, torch.float64)
+    call("ep_single_mode_fold_bwd_" + _scalar(params), len(dims) - 1, _dims_array(dims), _ptr(params),
+         _ptr(grad_eff), _ptr(dloss_dlam), _ptr(grad), _stream())
+    return grad
 
 
 # ------------------------------------------------------------------------------- halo rows

@@ -401,6 +401,58 @@ EP_API int ep_adam_clip_step_f32(size_t n, float* p, const float* g, float* m, f
                           const float* hyper_dev, float beta1, float beta2, float eps,
                           float weight_decay, int step, float max_norm, const double* sq_norm,
                           ep_stream_t stream);
+/* fp64 forms for networks trained in double (delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1 trains
+ * EigenfunctionNN with Adam(betas=(0.999, 0.9999)) in fp64).  Same update, order and clipping semantics (no clipping
+ * when max_norm <= 0 or sq_norm is NULL); hyper_dev (device, may be NULL) = {double lr, double t} with t an integer. */
+EP_API int ep_grad_sqnorm_f64(size_t n, const double* g, double* sq_out, ep_stream_t stream);
+EP_API int ep_adam_clip_step_f64(size_t n, double* p, const double* g, double* m, double* v, double lr,
+                                 const double* hyper_dev, double beta1, double beta2, double eps, double weight_decay,
+                                 int step, double max_norm, const double* sq_norm, ep_stream_t stream);
+
+/* ---- one eigenfunction at a time: delta_pinns_validation/iterative_eigenvalues_on_cloud.ipynb cell 1 ---------------
+ * (EigenfunctionNN; compute_eigenvalue_loss, compute_normalization_loss, compute_orthogonality_loss), the pieces of an
+ * autograd-free training step (csrc/single_mode.cu).  u, Lu = L u, Mu = M u: n x 1 contiguous (ep_spmm2_csr_* at k = 1);
+ * w: the eigenvalue weight (device, one value), lambda = |w|; Q: n x P row-major (ldq >= P), column p = M u_p of the
+ * p-th earlier mode (constant; may be NULL when P = 0).  0 <= P <= ep_single_mode_max_prev() (64; larger P is
+ * EP_ERR_UNSUPPORTED), n >= 1.  With r = Lu - lambda Mu:
+ *   forward   loss[0..4) = [total, eig, norm, ortho] (fp64, device): eig = mean(r^2), norm = (u^T M u - 1)^2,
+ *             ortho = sum_p (u^T Q_p)^2, total = eig + norm + ortho_weight * ortho;
+ *             coef[0..3+P) (fp64, device) = [2/n, 4 (u^T M u - 1), dL/dlambda = -(2/n) sum r o Mu, c_p = 2 ortho_weight
+ *             u^T Q_p].  Sums are fp64, per CTA into the workspace (ep_single_mode_workspace_bytes(P)), then reduced
+ *             by one CTA in a fixed order: deterministic and graph-capturable.
+ *   backward  gL = (2/n) r, gM = -(2/n) lambda r, D = 4 (u^T M u - 1) Mu + Q c  (r recomputed, not stored); then
+ *             ep_spmm2_sum_csr_*(L, M, gL, gM, D) = dL/du for symmetric L, M. */
+EP_API int ep_single_mode_max_prev(void);
+EP_API size_t ep_single_mode_workspace_bytes(int P);
+EP_API int ep_single_mode_fwd_f32(int n, int P, const float* u, const float* Lu, const float* Mu, const float* Q,
+                                  int ldq, const float* w, double ortho_weight, double* loss, double* coef,
+                                  void* workspace, size_t workspace_bytes, ep_stream_t stream);
+EP_API int ep_single_mode_fwd_f64(int n, int P, const double* u, const double* Lu, const double* Mu, const double* Q,
+                                  int ldq, const double* w, double ortho_weight, double* loss, double* coef,
+                                  void* workspace, size_t workspace_bytes, ep_stream_t stream);
+EP_API int ep_single_mode_bwd_f32(int n, int P, const float* Lu, const float* Mu, const float* Q, int ldq,
+                                  const float* w, const double* coef, float* gL, float* gM, float* D,
+                                  ep_stream_t stream);
+EP_API int ep_single_mode_bwd_f64(int n, int P, const double* Lu, const double* Mu, const double* Q, int ldq,
+                                  const double* w, const double* coef, double* gL, double* gM, double* D,
+                                  ep_stream_t stream);
+/* lambda appended to every layer's input, folded into the bias: layer(h (+) lambda) = h W[:, :d]^T + (b + lambda
+ * W[:, d]).  dims: HOST array of n_layers + 1 widths (input first), 1 <= n_layers <= 8.  Flat device layouts, per layer
+ * l with input width d and output width o, in layer order:
+ *   params, grad     [W_l (o x (d + 1), row-major) | b_l (o)] ... then w (one value)
+ *   eff, grad_eff    [W_eff,l (o x d) | b_eff,l (o)] ...
+ * Forward: W_eff,l = W_l[:, :d], b_eff,l = b_l + lambda W_l[:, d] (product, then sum: as the autograd form rounds).
+ * Backward from dW_eff, db_eff (grad_eff) and dL/dlambda of the loss (device fp64, may be NULL = 0):
+ *   dW_l[:, :d] = dW_eff,l, dW_l[:, d] = lambda db_eff,l, db_l = db_eff,l,
+ *   dw = sign(w) (dL/dlambda + sum_l db_eff,l^T W_l[:, d])   (sign(0) = 0, torch's gradient of |w|). */
+EP_API int ep_single_mode_fold_fwd_f32(int n_layers, const int* dims, const float* params, float* eff,
+                                       ep_stream_t stream);
+EP_API int ep_single_mode_fold_fwd_f64(int n_layers, const int* dims, const double* params, double* eff,
+                                       ep_stream_t stream);
+EP_API int ep_single_mode_fold_bwd_f32(int n_layers, const int* dims, const float* params, const float* grad_eff,
+                                       const double* dloss_dlam, float* grad, ep_stream_t stream);
+EP_API int ep_single_mode_fold_bwd_f64(int n_layers, const int* dims, const double* params, const double* grad_eff,
+                                       const double* dloss_dlam, double* grad, ep_stream_t stream);
 
 /* ---- samplers: samplers.py:97-143 (farthest point), :9-94 (voxel) ----------------------
  * fp64, bit-exact w.r.t. numpy: d = sqrt((dx*dx + dy*dy) + dz*dz) with IEEE round-to-nearest
